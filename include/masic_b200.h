@@ -142,8 +142,8 @@ void masic_conv_plan_destroy(MasicConvPlan* plan);
 int masic_conv_plan_info(const MasicConvPlan* plan, double* flops, double* hbm_bytes,
                          int* n_work_items, int* smem_bytes);
 
-/* Debug aid: clock64() stamps of CTA 0 (64 work items x 16 slots) when the plan was created with
- * MASIC_CONV_TRACE=1 in the environment; MASIC_ENOSUP otherwise. */
+/* Kept for ABI compatibility: the kernels no longer record clock64() stamps, so this always returns
+ * MASIC_ENOSUP. */
 int masic_conv_plan_trace(const MasicConvPlan* plan, long long* out_host);
 
 /* Pack torch-layout fp32 weights into the bf16 k-block layout the plan reads.

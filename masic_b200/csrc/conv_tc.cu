@@ -32,8 +32,6 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <vector>
@@ -109,9 +107,6 @@ struct KParams {
   uint32_t idesc_norm;   // the GDN norm MMA always runs on bf16 operands (x^2 rounded on the ALU pipe, gamma' bf16)
   int f16;         // 16-bit operand / activation format: 0 = bf16, 1 = fp16 (cvt16.cuh)
   int gdn2;        // 1: EPI_GDN2 (two epilogue teams, resident weights, one tile per item)
-  int gdnt;        // 1: EPI_GDNT (one epilogue team per accumulator slot, norm in place)
-  int debug;       // timing experiments only (results are garbage): bit0 skip A loads, bit1 skip B loads, bit2 skip stores,
-                   // bit3 skip the GDN norm MMA, bit4 skip the whole epilogue
 };
 
 // misc smem region layout (byte offsets from smem_misc_off)
@@ -262,13 +257,7 @@ __device__ __forceinline__ Item next_item(const KParams& p, Cursor& c, int u_end
 
 // EPI selects the epilogue at compile time so that each variant gets its own register allocation (the GDN epilogue
 // is issue- and latency-bound: a spill there costs ~40 % on the 608x1088 layers)
-constexpr int EPI_PLAIN = 0, EPI_GDN = 1, EPI_RES = 2, EPI_GDN2 = 3, EPI_GDNT = 4;
-// EPI_GDNT ("teams"): the fused GDN epilogue of EPI_GDN with the item's two tiles drained CONCURRENTLY, one team of 8
-// warps per accumulator slot (64 channels per thread instead of 32), each team with its own A2 / staging blocks and
-// its own norm-MMA barrier; the norm is still written in place over the accumulator, so a thread keeps 64 fp32 x values
-// in registers across the MMA: the four epilogue warpgroups raise their register budget to 104 with setmaxnreg and the
-// role warpgroup drops to 64 — the CTA pool must balance exactly ((96 - 64) x 128 = (104 - 96) x 512 registers), or the
-// TRY_ALLOC of the last epilogue warpgroup spins forever.  The per-tile chain is latency-bound, so two tiles in flight nearly halve it.
+constexpr int EPI_PLAIN = 0, EPI_GDN = 1, EPI_RES = 2, EPI_GDN2 = 3;
 // EPI_GDN2 (layers whose whole weight set stays in shared memory, i.e. g_a_conv1): one tile per work item, TWO epilogue
 // teams of 8 warps that alternate over the items, each with its own accumulator, its own norm accumulator (the norm
 // MMA no longer overwrites x, so nothing has to stay in registers across it) and its own A2 / staging blocks.  The
@@ -322,14 +311,14 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
     }
     mbar_init(sMisc + MISC_GDN_BAR, 1);
     mbar_init(sMisc + MISC_G_FULL, 1);
-    mbar_init(sMisc + MISC_A2_READY, (EPI == EPI_GDN2 || EPI == EPI_GDNT) ? 1 : 2);   // GDN2 / GDNT: the second team's norm-MMA barrier
+    mbar_init(sMisc + MISC_A2_READY, EPI == EPI_GDN2 ? 1 : 2);   // GDN2: the second team's norm-MMA barrier
     fence_mbar_init();
   }
   if (warp == 3) {
     if (CG2) { tmem_alloc_cg2(sMisc + MISC_TMEM_PTR, TMEM_COLS); tmem_relinquish_cg2(); }
     else { tmem_alloc(sMisc + MISC_TMEM_PTR, TMEM_COLS); tmem_relinquish(); }
   }
-  if ((EPI == EPI_GDN || EPI == EPI_GDN2 || EPI == EPI_GDNT) && threadIdx.x >= 128) {       // the single n-tile's bias / beta' stay in smem for the whole kernel
+  if ((EPI == EPI_GDN || EPI == EPI_GDN2) && threadIdx.x >= 128) {       // the single n-tile's bias / beta' stay in smem for the whole kernel
     float* bs = reinterpret_cast<float*>(smem_gen + p.smem_misc_off + MISC_BIAS);
     float* be = reinterpret_cast<float*>(smem_gen + p.smem_misc_off + MISC_BETA);
     const int i = threadIdx.x - 128;
@@ -350,11 +339,7 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
 
   // Role loops are WARP-UNIFORM (all 32 lanes walk them, barrier waits included) and only the
   // issue instructions sit under elect_one(): tcgen05.mma / TMA are uniform-datapath instructions.
-  const bool free_run = (p.debug & 32) != 0;     // timing experiment: MMA issuers ignore the A/B rings entirely
-  // EPI_GDNT: the role warpgroup (warps 0-3) hands registers to the four epilogue warpgroups
-  if (warp < 4) {
-  if (EPI == EPI_GDNT) asm volatile("setmaxnreg.dec.sync.aligned.u32 64;");     // ONE instruction for the whole role warpgroup
-  if (warp == 0 && !free_run) {
+  if (warp == 0) {
     // ===================== A producer: activation strips =====================
     uint32_t st = 0, ph = 0;
     const uint32_t n_st = p.a_stages, strip_bytes = p.strip_bytes, st_bytes = p.pair * p.strip_bytes;
@@ -367,22 +352,18 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
         const uint32_t full = sMisc + MISC_A_FULL + 8 * st;
         mbar_wait(sMisc + MISC_A_EMPTY + 8 * st, ph ^ 1);
         if (elect_one()) {
-          if (p.debug & 1) {
-            if (rank == 0) mbar_arrive(full);
-          } else {
-            // the leader's barrier collects the strips of every tile of the item, whichever CTA stages them
-            if (rank == 0) mbar_expect_tx(full, it.cnt * strip_bytes);
-            const uint32_t fl = leader_bar(full);
+          // the leader's barrier collects the strips of every tile of the item, whichever CTA stages them
+          if (rank == 0) mbar_expect_tx(full, it.cnt * strip_bytes);
+          const uint32_t fl = leader_bar(full);
 #pragma unroll
-            for (int t = 0; t < 2; ++t) {
-              if (it.valid[t]) {
-                if (CG2)
-                  tma_load_5d_cg2(sA + st * st_bytes + t * strip_bytes, &p.tmA, fl, sp.c0 + gc0, it.x0[t] + sp.dx, sp.p2,
-                                  it.y0[t] + sp.dy, it.n[t]);
-                else
-                  tma_load_5d(sA + st * st_bytes + t * strip_bytes, &p.tmA, fl, sp.c0 + gc0, it.x0[t] + sp.dx, sp.p2,
-                              it.y0[t] + sp.dy, it.n[t]);
-              }
+          for (int t = 0; t < 2; ++t) {
+            if (it.valid[t]) {
+              if (CG2)
+                tma_load_5d_cg2(sA + st * st_bytes + t * strip_bytes, &p.tmA, fl, sp.c0 + gc0, it.x0[t] + sp.dx, sp.p2,
+                                it.y0[t] + sp.dy, it.n[t]);
+              else
+                tma_load_5d(sA + st * st_bytes + t * strip_bytes, &p.tmA, fl, sp.c0 + gc0, it.x0[t] + sp.dx, sp.p2,
+                            it.y0[t] + sp.dy, it.n[t]);
             }
           }
         }
@@ -390,9 +371,9 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
         if (++st == n_st) { st = 0; ph ^= 1; }
       }
     }
-  } else if (warp == 1 && !free_run) {
+  } else if (warp == 1) {
     // ===================== B producer: weight k-blocks (+ gamma once) =====================
-    if ((EPI == EPI_GDN || EPI == EPI_GDN2 || EPI == EPI_GDNT) && elect_one()) {
+    if ((EPI == EPI_GDN || EPI == EPI_GDN2) && elect_one()) {
       tma_prefetch_desc(&p.tmG);
       if (CG2) {          // each CTA holds the 64 N-rows of gamma' it feeds to the pair's norm MMA
         if (rank == 0) mbar_expect_tx(sMisc + MISC_G_FULL, 2 * STAGE_BLK_BYTES);
@@ -414,13 +395,9 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
       // MMAs take less time than one trip round the ring)
       if (u_begin < u_end && elect_one()) {
         const Variant& v0 = p.var[0];
-        if (p.debug & 2) {
-          mbar_arrive(sMisc + MISC_B_FULL);
-        } else {
-          mbar_expect_tx(sMisc + MISC_B_FULL, v0.n_bops * st_bytes);
-          for (int i = 0; i < v0.n_bops; ++i)
-            tma_load_2d(sB + i * st_bytes, &p.tmB, sMisc + MISC_B_FULL, 0, p.bops[v0.bop_off + i]);
-        }
+        mbar_expect_tx(sMisc + MISC_B_FULL, v0.n_bops * st_bytes);
+        for (int i = 0; i < v0.n_bops; ++i)
+          tma_load_2d(sB + i * st_bytes, &p.tmB, sMisc + MISC_B_FULL, 0, p.bops[v0.bop_off + i]);
       }
       __syncwarp();
     } else
@@ -434,13 +411,9 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
         const uint32_t full = sMisc + MISC_B_FULL + 8 * st;
         mbar_wait(sMisc + MISC_B_EMPTY + 8 * st, ph ^ 1);
         if (elect_one()) {
-          if (p.debug & 2) {
-            if (rank == 0) mbar_arrive(full);
-          } else {
-            if (rank == 0) mbar_expect_tx(full, CG2 ? 2 * st_bytes : st_bytes);
-            if (CG2) tma_load_2d_cg2(sB + st * st_bytes, &p.tmB, leader_bar(full), 0, row0 + nrow);
-            else tma_load_2d(sB + st * st_bytes, &p.tmB, full, 0, row0 + nrow);
-          }
+          if (rank == 0) mbar_expect_tx(full, CG2 ? 2 * st_bytes : st_bytes);
+          if (CG2) tma_load_2d_cg2(sB + st * st_bytes, &p.tmB, leader_bar(full), 0, row0 + nrow);
+          else tma_load_2d(sB + st * st_bytes, &p.tmB, full, 0, row0 + nrow);
         }
         __syncwarp();
         if (++st == n_st) { st = 0; ph ^= 1; }
@@ -458,8 +431,10 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
     const uint64_t descA0 = umma_desc_sw128(sA) + slot * (p.strip_bytes >> 4), descB0 = umma_desc_sw128(sB);
     const uint32_t a_step = (p.pair * p.strip_bytes) >> 4, b_step = p.b_stage_bytes >> 4;
     const uint32_t idesc = p.idesc;
-    const bool b_res = p.b_resident != 0;
-    if (b_res && u_begin < u_end) mbar_wait(sMisc + MISC_B_FULL, 0);     // the whole weight set has landed
+    // with the range test folded in, b_res is a computed value that ptxas keeps in a uniform predicate; the bare
+    // kernel parameter was re-read from the constant bank twice per tap of the loop below
+    const bool b_res = p.b_resident != 0 && u_begin < u_end;
+    if (b_res) mbar_wait(sMisc + MISC_B_FULL, 0);     // the whole weight set has landed
     int n_item = 0;
     for (Cursor cur = cursor_init(p, u_begin); cur.u < u_end; ++n_item) {
       const Item it = next_item<CG2>(p, cur, u_end, rank);
@@ -473,12 +448,12 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
       for (int i = i0; i < i1; ++i) {
         const Strip sp = p.strips[i];
         const uint32_t nk = sp.nk & 15u, k0 = sp.nk >> 4;
-        if (!free_run) mbar_wait(sMisc + MISC_A_FULL + 8 * sa, pa);
+        mbar_wait(sMisc + MISC_A_FULL + 8 * sa, pa);
         uint64_t adesc = descA0 + (sa * a_step + static_cast<uint32_t>(sp.a_row0) * 64u + 2u * k0);
         const int64_t a_inc = static_cast<int64_t>(sp.a_step) * 64;
         const int n_taps = sp.n_taps;
         for (int j = 0; j < n_taps; ++j) {
-          if (!free_run && !b_res) mbar_wait(sMisc + MISC_B_FULL + 8 * sb, pb);
+          if (!b_res) mbar_wait(sMisc + MISC_B_FULL + 8 * sb, pb);
           tc_fence_after();
           if (elect_one()) {
             const uint64_t bdesc = descB0 + (sb * b_step + 2u * k0);
@@ -496,9 +471,9 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
                 for (uint32_t k = 0; k < nk; ++k) mma(d0, adesc + 2 * k, bdesc + 2 * k, k ? 1u : acc);
               }
             }
-            if (!free_run && !b_res) commit(sMisc + MISC_B_EMPTY + 8 * sb);
+            if (!b_res) commit(sMisc + MISC_B_EMPTY + 8 * sb);
             if (j + 1 == n_taps) {
-              if (!free_run) commit(sMisc + MISC_A_EMPTY + 8 * sa);
+              commit(sMisc + MISC_A_EMPTY + 8 * sa);
               if (i + 1 == i1) commit(sMisc + MISC_ACC_FULL + 8 * buf);
             }
           }
@@ -510,144 +485,6 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
         if (++sa == n_sa) { sa = 0; pa ^= 1; }
       }
     }
-  }
-  } else if (EPI == EPI_GDNT) {
-    // ===================== epilogue, one team per accumulator slot (see EPI_GDNT above) =====================
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 104;");
-    const int team = (warp - 4) >> 3;                             // = slot of the item this team drains
-    const int hf = ((warp - 4) >> 2) & 1;                         // channels 64 hf .. 64 hf + 63 = A2 / staging block hf of the team
-    const int ew = warp & 3;
-    const int t = ew * 32 + lane;
-    const uint32_t lane_sel = static_cast<uint32_t>(ew * 32) << 16;
-    const uint32_t tbar = 1 + team;
-    const bool leader = (t == 0 && hf == 0);
-    const uint32_t sbuf = sStage + team * 2 * STAGE_BLK_BYTES;
-    const uint32_t bias_s = sMisc + MISC_BIAS, beta_s = sMisc + MISC_BETA;
-    const uint32_t gbar = sMisc + (team ? MISC_A2_READY : MISC_GDN_BAR);
-    const bool fwd = (p.gdn == MASIC_GDN_FWD);
-    const bool nostore = (p.debug & 4) != 0;
-    const uint32_t arow = sbuf + hf * STAGE_BLK_BYTES + t * 128;
-    uint32_t gpar = 0;
-    if (hf == 0 && ew == 0) mbar_wait(sMisc + MISC_G_FULL, 0);   // gamma' resident before this warp issues norm MMAs
-    int n_item = 0;
-    for (Cursor cur = cursor_init(p, u_begin); cur.u < u_end; ++n_item) {
-      const Item it = next_item<CG2>(p, cur, u_end, rank);
-      const Variant& v = p.var[it.var];
-      const int buf = n_item & 1;
-      mbar_wait(sMisc + MISC_ACC_FULL + 8 * buf, (n_item >> 1) & 1);
-      tc_fence_after();
-      if ((p.debug & 16) || team >= it.nslots) {                  // nothing to drain (odd last item) / timing experiment
-        tc_fence_before();
-        mbar_arrive(sMisc + MISC_ACC_EMPTY + 8 * buf);
-        continue;
-      }
-      const int tn = team ? it.n[1] : it.n[0], ty0 = team ? it.y0[1] : it.y0[0], tx0 = team ? it.x0[1] : it.x0[0];
-      const uint32_t acc_addr = tmem_base + lane_sel + buf * 256 + team * 128;
-      float rs = 1.0f;
-      if (p.rowscale) {
-        const int y = ty0 + (t >> 3), x = tx0 + (t & 7);
-        if (y < p.rs_H && x < p.rs_W)
-          rs = __ldg(p.rowscale + (static_cast<size_t>(tn * p.rs_H + y) * p.rs_W + x) * p.rs_stride + p.rs_off);
-      }
-      uint64_t x2[32];                                            // x = acc + bias: 64 channels, two per register pair
-      if (leader) tma_store_wait_read<0>();                       // the team's previous output tile has left the staging blocks
-      named_bar_sync(tbar, 256);
-      // ---- pass 1: x stays in registers; A2[:, 64 hf .. +63] = 16-bit(x^2)
-#pragma unroll
-      for (int c = 0; c < 2; ++c) {
-        const int cb = hf * 64 + c * 32;
-        uint32_t r[32];
-        tmem_ld16(acc_addr + cb, *reinterpret_cast<uint32_t(*)[16]>(&r[0]));
-        tmem_ld16(acc_addr + cb + 16, *reinterpret_cast<uint32_t(*)[16]>(&r[16]));
-        tmem_ld_wait();
-#pragma unroll
-        for (int q = 0; q < 8; ++q) {
-          uint64_t b0, b1;
-          ld_shared_p2(bias_s + (cb + 4 * q) * 4, b0, b1);
-          x2[16 * c + 2 * q] = add2(pk2u(r[4 * q], r[4 * q + 1]), b0);
-          x2[16 * c + 2 * q + 1] = add2(pk2u(r[4 * q + 2], r[4 * q + 3]), b1);
-        }
-#pragma unroll
-        for (int c8 = 0; c8 < 4; ++c8) {
-          const uint64_t* xx = &x2[16 * c + 4 * c8];
-          st_shared_v4(arow + (((4 * c + c8) ^ (t & 7)) << 4), pack_norm_operand<F16>(mul2(xx[0], xx[0])),
-                       pack_norm_operand<F16>(mul2(xx[1], xx[1])), pack_norm_operand<F16>(mul2(xx[2], xx[2])),
-                       pack_norm_operand<F16>(mul2(xx[3], xx[3])));
-        }
-      }
-      fence_proxy_async_smem();
-      tc_fence_before();
-      named_bar_sync(tbar, 256);
-      if (!(p.debug & 8)) {
-        if (hf == 0 && ew == 0) {
-          tc_fence_after();
-          if (elect_one()) {
-            // norm = x^2 * gamma'^T written IN PLACE over the team's accumulator
-            const uint32_t d2 = tmem_base + buf * 256 + team * 128;
-            const uint64_t dh = umma_desc_sw128(0);
-#pragma unroll
-            for (int kb = 0; kb < 2; ++kb) {
-              const uint64_t a2 = dh | (((sbuf + kb * STAGE_BLK_BYTES) & 0x3FFFFu) >> 4);
-              const uint64_t g2 = dh | (((sG + kb * STAGE_BLK_BYTES) & 0x3FFFFu) >> 4);
-#pragma unroll
-              for (int k = 0; k < 4; ++k) umma_bf16(d2, a2 + 2 * k, g2 + 2 * k, p.idesc_norm, (kb | k) ? 1u : 0u);
-            }
-            umma_commit(gbar);
-          }
-          __syncwarp();
-        }
-        mbar_wait(gbar, gpar);
-        gpar ^= 1;
-      }
-      tc_fence_after();
-      // ---- pass 2: out = x * rsqrt(beta' + norm)  (IGDN: x * sqrt(.)); staging rows re-use the A2 rows
-      const uint64_t rs2 = pk2(rs, rs);
-#pragma unroll
-      for (int c = 0; c < 2; ++c) {
-        const int cb = hf * 64 + c * 32;
-        uint32_t r[32];
-        tmem_ld16(acc_addr + cb, *reinterpret_cast<uint32_t(*)[16]>(&r[0]));
-        tmem_ld16(acc_addr + cb + 16, *reinterpret_cast<uint32_t(*)[16]>(&r[16]));
-        tmem_ld_wait();
-        if (c == 1) {                                             // last TMEM read of the item by this thread
-          tc_fence_before();
-          mbar_arrive(sMisc + MISC_ACC_EMPTY + 8 * buf);
-        }
-#pragma unroll
-        for (int q = 0; q < 8; ++q) {
-          uint64_t e0, e1;
-          ld_shared_p2(beta_s + (cb + 4 * q) * 4, e0, e1);
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const uint64_t nrm = add2(pk2u(r[4 * q + 2 * e], r[4 * q + 2 * e + 1]), e ? e1 : e0);
-            float n0, n1;
-            upk2(nrm, n0, n1);
-            uint64_t f = pk2(rsqrt_approx(n0), rsqrt_approx(n1));
-            if (!fwd) f = mul2(f, nrm);
-            uint64_t y = mul2(x2[16 * c + 2 * q + e], f);
-            if (p.rowscale) y = mul2(y, rs2);
-            x2[16 * c + 2 * q + e] = y;
-          }
-        }
-#pragma unroll
-        for (int c8 = 0; c8 < 4; ++c8) {
-          const uint64_t* xx = &x2[16 * c + 4 * c8];
-          st_shared_v4(arow + (((4 * c + c8) ^ (t & 7)) << 4), pack16x2_p(xx[0], f16), pack16x2_p(xx[1], f16),
-                       pack16x2_p(xx[2], f16), pack16x2_p(xx[3], f16));
-        }
-      }
-      fence_proxy_async_smem();
-      named_bar_sync(tbar, 256);
-      const bool valid = team ? it.valid[1] : it.valid[0];
-      if (leader && !nostore && valid) {
-#pragma unroll
-        for (int kb = 0; kb < 2; ++kb)
-          tma_store_5d(&p.tmO, sbuf + kb * STAGE_BLK_BYTES, p.out_coff + v.out_c0 + it.nt * p.n_tile + 64 * kb, tx0, v.out_p2,
-                       ty0, tn);
-        tma_store_commit();
-      }
-    }
-    if (leader) tma_store_wait_all<0>();
   } else if (EPI == EPI_GDN2 && warp >= 4) {
     // ===================== epilogue, two teams (see EPI_GDN2 above) =====================
     // TMEM columns: accumulator of team T at 128 T, its norm at 256 + 128 T.  Team T = items with (n_item & 1) == T.
@@ -664,7 +501,6 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
     const uint32_t bias_s = sMisc + MISC_BIAS, beta_s = sMisc + MISC_BETA;
     const uint32_t gbar = sMisc + (team ? MISC_A2_READY : MISC_GDN_BAR);
     const bool fwd = (p.gdn == MASIC_GDN_FWD);
-    const bool nostore = (p.debug & 4) != 0;
     const uint32_t acc_addr = tmem_base + lane_sel + team * 128;
     const uint32_t nrm_addr = tmem_base + lane_sel + 256 + team * 128;
     const uint32_t arow = sbuf + hf * STAGE_BLK_BYTES + t * 128;
@@ -677,11 +513,6 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
       const Variant& v = p.var[it.var];
       mbar_wait(sMisc + MISC_ACC_FULL + 8 * team, (n_item >> 1) & 1);
       tc_fence_after();
-      if (p.debug & 16) {                         // timing experiment: release the accumulator untouched
-        tc_fence_before();
-        mbar_arrive(sMisc + MISC_ACC_EMPTY + 8 * team);
-        continue;
-      }
       float rs = 1.0f;
       if (p.rowscale) {
         const int y = it.y0[0] + (t >> 3), x = it.x0[0] + (t & 7);
@@ -716,26 +547,24 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
       fence_proxy_async_smem();
       tc_fence_before();
       named_bar_sync(tbar, 256);
-      if (!(p.debug & 8)) {
-        if (hf == 0 && ew == 0) {                                 // one warp of the team; one elected lane issues the 8 MMAs
-          tc_fence_after();
-          if (elect_one()) {
-            const uint32_t d2 = tmem_base + 256 + team * 128;
-            const uint64_t dh = umma_desc_sw128(0);
+      if (hf == 0 && ew == 0) {                                 // one warp of the team; one elected lane issues the 8 MMAs
+        tc_fence_after();
+        if (elect_one()) {
+          const uint32_t d2 = tmem_base + 256 + team * 128;
+          const uint64_t dh = umma_desc_sw128(0);
 #pragma unroll
-            for (int kb = 0; kb < 2; ++kb) {
-              const uint64_t a2 = dh | (((sbuf + kb * STAGE_BLK_BYTES) & 0x3FFFFu) >> 4);
-              const uint64_t g2 = dh | (((sG + kb * STAGE_BLK_BYTES) & 0x3FFFFu) >> 4);
+          for (int kb = 0; kb < 2; ++kb) {
+            const uint64_t a2 = dh | (((sbuf + kb * STAGE_BLK_BYTES) & 0x3FFFFu) >> 4);
+            const uint64_t g2 = dh | (((sG + kb * STAGE_BLK_BYTES) & 0x3FFFFu) >> 4);
 #pragma unroll
-              for (int k = 0; k < 4; ++k) umma_bf16(d2, a2 + 2 * k, g2 + 2 * k, p.idesc_norm, (kb | k) ? 1u : 0u);
-            }
-            umma_commit(gbar);
+            for (int k = 0; k < 4; ++k) umma_bf16(d2, a2 + 2 * k, g2 + 2 * k, p.idesc_norm, (kb | k) ? 1u : 0u);
           }
-          __syncwarp();
+          umma_commit(gbar);
         }
-        mbar_wait(gbar, gpar);
-        gpar ^= 1;
+        __syncwarp();
       }
+      mbar_wait(gbar, gpar);
+      gpar ^= 1;
       tc_fence_after();
       // ---- pass 2: out = (acc + bias) * rsqrt(beta' + norm)   (IGDN: * sqrt); the staging rows re-use the A2 rows
 #pragma unroll
@@ -780,7 +609,7 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
       }
       fence_proxy_async_smem();
       named_bar_sync(tbar, 256);
-      if (leader && !nostore && it.valid[0]) {
+      if (leader && it.valid[0]) {
 #pragma unroll
         for (int kb = 0; kb < 2; ++kb)
           tma_store_5d(&p.tmO, sbuf + kb * STAGE_BLK_BYTES, p.out_coff + v.out_c0 + it.nt * p.n_tile + 64 * kb, it.x0[0],
@@ -809,7 +638,6 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
     uint32_t flip = 0, gdn_par = 0;
     const float* __restrict__ bias_g = p.bias;
     const bool fwd = (p.gdn == MASIC_GDN_FWD);
-    const bool nostore = (p.debug & 4) != 0;
     const int sw = (p.blk_pitch == 128) ? (t & 7) : 0;
     // plain path: a block's 16-channel chunks are split between the pair's two groups (bf16 rows hold up to 4 chunks,
     // fp32 rows 2); a group handles at most two
@@ -830,10 +658,6 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
       const float* __restrict__ bias_t = bias_g ? bias_g + it.nt * p.n_tile : nullptr;
       mbar_wait(sMisc + MISC_ACC_FULL + 8 * buf, (n_item >> 1) & 1);
       tc_fence_after();
-      if (p.debug & 16) {                         // timing experiment: release the accumulators untouched
-        release_acc(buf);
-        continue;
-      }
       if (EPI == EPI_GDN) {
       for (int tt = 0; tt < it.nslots; ++tt) {
         const uint32_t acc_addr = tmem_base + lane_sel + buf * 256 + tt * 128;
@@ -875,7 +699,6 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
           fence_proxy_async_smem();
           tc_fence_before();
           named_bar_sync(3, EPI_THREADS);
-          if (!(p.debug & 8)) {
           if (grp == 0 && ew == 0) {                      // warp-uniform; one elected lane issues the 8 MMAs
             if (CG2) {        // the pair's norm MMA reads both CTAs' A2: tell the leader this CTA's half is in place
               if (elect_one()) mbar_arrive_cluster(leader_bar(sMisc + MISC_A2_READY));
@@ -903,7 +726,6 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
           }
           mbar_wait(sMisc + MISC_GDN_BAR, gdn_par);
           gdn_par ^= 1;
-          }
           tc_fence_after();
           // ---- pass 2: out[:, 32g .. 32g+32) = x * rsqrt(beta + norm)  (IGDN: x * sqrt(.))
           tmem_ld16(acc_addr + cb, *reinterpret_cast<uint32_t(*)[16]>(&r[0]));
@@ -938,7 +760,7 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
           }
           fence_proxy_async_smem();
           named_bar_sync(pbar, 256);
-          if (leader && !nostore && valid) {
+          if (leader && valid) {
             tma_store_5d(&p.tmO, sbuf, p.out_coff + v.out_c0 + it.nt * p.n_tile + 64 * pr, tx0, v.out_p2, ty0,
                          tn);
             tma_store_commit();
@@ -1061,7 +883,7 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
           }
           fence_proxy_async_smem();
           named_bar_sync(pbar, 256);
-          if (leader && !nostore && valid) {
+          if (leader && valid) {
             if (p.blk_img)
               tma_store_5d(&p.tmO, sb2, p.out_coff + v.out_c0 + p.nt_out_c[it.nt], tx0, v.out_p2, ty0, tn * nblk + j);
             else
@@ -1385,8 +1207,8 @@ extern "C" int masic_conv_plan_create(const MasicConvDesc* dp, MasicConvPlan** p
   kp.n_tile = d.n_tile;
   kp.n_ntiles = d.c_out_pad / d.n_tile;
   // CTA pairs (tcgen05 cta_group::2): each CTA stages half of every weight k-block and the pair issues M = 256 MMAs
-  { const char* e = getenv("MASIC_CONV_CG2"); kp.cg2 = e ? (atoi(e) != 0) : (d.cta_pairs != 0); }   // env overrides the plan
-  { const char* e = getenv("MASIC_CONV_PDL"); kp.pdl = e ? (atoi(e) != 0) : (d.pdl != 0); }
+  kp.cg2 = d.cta_pairs != 0;
+  kp.pdl = d.pdl != 0;
   kp.idesc = kp.cg2 ? umma_idesc_bf16_m256(d.n_tile) : umma_idesc_bf16(d.n_tile);
   kp.idesc_norm = kp.idesc;
   kp.f16 = d.f16 != 0;
@@ -1406,11 +1228,6 @@ extern "C" int masic_conv_plan_create(const MasicConvDesc* dp, MasicConvPlan** p
   // EPI_GDN2: fused GDN on a layer whose whole weight set (<= 6 k-blocks of 16 KB: g_a_conv1's five) stays in shared
   // memory next to gamma', four staging blocks and a double-buffered strip ring
   kp.gdn2 = d.gdn && !kp.cg2 && kp.n_var == 1 && kp.var[0].n_bops <= 6;
-  { const char* e = getenv("MASIC_CONV_GDN2"); if (e && atoi(e) == 0) kp.gdn2 = 0; }
-  // EPI_GDNT is built and tested but measured no faster than EPI_GDN (the two teams start on the same ACC_FULL and run in
-  // lock step, so their stalls coincide): opt-in through MASIC_CONV_GDNT=1
-  { const char* e = getenv("MASIC_CONV_GDNT"); kp.gdnt = d.gdn && !kp.cg2 && (e ? atoi(e) != 0 : 0); }
-  if (kp.gdnt) kp.gdn2 = 0;
   if (kp.gdn2) kp.pair = 1;
   kp.n_spatial = kp.tiles_x * kp.tiles_y * kp.n_img;
   kp.n_tiles_total = kp.n_spatial * kp.n_var * kp.n_ntiles;
@@ -1421,21 +1238,16 @@ extern "C" int masic_conv_plan_create(const MasicConvDesc* dp, MasicConvPlan** p
   const int a_stage_bytes = kp.pair * kp.strip_bytes;
   // staging: with GDN two blocks (together the A2 operand of the norm MMA, then the output tile);
   // otherwise two per epilogue group so a block's TMA store drains behind the next block
-  const int n_stage_blk = (d.gdn && !kp.gdn2 && !kp.gdnt) ? 2 : 4;
+  const int n_stage_blk = (d.gdn && !kp.gdn2) ? 2 : 4;
   const int gamma_bytes = d.gdn ? (kp.cg2 ? STAGE_BLK_BYTES : 2 * STAGE_BLK_BYTES) : 0;
   const int fixed = gamma_bytes + n_stage_blk * STAGE_BLK_BYTES + MISC_BYTES + 1024 /*align*/;
-  // MASIC_CONV_SMEM_RESERVE=bytes leaves that much shared memory of the SM unused, so that a CTA of a CUDA-core kernel
-  // (warp, likelihood: other stream, other engine) can be resident beside the persistent conv CTA
-  int reserve = 0;
-  { const char* e = getenv("MASIC_CONV_SMEM_RESERVE"); if (e && atoi(e) > 0 && atoi(e) <= 96 * 1024) reserve = atoi(e); }
-  const int budget = 227 * 1024 - fixed - reserve;            // ring bytes
+  const int budget = 227 * 1024 - fixed;                      // ring bytes
   int sa = 2, sb = 2;
   // resident weights: single program, single n-tile, and the whole k-block list fits next to a double-buffered A ring
   const int n_bops0 = kp.var[0].n_bops;
   kp.b_resident = !kp.cg2 && kp.n_var == 1 && kp.n_ntiles == 1 && (d.n_tile <= 64 || kp.gdn2) &&
                   2 * a_stage_bytes + n_bops0 * kp.b_stage_bytes <= budget;
   if (kp.gdn2 && !kp.b_resident) { delete pl; return MASIC_EINVAL; }
-  { const char* e = getenv("MASIC_CONV_BRES"); if (e && atoi(e) == 0) kp.b_resident = 0; }
   if (kp.b_resident) sb = n_bops0;
   if (sa * a_stage_bytes + sb * kp.b_stage_bytes > budget) { delete pl; return MASIC_EINVAL; }
   // deepen the rings with what is left (B first: a B stage is consumed by a single tap)
@@ -1443,12 +1255,6 @@ extern "C" int masic_conv_plan_create(const MasicConvDesc* dp, MasicConvPlan** p
     grew = false;
     if (!kp.b_resident && sb < MAX_STAGES && sb < 6 && sa * a_stage_bytes + (sb + 1) * kp.b_stage_bytes <= budget) { ++sb; grew = true; }
     if (sa < 4 && (sa + 1) * a_stage_bytes + sb * kp.b_stage_bytes <= budget) { ++sa; grew = true; }
-  }
-  {   // experiments: MASIC_CONV_STAGES="sa,sb" caps the ring depths
-    const char* e = getenv("MASIC_CONV_STAGES");
-    int ea = 0, eb = 0;
-    if (!kp.b_resident && e && sscanf(e, "%d,%d", &ea, &eb) == 2 && ea >= 2 && eb >= 2 && ea <= MAX_STAGES && eb <= MAX_STAGES &&
-        ea * a_stage_bytes + eb * kp.b_stage_bytes <= budget) { sa = ea; sb = eb; }
   }
   kp.a_stages = sa; kp.b_stages = sb;
   kp.smem_b_off = sa * a_stage_bytes;
@@ -1506,13 +1312,11 @@ extern "C" int masic_conv_plan_create(const MasicConvDesc* dp, MasicConvPlan** p
     kp.res0 = static_cast<const __nv_bfloat16*>(d.residual0); kp.res0_pitch = d.res0_cpitch; kp.res0_coff = d.res0_coff;
     kp.res1 = static_cast<const __nv_bfloat16*>(d.residual1); kp.res1_pitch = d.res1_cpitch; kp.res1_coff = d.res1_coff;
   } else if (d.residual1) { delete pl; return MASIC_EINVAL; }
-  { const char* e = getenv("MASIC_CONV_DEBUG"); kp.debug = e ? atoi(e) : 0; }
   pl->total_work = kp.n_tiles_total;
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   pl->grid = pl->total_work < sms ? pl->total_work : sms;
-  { const char* e = getenv("MASIC_CONV_GRID"); if (e && atoi(e) > 0 && atoi(e) < pl->grid) pl->grid = atoi(e); }
   if (kp.cg2) {          // one work range per CTA pair; a pair handles at least two tiles at a time
     int pairs = (pl->total_work + 1) / 2;
     if (pairs > pl->grid / 2) pairs = pl->grid / 2;
@@ -1540,11 +1344,11 @@ extern "C" int masic_conv_plan_create(const MasicConvDesc* dp, MasicConvPlan** p
   static bool attr_set = false;
   if (!attr_set) {
 #define MASIC_K2(C, E) (const void*)conv_tc_kernel<C, E, false>, (const void*)conv_tc_kernel<C, E, true>
-    const void* fns[16] = {MASIC_K2(false, EPI_PLAIN), MASIC_K2(false, EPI_GDN), MASIC_K2(false, EPI_RES),
+    const void* fns[14] = {MASIC_K2(false, EPI_PLAIN), MASIC_K2(false, EPI_GDN), MASIC_K2(false, EPI_RES),
                            MASIC_K2(true, EPI_PLAIN),  MASIC_K2(true, EPI_GDN),  MASIC_K2(true, EPI_RES),
-                           MASIC_K2(false, EPI_GDN2),  MASIC_K2(false, EPI_GDNT)};
+                           MASIC_K2(false, EPI_GDN2)};
 #undef MASIC_K2
-    for (int i = 0; i < 16 && ce == cudaSuccess; ++i)
+    for (int i = 0; i < 14 && ce == cudaSuccess; ++i)
       ce = cudaFuncSetAttribute(fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (ce != cudaSuccess) { delete pl; return (int)ce; }
     attr_set = true;
@@ -1574,7 +1378,7 @@ extern "C" int masic_conv_plan_launch(const MasicConvPlan* pl, void* stream) {
     ++na;
   }
   cfg.attrs = attr; cfg.numAttrs = na;
-  const int epi = pl->kp.gdn ? (pl->kp.gdnt ? EPI_GDNT : (pl->kp.gdn2 ? EPI_GDN2 : EPI_GDN)) : (pl->kp.res0 ? EPI_RES : EPI_PLAIN);
+  const int epi = pl->kp.gdn ? (pl->kp.gdn2 ? EPI_GDN2 : EPI_GDN) : (pl->kp.res0 ? EPI_RES : EPI_PLAIN);
   const bool f16 = pl->kp.f16 != 0;
 #define MASIC_LAUNCH(C, E) \
   return f16 ? (int)cudaLaunchKernelEx(&cfg, conv_tc_kernel<C, E, true>, pl->kp) \
@@ -1584,7 +1388,6 @@ extern "C" int masic_conv_plan_launch(const MasicConvPlan* pl, void* stream) {
     if (epi == EPI_RES) { MASIC_LAUNCH(true, EPI_RES); }
     MASIC_LAUNCH(true, EPI_PLAIN);
   }
-  if (epi == EPI_GDNT) { MASIC_LAUNCH(false, EPI_GDNT); }
   if (epi == EPI_GDN2) { MASIC_LAUNCH(false, EPI_GDN2); }
   if (epi == EPI_GDN) { MASIC_LAUNCH(false, EPI_GDN); }
   if (epi == EPI_RES) { MASIC_LAUNCH(false, EPI_RES); }

@@ -11,7 +11,6 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 #include "../../include/masic_b200.h"
 #include "cvt16.cuh"
@@ -856,11 +855,10 @@ extern "C" int masic_warp_perspective_fwd3(const float* src, int n, int c, int h
   if (h_out < 2 || w_out < 2) return MASIC_ENOSUP;
   if ((long)h * w >= (1L << 31)) return MASIC_ENOSUP;
   // the engine's configurations: 3- or 1-channel images, 16-bit copies (if any) as fp16 hi|lo pixels of pitch 8 and
-  // as the aligned plain-fp16 half of a shared 8-channel pixel (MASIC_WARP_FAST=0: the generic kernel)
-  static const bool fast_ok = []() { const char* e = getenv("MASIC_WARP_FAST"); return !(e && atoi(e) == 0); }();
+  // as the aligned plain-fp16 half of a shared 8-channel pixel
   const bool fmt16_ok = !dst_nhwc_bf16 || (c == 3 && bf_pitch == 8 && f16 == (MASIC_FMT_F16 | MASIC_FMT_SPLIT));
   const bool fmt2_ok = !dst2_nhwc16 || (c == 3 && d2_pitch == 8 && (d2_coff & 3) == 0 && (d2_f16 & 1) == 1);
-  if (fast_ok && (c == 3 || c == 1) && fmt16_ok && fmt2_ok && (long)n * c * h * w < (1L << 40)) {
+  if ((c == 3 || c == 1) && fmt16_ok && fmt2_ok && (long)n * c * h * w < (1L << 40)) {
     dim3 fgrid((w_out + WF_BLK * WF_PPT - 1) / (WF_BLK * WF_PPT), h_out, n);
     auto fk = c == 3 ? warp_fast_kernel<3> : warp_fast_kernel<1>;
     fk<<<fgrid, WF_BLK, 0, static_cast<cudaStream_t>(stream)>>>(

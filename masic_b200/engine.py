@@ -20,14 +20,13 @@ The engine is built for a fixed (batch, H, W); H and W must be multiples of 64
 from __future__ import annotations
 
 import ctypes as C
-import os
 from typing import Callable, Dict, List, Optional, Tuple
 
 import torch
 
 from . import _lib
 from ._lib import MasicError, check
-from .convplan import (ACT_LEAKY, ACT_NONE, ACT_RELU, CONV, CONV_XFOLD8, DECONV_S2, DECONV_S2_SUBPIX, GDN_FWD, GDN_INV,
+from .convplan import (ACT_LEAKY, ACT_NONE, ACT_RELU, CONV, CONV_XFOLD8, DECONV_S2, GDN_FWD, GDN_INV,
                        GDN_NONE, MASK_A_5x5, ConvPlan, DeconvImgPlan, PackedConv, fold8_weights_5x5_s1)
 
 F16 = _lib.FMT_F16              # the inference engines run on fp16 operands / activations (csrc/cvt16.cuh)
@@ -73,9 +72,6 @@ class HSICEngine:
         return self.sd[name].float().contiguous()
 
     def _add(self, name: str, fn: Callable[[], None]):
-        skip = os.environ.get("MASIC_ENGINE_SKIP")     # timing experiments only (results are wrong): drop matching steps
-        if skip and any(t and t in name for t in skip.split(",")):
-            fn = lambda: None
         self.steps.append((name, fn))
         self.sched.append(("run", len(self.steps) - 1, self._lane))
 
@@ -143,7 +139,6 @@ class HSICEngine:
     def _decoder(self, tag: str, dec: str, yq_bf16, out_img, igdn_prefix=None, out16=None):
         """g_s: 3x (deconv5 s2 + IGDN) + deconv5 s2 -> 3 — MASIC.py:544-554.  The last layer runs in col2im form
         (csrc/deconv_img.cu) and writes the NCHW fp32 image `out_img`, with after_gdn fused for the right view."""
-        import os
         B, H, W, N, M = self.B, self.H, self.W, self.N, self.M
         g1 = self._buf(B, H // 8, W // 8, N)
         g2 = self._buf(B, H // 4, W // 4, N)
@@ -159,21 +154,10 @@ class HSICEngine:
         self._conv(f"{tag}.deconv3+igdn", p3, g2, g3)
         ib = self._w(igdn_prefix + ".beta") if igdn_prefix else None
         ig = self._w(igdn_prefix + ".gamma") if igdn_prefix else None
-        if os.environ.get("MASIC_DECONV_IMG", "1") != "0":
-            plan = DeconvImgPlan(x=g3, weight=self._w(f"{dec}.g_s_conv4.weight"), bias=self._w(f"{dec}.g_s_conv4.bias"),
-                                 out=out_img, igdn_beta=ib, igdn_gamma=ig, out16=out16, out16_coff=0, out16_xoff=XOFF)
-            self.plans[f"{tag}.deconv4(col2im)"] = plan
-            self._add(f"{tag}.deconv4(col2im)", plan.launch)
-            return
-        assert out16 is None, "the 16-bit NHWC copy of the decoder output needs the col2im deconv (MASIC_DECONV_IMG=1)"
-        # the earlier form (MASIC_DECONV_IMG=0): sub-pixel conv_tc plan (N = 4 phases x 3 -> 16) + pixel interleave
-        sp = self._buf(B, H // 2, W // 2, 16, dtype=torch.float32)
-        p4 = self._pack(f"{dec}.g_s_conv4", kind=DECONV_S2_SUBPIX, c_in=N, c_out=3, n_tile=16, transposed=True)
-        self._conv(f"{tag}.deconv4(subpix)", p4, g3, sp)
-        self._keep += [ib, ig]
-        self._add(f"{tag}.unshuffle", lambda: check(self.lib.masic_subpix_to_nchw(
-            sp.data_ptr(), B, H // 2, W // 2, 16, GDN_INV if igdn_prefix else 0, None if ib is None else ib.data_ptr(),
-            None if ig is None else ig.data_ptr(), 1e-6, out_img.data_ptr(), None, 0, F16, self._s()), "masic_subpix_to_nchw"))
+        plan = DeconvImgPlan(x=g3, weight=self._w(f"{dec}.g_s_conv4.weight"), bias=self._w(f"{dec}.g_s_conv4.bias"),
+                             out=out_img, igdn_beta=ib, igdn_gamma=ig, out16=out16, out16_coff=0, out16_xoff=XOFF)
+        self.plans[f"{tag}.deconv4(col2im)"] = plan
+        self._add(f"{tag}.deconv4(col2im)", plan.launch)
 
     def _hyper(self, tag: str, idx: int, y_abs_bf16, gmm_in, rowscale=None):
         """h_a -> EntropyBottleneck -> h_s_up (MASIC.py:747-754 / :786-793).  Writes params into
@@ -263,8 +247,7 @@ class HSICEngine:
         p1 = PackedConv(ksize=1, c_in=6 * M, c_out=13 * M, n_tile=192, weight=w1, bias=b1, f16=F16)
         self.packs[f"{tag}.gmm.l1(3 branches)"] = p1            # the wave decoder runs the same grouped launches
         plan = ConvPlan(packed=p1, x=l0, out=l1, act=[ACT_RELU] * nt(4 * M) + [ACT_LEAKY] * nt(9 * M),
-                        nt_in_coff=[0] * nt(4 * M) + [6 * M] * nt(4 * M) + [12 * M] * nt(5 * M),
-                        cta_pairs=os.environ.get("MASIC_GMM_L1_CG2", "0") != "0")
+                        nt_in_coff=[0] * nt(4 * M) + [6 * M] * nt(4 * M) + [12 * M] * nt(5 * M))
         self.plans[f"{tag}.gmm.l1(3 branches)"] = plan
         self._add(f"{tag}.gmm.l1(3 branches)", plan.launch)
         smw = self._buf(3 * B, h16, w16, MK, dtype=torch.float32)     # sigma | mu | weight logits, each dense [B][P][MK]
@@ -276,12 +259,10 @@ class HSICEngine:
         tiles = list(range(0, MK, 192))
         plan = ConvPlan(packed=p2, x=l1, out=smw, act=[ACT_RELU] * nt(MK) + [ACT_NONE] * nt(MK),
                         nt_in_coff=[0] * nt(MK) + [4 * M] * nt(MK), nt_out_coff=tiles + tiles,
-                        nt_out_img=[0] * nt(MK) + [B] * nt(MK),
-                        cta_pairs=os.environ.get("MASIC_GMM_L2_CG2", "0") != "0")
+                        nt_out_img=[0] * nt(MK) + [B] * nt(MK))
         self.plans[f"{tag}.gmm.l2(sigma|means)"] = plan
         self._add(f"{tag}.gmm.l2(sigma|means)", plan.launch)
-        self._conv(f"{tag}.gmm.weights.l2", self.packs[f"{tag}.gmm.weights.l2"], l1, wl, in_coff=8 * M,
-                   cta_pairs=os.environ.get("MASIC_GMM_L2_CG2", "0") != "0")
+        self._conv(f"{tag}.gmm.weights.l2", self.packs[f"{tag}.gmm.weights.l2"], l1, wl, in_coff=8 * M)
         self.buf[f"{tag}.sigma"], self.buf[f"{tag}.mu"], self.buf[f"{tag}.wlogit"] = sig, mu, wl
         return sig, mu, wl
 
@@ -331,7 +312,7 @@ class HSICEngine:
                   "masic_warp_perspective_fwd3")
         self._add(tag, step)
 
-    def _conv_small(self, tag, in0, in1, wname, *, ksize, stride, transposed_s1=False, act=ACT_NONE, gdn=GDN_NONE,
+    def _conv_small(self, tag, in0, in1, wname, *, ksize, stride, act=ACT_NONE, gdn=GDN_NONE,
                     gdn_prefix=None, out=None, out_bf=None):
         w = self._w(wname + ".weight")
         b = self._w(wname + ".bias")
@@ -340,11 +321,11 @@ class HSICEngine:
         self._keep += [w, b, beta, gamma]
         n, c0, h, wd = in0.shape
         c1 = 0 if in1 is None else in1.shape[1]
-        c_out = w.shape[1] if transposed_s1 else w.shape[0]
+        c_out = w.shape[0]
 
         def step():
             check(self.lib.masic_conv_small_nchw(in0.data_ptr(), c0, None if in1 is None else in1.data_ptr(), c1, n, h,
-                                                 wd, w.data_ptr(), int(transposed_s1), b.data_ptr(), c_out, ksize,
+                                                 wd, w.data_ptr(), 0, b.data_ptr(), c_out, ksize,
                                                  stride, act, gdn, None if beta is None else beta.data_ptr(),
                                                  None if gamma is None else gamma.data_ptr(), 1e-6,
                                                  None if out is None else out.data_ptr(),
@@ -395,38 +376,20 @@ class HSICEngine:
             check(lib.masic_warp_prepare(self.Hm.data_ptr(), B, H, W, H, W, 1, Tinv.data_ptr(), self._s()), "masic_warp_prepare")))
         self._record("T")
         # x1 and the all-ones image are warped by ONE launch (same transform: the fp64 coordinates, ~60 % of the kernel's
-        # instructions, are evaluated once); MASIC_WARP_MASK_FUSED=0 keeps the two launches
+        # instructions, are evaluated once)
         x1_warp = self._buf(B, 3, H, W, dtype=f32)
-        mask_fused = os.environ.get("MASIC_WARP_MASK_FUSED", "1") != "0"
-        if mask_fused:
-            self._warp("R.warp(x1)+mask_R", self.x1, T, x1_warp, ones=o["x1_mask_R"])
-        else:
-            self._warp("mask_R=warp(ones)", None, T, o["x1_mask_R"], channels=1)
+        self._warp("R.warp(x1)+mask_R", self.x1, T, x1_warp, ones=o["x1_mask_R"])
         self._warp("mask_L=warp(mask_R,Hinv)", o["x1_mask_R"], Tinv, o["x1_mask_L"], channels=1)
         # mask2weights: 4x (conv3 s2 [+ReLU]) + softmax over 3 (MASIC.py:472-506)
         mk = "mask2weights_unit.maskconv"
         mw = self._buf(B, h16, w16, 3, dtype=f32)        # per-pixel fusion weights, NHWC
         self.mask_weights = mw
-        if os.environ.get("MASIC_MASK2W_FUSED", "1") != "0":
-            mp = [self._w(f"{mk}.{i}.{t}") for i in (0, 2, 4, 6) for t in ("weight", "bias")]
-            self._keep += mp
-            self._add("mask2weights(fused)", lambda: check(lib.masic_mask2weights(
-                o["x1_mask_R"].data_ptr(), B, H, W, *[t.data_ptr() for t in mp], None, mw.data_ptr(), self._s()),
-                "masic_mask2weights"))
-        else:
-            k1 = self._buf(B, 3, H // 2, W // 2, dtype=f32)
-            k2 = self._buf(B, 6, H // 4, W // 4, dtype=f32)
-            k3 = self._buf(B, 6, H // 8, W // 8, dtype=f32)
-            k4 = self._buf(B, 3, h16, w16, dtype=f32)
-            self._conv_small("mask2weights.conv1", o["x1_mask_R"], None, f"{mk}.0", ksize=3, stride=2, act=ACT_RELU, out=k1)
-            self._conv_small("mask2weights.conv2", k1, None, f"{mk}.2", ksize=3, stride=2, act=ACT_RELU, out=k2)
-            self._conv_small("mask2weights.conv3", k2, None, f"{mk}.4", ksize=3, stride=2, act=ACT_RELU, out=k3)
-            self._conv_small("mask2weights.conv4", k3, None, f"{mk}.6", ksize=3, stride=2, out=k4)
-            self._add("mask2weights.softmax", lambda: check(lib.masic_softmax_channels(
-                k4.data_ptr(), B, 3, h16 * w16, None, mw.data_ptr(), self._s()), "masic_softmax_channels"))
+        mp = [self._w(f"{mk}.{i}.{t}") for i in (0, 2, 4, 6) for t in ("weight", "bias")]
+        self._keep += mp
+        self._add("mask2weights(fused)", lambda: check(lib.masic_mask2weights(
+            o["x1_mask_R"].data_ptr(), B, H, W, *[t.data_ptr() for t in mp], None, mw.data_ptr(), self._s()),
+            "masic_mask2weights"))
         self._record("mw")
-        if not mask_fused:
-            self._warp("R.warp(x1)", self.x1, T, x1_warp)
         x2in_bf = self._buf(B, H, W + XPAD, IMG_CP)
         self._conv_small("R.pre_conv+pre_gdn", x1_warp, self.x2, "encoder2.pre_conv", ksize=5, stride=1, gdn=GDN_FWD,
                          gdn_prefix="encoder2.pre_gdn", out_bf=x2in_bf)
@@ -463,38 +426,28 @@ class HSICEngine:
         self._decoder("L.g_s", "decoder1", y1_rnd, o["x1_hat"])                                    # :777
         # x1_hat warped once (the reference computes it twice, :821 and :833)
         x1hw_bf = self._buf(B, H, W + XPAD, IMG_CP)
-        # after_conv on the tensor cores (MASIC_AFTER_CONV_TC=0: the CUDA-core kernel on fp32 planes): its two inputs
-        # are written straight into ONE channels-last 16-bit image [after_gdn(g_s(y2_hat)) (3) 0 | x1_hat_warp (3) 0],
-        # each producer with one aligned 8-byte store per pixel
-        ac_tc = (os.environ.get("MASIC_AFTER_CONV_TC", "1") != "0" and os.environ.get("MASIC_DECONV_IMG", "1") != "0"
-                 and W % 8 == 0)
-        ac_in = self._buf(B, H, W + XPAD, IMG_CP) if ac_tc else None
-        x1hw = None if ac_tc else self._buf(B, 3, H, W, dtype=f32)
+        # after_conv on the tensor cores: its two inputs are written straight into ONE channels-last 16-bit image
+        # [after_gdn(g_s(y2_hat)) (3) 0 | x1_hat_warp (3) 0], each producer with one aligned 8-byte store per pixel
+        ac_in = self._buf(B, H, W + XPAD, IMG_CP)
         self._wait("T")
-        self._warp("R.warp(x1_hat)", o["x1_hat"], T, x1hw, x1hw_bf, dst2=ac_in, dst2_coff=4)
+        self._warp("R.warp(x1_hat)", o["x1_hat"], T, None, x1hw_bf, dst2=ac_in, dst2_coff=4)
         y1w = self._encoder("R.g_a(enc1 on warped x1_hat)", enc1, x1hw_bf)                         # :822
         self._wait("mw")
         self._wait("right")
         self._latent_prep("R.y1warp", y1w, None, gmm2_in, rnd_coff=4 * M, rowscale=mw, rs_off=2)   # round(.) * w2
         s2, m2, w2 = self._gmm_net("R", "_h_s2_same_resolution", 5 * M, False, gmm2_in)            # :827
         self._gmm_likelihood("R", y2, s2, m2, w2, o["y2_hat"], o["lik_y2"])                        # :829
-        if ac_tc:
-            self._decoder("R.g_s", "decoder2", y2_rnd, None, igdn_prefix="decoder2.after_gdn", out16=ac_in)   # :834, :615
-            wf, bf_, tmask = fold8_weights_5x5_s1(self._w("decoder2.after_conv.weight"), self._w("decoder2.after_conv.bias"),
-                                                  transposed=True, slots=(0, 1, 2, 4, 5, 6))
-            pk = PackedConv(ksize=5, c_in=64, c_out=48, n_tile=48, weight=wf, bias=bf_, f16=F16)
-            self.packs["R.after_conv"] = pk
-            plan = ConvPlan(packed=pk, x=ac_in.view(B, H, (W + XPAD) // 8, 64), stride=1, tap_mask=tmask, w_in=W // 8,
-                            out=o["x2_hat"].view(B * 3, H, W // 8, 8), out_blk_images=True)
-            plan.flops = 2.0 * B * H * W * 6 * 3 * 25         # useful work (the folded GEMM multiplies mostly zeros)
-            plan.hbm_bytes = B * H * W * (16.0 + 12.0)
-            self.plans["R.after_conv"] = plan
-            self._add("R.after_conv", plan.launch)
-        else:
-            after1 = self._buf(B, 3, H, W, dtype=f32)
-            self._decoder("R.g_s", "decoder2", y2_rnd, after1, igdn_prefix="decoder2.after_gdn")        # :834, :615
-            self._conv_small("R.after_conv", after1, x1hw, "decoder2.after_conv", ksize=5, stride=1, transposed_s1=True,
-                             out=o["x2_hat"])
+        self._decoder("R.g_s", "decoder2", y2_rnd, None, igdn_prefix="decoder2.after_gdn", out16=ac_in)   # :834, :615
+        wf, bf_, tmask = fold8_weights_5x5_s1(self._w("decoder2.after_conv.weight"), self._w("decoder2.after_conv.bias"),
+                                              transposed=True, slots=(0, 1, 2, 4, 5, 6))
+        pk = PackedConv(ksize=5, c_in=64, c_out=48, n_tile=48, weight=wf, bias=bf_, f16=F16)
+        self.packs["R.after_conv"] = pk
+        plan = ConvPlan(packed=pk, x=ac_in.view(B, H, (W + XPAD) // 8, 64), stride=1, tap_mask=tmask, w_in=W // 8,
+                        out=o["x2_hat"].view(B * 3, H, W // 8, 8), out_blk_images=True)
+        plan.flops = 2.0 * B * H * W * 6 * 3 * 25         # useful work (the folded GEMM multiplies mostly zeros)
+        plan.hbm_bytes = B * H * W * (16.0 + 12.0)
+        self.plans["R.after_conv"] = plan
+        self._add("R.after_conv", plan.launch)
         self._wait("left_entropy")
         self.flops = sum(p.flops for p in self.plans.values())
 

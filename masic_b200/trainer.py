@@ -30,7 +30,6 @@ No CPU fallback: everything raises on non-CUDA tensors.
 from __future__ import annotations
 
 import ctypes as C
-import os
 from typing import Callable, Dict, List, Optional, Tuple
 
 import torch
@@ -90,9 +89,7 @@ class _Layer:
             tr.repack.append((self.pack, self.w, self.b))
         # CTA pairs where they measured faster in the inference engine: the 128 -> 128 5x5 stride-2 layers (and their
         # data gradients, which are the same operator transposed) and the wide 1x1 / 3x3 / masked layers
-        import os
-        pairs = os.environ.get("MASIC_TRAIN_PAIRS", "1") == "1" and (
-            (k == 5 and stride == 2 and c_in == 128 and c_out == 128 and not transposed) or (k == 1 and c_out >= 3000))
+        pairs = (k == 5 and stride == 2 and c_in == 128 and c_out == 128 and not transposed) or (k == 1 and c_out >= 3000)
         self.fwd_plan = ConvPlan(packed=self.pack, stride=stride, tap_mask=tap_mask, x=x, in_coff=in_coff, out=out,
                                  out_coff=out_coff, act=act, cta_pairs=pairs)
         # ---- weight gradient: conv: LO = dL/dout, HI = input; deconv: LO = input, HI = dL/dout
@@ -237,13 +234,9 @@ class _GDN3:
 
 
 class HSICTrainer:
-    EARLY_MODULES = frozenset(("entropy_bottleneck2", "encoder2", "decoder2", "decoder1", "_h_a2", "h_s2_up",
-                               "context_prediction2", "_h_s2_same_resolution", "mask2weights_unit"))
-
     def __init__(self, model, batch: int, height: int, width: int, device, lmbda: float = 0.01,
                  use_graph: bool = True):
         self.use_graph, self.graph, self._warm = use_graph, None, False
-        self.graph_a = self.graph_b = None
         if height % 64 or width % 64:
             raise ValueError("HSIC needs H and W to be multiples of 64")
         self.lib = _lib.load()
@@ -261,17 +254,12 @@ class HSICTrainer:
         total = sum(p.numel() for p in self._params.values())
         self.flat_grad = torch.zeros(total, device=self.dev)
         self._grads: Dict[str, torch.Tensor] = {}
-        # Layout of the flat gradient buffer: the modules whose gradients are FINAL two thirds of the way through the
-        # backward pass (the right view's own transforms and nets, both decoders) come first, so that their mean over the
-        # ranks is ONE all-reduce of a contiguous prefix that overlaps the rest of the backward pass (train_step).
+        # Layout of the flat gradient buffer: the parameters in named_parameters() order, each gradient a view of its
+        # slice, so that the data-parallel mean over the ranks is ONE all-reduce of the whole buffer (train_step).
         off = 0
-        for early in (True, False):
-            for n, p in self._params.items():
-                if (n.split(".")[0] in self.EARLY_MODULES) == early:
-                    self._grads[n] = self.flat_grad[off:off + p.numel()].view(p.shape)
-                    off += p.numel()
-            if early:
-                self.n_early = off
+        for n, p in self._params.items():
+            self._grads[n] = self.flat_grad[off:off + p.numel()].view(p.shape)
+            off += p.numel()
         self.repack: List[Tuple[PackedConv, torch.Tensor, Optional[torch.Tensor]]] = []
         self._pack_batch = None
         self.gdn_prep: List[_GDN] = []
@@ -280,10 +268,8 @@ class HSICTrainer:
         self.fwd_ops: List[Tuple[str, Callable[[], None]]] = []
         self.bwd_ops: List[Tuple[str, Callable[[], None]]] = []
         self.flops_fwd = 0.0
-        self.wg_overlap = os.environ.get("MASIC_TRAIN_WG_STREAM", "1") != "0"
-        self.lanes = os.environ.get("MASIC_TRAIN_LANES", "1") != "0"
         with torch.cuda.device(self.dev):
-            self._wg_stream = torch.cuda.Stream(device=self.dev) if self.wg_overlap else None
+            self._wg_stream = torch.cuda.Stream(device=self.dev)
             self._lane_streams: List[torch.cuda.Stream] = []
             self._build()
 
@@ -310,9 +296,6 @@ class HSICTrainer:
     # extending it.  All of them share ONE side stream: they also share one partial-sum workspace.  Every operand
     # buffer of the step is allocated once and never reused, so the fork event is the only ordering they need.
     def wg_async(self, fn):
-        if not self.wg_overlap:
-            fn()
-            return
         ev = torch.cuda.Event()
         ev.record()
         self._wg_stream.wait_event(ev)
@@ -320,10 +303,9 @@ class HSICTrainer:
             fn()
 
     def wg_join(self):
-        if self.wg_overlap:
-            ev = torch.cuda.Event()
-            ev.record(self._wg_stream)
-            torch.cuda.current_stream().wait_event(ev)
+        ev = torch.cuda.Event()
+        ev.record(self._wg_stream)
+        torch.cuda.current_stream().wait_event(ev)
 
     # ------------------------------------------------------------------ sub-graphs
     def _encoder_pass(self, tag: str, enc: str, img_bf: torch.Tensor, img_nchw: torch.Tensor, accumulate: bool,
@@ -507,7 +489,7 @@ class HSICTrainer:
                 sl = slice(6 * M * i, 6 * M * (i + 1))
                 self.grad(f"{net}.{b}.0.weight").copy_(dw0[:, sl] if t else dw0[sl])
                 self.grad(f"{net}.{b}.0.bias").copy_(db0[sl])
-        self.post_bwd.append((net, scatter))
+        self.post_bwd.append(scatter)
         l1, gl1 = self._z(B, h16, w16, 8 * M), self._z(B, h16, w16, 8 * M)
         l1w, gl1w = self._z(B, h16, w16, MK), self._z(B, h16, w16, MK)
         sig, mu, wl = (self._z(B, h16, w16, MK, dtype=F32) for _ in range(3))
@@ -545,7 +527,7 @@ class HSICTrainer:
         lib = self.lib
         dev = self.dev
         self.pre_repack: List[Callable[[], None]] = []
-        self.post_bwd: List[Tuple[str, Callable[[], None]]] = []
+        self.post_bwd: List[Callable[[], None]] = []
         self.noise = {k: self._z(B, (h16 // 4) if k.startswith("z") else h16, (w16 // 4) if k.startswith("z") else w16,
                                  N if k.startswith("z") else M, dtype=F32) for k in NOISE_KEYS}     # NHWC
         self.x1 = self._z(B, 3, H, W, dtype=F32)
@@ -760,25 +742,11 @@ class HSICTrainer:
         self.Bk("L.latent_merge", lambda: T.latent_merge_bwd(y1, dy1_lik, g_y1hat, g_y1ctx, g_y1abs, gy1))
         self.Bk("L.encoder", encA["bwd"])
         # the 2 x 15 reparam backwards of the fused-GDN layers as one launch
-        # ... in two batches: the layers of the early-final modules (flat-buffer prefix) and the rest
-        def rp(early):
-            return T.ReparamBatch([j for g in self.gdn_finish if (g.name.split(".")[0] in self.EARLY_MODULES) == early
-                                   for j in ((g.dbeta_p, g.beta, 1e-6, g.dbeta), (g.dgamma_p, g.gamma, 0.0, g.dgamma))])
-        self._reparam0, self._reparam1 = rp(True), rp(False)
-        sc0 = [f for net_name, f in self.post_bwd if net_name.split(".")[0] in self.EARLY_MODULES]
-        sc1 = [f for net_name, f in self.post_bwd if net_name.split(".")[0] not in self.EARLY_MODULES]
+        self._reparam = T.ReparamBatch([j for g in self.gdn_finish for j in ((g.dbeta_p, g.beta, 1e-6, g.dbeta),
+                                                                             (g.dgamma_p, g.gamma, 0.0, g.dgamma))])
         self.Bk("wgrad.join", self.wg_join)
-        self.Bk("gdn.reparam", lambda: (self._reparam0.launch(), self._reparam1.launch()))
-        self.Bk("scatter", lambda: [f() for f in sc0 + sc1])
-        # Split form of the same backward pass for data-parallel runs (train_step): part A ends after L.decoder with the
-        # streams joined and the early-final gradients complete, part B is the rest.
-        names = [n for n, _ in self.bwd_ops]
-        cut = names.index("L.decoder") + 1
-        end = names.index("wgrad.join")
-        self.bwd_ops_a = self.bwd_ops[:cut] + [("wgrad.join", self.wg_join), ("gdn.reparam", self._reparam0.launch),
-                                               ("scatter", lambda: [f() for f in sc0])]
-        self.bwd_ops_b = self.bwd_ops[cut:end] + [("wgrad.join", self.wg_join), ("gdn.reparam", self._reparam1.launch),
-                                                  ("scatter", lambda: [f() for f in sc1])]
+        self.Bk("gdn.reparam", self._reparam.launch)
+        self.Bk("scatter", lambda: [f() for f in self.post_bwd])
         # hyper-synthesis conv3x3 of the LEFT view writes / reads channel slice [0, 2M) of the 4M-wide gmm1_in; its
         # gradient arrives in g_gmm1_in[..., 0:2M] (written by net1's layer-0 dgrad) — same layout, nothing to do.
 
@@ -840,37 +808,6 @@ class HSICTrainer:
             else:
                 self.noise[k].copy_(noise[k].permute(0, 2, 3, 1))
 
-    @torch.no_grad()
-    def _step_grads_bucketed(self, x1, x2, h_matrix, noise, reduce_fn):
-        """The data-parallel form of step_grads: the step as TWO CUDA graphs.  After graph A (forward + the backward pass
-        up to L.decoder) the gradients of the early-final modules — the first `n_early` floats of the flat buffer — are
-        complete: reduce_fn(flat_grad[:n_early]) starts their all-reduce, which runs on NCCL's stream while graph B
-        (the left view's nets, hyperprior and encoder1 backward) runs on this one; the remaining floats are reduced
-        after graph B.  Returns the two work handles."""
-        with torch.cuda.device(self.dev):
-            self._load_inputs(x1, x2, h_matrix, noise)
-            if not self._warm:                           # first call: eager, also warms every plan
-                self._issue(True)
-                self._warm = True
-                h0 = reduce_fn(self.flat_grad[:self.n_early])
-                h1 = reduce_fn(self.flat_grad[self.n_early:])
-            else:
-                if self.graph_a is None:
-                    torch.cuda.synchronize(self.dev)
-                    ga, gb = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(ga):
-                        self._issue(True, "a")
-                    with torch.cuda.graph(gb):
-                        self._issue(True, "b")
-                    self.graph_a, self.graph_b = ga, gb
-                self.graph_a.replay()
-                h0 = reduce_fn(self.flat_grad[:self.n_early])
-                self.graph_b.replay()
-                h1 = reduce_fn(self.flat_grad[self.n_early:])
-            for n, p in self._params.items():
-                p.grad = self._grads[n]
-            return h0, h1
-
     def read_losses(self) -> Dict[str, float]:
         """Loss terms of the last step (one device -> host read; synchronises with the step)."""
         r = torch.cat([self.rd_out, self.aux_out]).tolist()
@@ -893,10 +830,6 @@ class HSICTrainer:
     # joined before L.latent_merge: 8.37 vs 8.28 ms — the lanes already keep the SMs busy)
 
     def _run_lanes(self, ops, lanes):
-        if not self.lanes:
-            for _, fn in ops:
-                fn()
-            return
         main = torch.cuda.current_stream()
         while len(self._lane_streams) < len(lanes):
             self._lane_streams.append(torch.cuda.Stream(device=self.dev))
@@ -931,22 +864,14 @@ class HSICTrainer:
                     fork(i)
         assert len(joined) == len(lanes), "a lane was never joined"
 
-    def _issue(self, refresh: bool, part: Optional[str] = None):
-        """part None: the whole step; 'a': zeroing, re-packs, forward and the backward pass up to L.decoder (streams
-        joined, early-final gradients complete); 'b': the rest of the backward pass."""
-        if part != "b":
-            self.flat_grad.zero_()
-            for t in self.zero_each_step:
-                t.zero_()
-            if refresh:
-                self.refresh_weights()
-            self._run_lanes(self.fwd_ops, self.FWD_LANES)
-        if part is None:
-            self._run_lanes(self.bwd_ops, self.BWD_LANES)
-        elif part == "a":
-            self._run_lanes(self.bwd_ops_a, self.BWD_LANES)
-        else:
-            self._run_lanes(self.bwd_ops_b, ())
+    def _issue(self, refresh: bool):
+        self.flat_grad.zero_()
+        for t in self.zero_each_step:
+            t.zero_()
+        if refresh:
+            self.refresh_weights()
+        self._run_lanes(self.fwd_ops, self.FWD_LANES)
+        self._run_lanes(self.bwd_ops, self.BWD_LANES)
 
     def train_step(self, x1: torch.Tensor, x2: torch.Tensor, h_matrix: torch.Tensor, optimizer, aux_optimizer,
                    noise: Optional[Dict[str, torch.Tensor]] = None, group=None,
@@ -956,25 +881,11 @@ class HSICTrainer:
         `optimizer` holds model.parameters() (everything but the bottlenecks), `aux_optimizer` model.aux_parameters()
         (MASIC.py:77-94).  The gradients live in ONE flat fp32 buffer, so the all-reduce is a single NCCL call over
         NVLink/NVSwitch (35 M floats = 140 MB); nothing else is communicated."""
-        import torch.distributed as dist
         # the loss scalars are read back AFTER the optimisers are enqueued: the host does not wait for the step's graph
         # before it launches the all-reduce and the two Adam steps
         from .sharding import all_reduce_mean_
-        world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
-        nccl = world > 1 and dist.get_backend(group) == "nccl"
-        if nccl and self.use_graph and os.environ.get("MASIC_TRAIN_BUCKETS", "0") != "0":
-            # opt-in (MASIC_TRAIN_BUCKETS=1): two buckets, the early-final half of the gradients averaged while the rest of
-            # the backward pass runs.  Correct (tools/train_bucket_check.py: every rank ends with identical parameters)
-            # but not faster: 8.48 against 8.38 ms per step on two GPUs, 8.69 against 8.58 on eight — splitting the graph
-            # joins the weight-gradient stream and the lane mid-way, and the collective's CTAs compete with persistent
-            # kernels for SMs
-            h0, h1 = self._step_grads_bucketed(x1, x2, h_matrix, noise,
-                                               lambda t: all_reduce_mean_(t, group=group, async_op=True))
-            h0.wait()                                                 # stream-side waits: the host does not block
-            h1.wait()
-        else:
-            self.step_grads(x1, x2, h_matrix, noise=noise, read_back=False)
-            all_reduce_mean_(self.flat_grad, group=group)             # one collective; no-op on a single rank
+        self.step_grads(x1, x2, h_matrix, noise=noise, read_back=False)
+        all_reduce_mean_(self.flat_grad, group=group)                 # one collective; no-op on a single rank
         if clip_max_norm is not None and clip_max_norm > 0:
             # torch.nn.utils.clip_grad_norm_(model.parameters(), clip_max_norm) of CompressAI's training loops, on the
             # flat buffer: the main parameters' gradients (everything but the two bottlenecks, MASIC.py:77-94)

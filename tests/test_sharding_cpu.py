@@ -156,7 +156,7 @@ def _w_mean(rank, world, tmp):
 @pytest.mark.parametrize("world", [2, 3])
 def test_all_reduce_mean_whole_and_split_buffer(world, tmp_path):
     """HSICTrainer.train_step's collective (sharding.all_reduce_mean_): the mean over the ranks, in place, identical
-    whether the flat buffer is reduced at once or as an asynchronous prefix + suffix (MASIC_TRAIN_BUCKETS=1)."""
+    whether the flat buffer is reduced at once or as an asynchronous prefix + suffix."""
     f = str(tmp_path / "m.pt")
     _spawn(_w_mean, world, f)
     want = torch.stack([torch.rand(1000, generator=torch.Generator().manual_seed(40 + r)) for r in range(world)]).mean(0)
