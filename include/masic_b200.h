@@ -138,6 +138,11 @@ typedef struct MasicConvPlan MasicConvPlan;   /* opaque: tensor maps + tile prog
 int masic_conv_plan_create(const MasicConvDesc* desc, MasicConvPlan** plan_out);
 int masic_conv_plan_launch(const MasicConvPlan* plan, void* stream);
 void masic_conv_plan_destroy(MasicConvPlan* plan);
+/* Training (CQE ResidualBlock backward): a plan with residual0 also stores act(conv + bias), before the residual adds,
+ * to channel coff + c of the bf16 NHWC buffer act_out (cpitch, coff multiples of 8; same spatial size as the output).
+ * The plan's own output is unchanged.  bf16 plans with a 16-bit output and no rowscale only; MASIC_ENOSUP on CTA
+ * pairs, fp16, PDL or planar output.  Plans that never call this launch exactly as before. */
+int masic_conv_plan_set_act_out(MasicConvPlan* plan, void* act_out_bf16, int cpitch, int coff);
 /* useful work of one launch, for roofline accounting */
 int masic_conv_plan_info(const MasicConvPlan* plan, double* flops, double* hbm_bytes,
                          int* n_work_items, int* smem_bytes);
@@ -438,6 +443,20 @@ int masic_cqe_feature_fuse(const void* self_bf16, int self_pitch, const void* ot
 /* MASIC.py:1495-1496: out_nchw[b][c][p] = conv_out_nhwc[b][p][c] + identity_nchw[b][c][p], c < 3 (fp32). */
 int masic_cqe_residual_image(const float* conv_out_nhwc, int pitch, const float* identity_nchw, int n, int h,
                              int w, float* out_nchw, void* stream);
+/* Training.  Backward of masic_cqe_feature_fuse for one view, g = dL/d(out) (bf16, pitch g_pitch >= 2c):
+ *   d_self[p][0:c] = g[p][0:c] * w1[p]                                      (bf16, written)
+ *   d_other += transpose of the bilinear warp of g[p][c:2c] * w0[p]        (fp32 NHWC, atomics: zero it first)
+ *   dweights[p][0] = sum_c g[p][c+.] * warp(other)[p][.],  dweights[p][1] = sum_c g[p][.] * self[p][.]
+ *                                                                           (NHWC (N,H,W,2) fp32, written)
+ * The two views cross: view L's fuse warps EB1(R) by H^-1, so its d_other is EB1(R)'s gradient, and the reverse. */
+int masic_cqe_feature_fuse_bwd(const void* g_bf16, int g_pitch, const void* self_bf16, int self_pitch,
+                               const void* other_bf16, int other_pitch, int c, const float* weights_nchw2,
+                               const double* t_prepared, int n, int h, int w, void* d_self_bf16, int d_self_pitch,
+                               float* d_other_f32, int d_other_pitch, float* dweights_nhwc2, void* stream);
+/* Backward of masic_cqe_blend_images w.r.t. the weights only (the images come from the frozen codec):
+ * dweights[p][0] += sum_c g[p][c] a[c][p], dweights[p][1] += sum_c g[p][3+c] b[c][p]; g fp32 NHWC (pitch >= 6). */
+int masic_cqe_blend_images_bwd(const float* g_nhwc, int g_pitch, const float* a_nchw, const float* b_nchw, int n,
+                               int h, int w, float* dweights_nhwc2, void* stream);
 
 /* ------------------------------------------------------------- criterion */
 /* RateDistortionLoss.forward (coremasic/mywork/test2_real.py:88-114, newtrain_codec_real.py:66-87) on the
@@ -510,6 +529,10 @@ int masic_eb_aux_loss(const float* quantiles, int c, const float* const* matrice
 /* g *= act'(y) in place (ReLU / LeakyReLU(0.01) after conv()/deconv()); bias_grad[c] += sum_p g (may be NULL). */
 int masic_act_bwd_bias(void* g_bf16, int g_pitch, int g_coff, const void* y_bf16, int y_pitch, int y_coff,
                        int act, int64_t n_pixels, int c, float* bias_grad, void* stream);
+/* The same out of place: dst = g * act'(y), g unchanged (a residual block's skip still reads it). */
+int masic_act_bwd_bias_out(const void* g_bf16, int g_pitch, int g_coff, const void* y_bf16, int y_pitch, int y_coff,
+                           int act, int64_t n_pixels, int c, void* dst_bf16, int dst_pitch, int dst_coff,
+                           float* bias_grad, void* stream);
 /* GDN.forward as separate steps (gdn.py:77-92) keeping x and norm for the backward: sq = x^2; (norm = 1x1 conv on
  * the tensor cores); y = x * rsqrt(norm) (inverse: x * sqrt(norm)). */
 int masic_gdn_square(const void* x_bf16, void* sq_bf16, int64_t numel, void* stream);

@@ -111,6 +111,7 @@ def _declare(lib: C.CDLL) -> None:
         "masic_conv_plan_info": (i, [vp, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                      C.POINTER(i), C.POINTER(i)]),
         "masic_conv_plan_trace": (i, [vp, vp]),
+        "masic_conv_plan_set_act_out": (i, [vp, vp, i, i]),
         "masic_packed_weight_bytes": (i64, [i, i, i, i]),
         "masic_pack_conv_weights": (i, [vp, i, i, i, i, i, i, vp, i, vp]),
         "masic_pack_batch_create": (i, [C.POINTER(PackJob), i, C.POINTER(vp)]),
@@ -178,6 +179,7 @@ def _declare(lib: C.CDLL) -> None:
                                vp, vp, vp]),
         "masic_eb_aux_loss": (i, [vp, i, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(f), vp, vp, vp]),
         "masic_act_bwd_bias": (i, [vp, i, i, vp, i, i, i, i64, i, vp, vp]),
+        "masic_act_bwd_bias_out": (i, [vp, i, i, vp, i, i, i, i64, i, vp, i, i, vp, vp]),
         "masic_gdn_square": (i, [vp, vp, i64, vp]),
         "masic_gdn_apply": (i, [vp, vp, i, vp, i64, vp]),
         "masic_gdn_bwd_a": (i, [vp, vp, vp, i, vp, i64, i, vp, vp]),
@@ -201,6 +203,8 @@ def _declare(lib: C.CDLL) -> None:
         "masic_cqe_blend_images": (i, [vp, vp, vp, i, i, i, vp, i, vp]),
         "masic_cqe_feature_fuse": (i, [vp, i, vp, i, i, vp, vp, i, i, i, vp, i, i, vp]),
         "masic_cqe_residual_image": (i, [vp, i, vp, i, i, i, vp, vp]),
+        "masic_cqe_feature_fuse_bwd": (i, [vp, i, vp, i, vp, i, i, vp, vp, i, i, i, vp, i, vp, i, vp, vp]),
+        "masic_cqe_blend_images_bwd": (i, [vp, i, vp, vp, i, i, i, vp, vp]),
         "masic_rd_metrics_scratch_bytes": (i64, []),
         "masic_rd_metrics": (i, [C.POINTER(vp), C.POINTER(i64), vp, vp, vp, vp, i, i, i, i, f, vp, vp, vp]),
     }

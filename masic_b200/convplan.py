@@ -156,7 +156,10 @@ class ConvPlan:
                  residual1: Optional[torch.Tensor] = None, res1_coff: int = 0,
                  nt_in_coff: Optional[Sequence[int]] = None, nt_out_coff: Optional[Sequence[int]] = None,
                  nt_out_img: Optional[Sequence[int]] = None, cta_pairs: bool = False, pdl: bool = False,
-                 w_in: Optional[int] = None, out_blk_images: bool = False):
+                 w_in: Optional[int] = None, out_blk_images: bool = False,
+                 act_out: Optional[torch.Tensor] = None, act_out_coff: int = 0):
+        """act_out (training, with residual0): bf16 buffer that also receives act(conv + bias) before the residual
+        adds, at channel act_out_coff (masic_conv_plan_set_act_out)."""
         lib = _lib.load()
         assert x.is_cuda and x.dtype in (torch.bfloat16, torch.float16) and x.dim() == 4 and x.is_contiguous()
         assert out.is_cuda and out.dim() == 4 and out.is_contiguous()
@@ -232,6 +235,12 @@ class ConvPlan:
         check(lib.masic_conv_plan_create(C.byref(d), C.byref(handle)), "masic_conv_plan_create")
         self._h = handle
         self._lib = lib
+        self.act_out = act_out
+        if act_out is not None:
+            assert act_out.is_cuda and act_out.dtype == torch.bfloat16 and act_out.is_contiguous()
+            assert act_out.shape[:3] == out.shape[:3], (act_out.shape, out.shape)
+            check(lib.masic_conv_plan_set_act_out(handle, act_out.data_ptr(), act_out.shape[3], act_out_coff),
+                  "masic_conv_plan_set_act_out")
         fl, by, nw, sm = C.c_double(), C.c_double(), C.c_int(), C.c_int()
         lib.masic_conv_plan_info(handle, C.byref(fl), C.byref(by), C.byref(nw), C.byref(sm))
         self.flops, self.hbm_bytes, self.work_items, self.smem_bytes = fl.value, by.value, nw.value, sm.value

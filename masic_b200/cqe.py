@@ -97,11 +97,20 @@ class Independent_EN(nn.Module):
             self._engines[key] = eng
         return eng
 
+    def trainer(self, batch: int, height: int, width: int, device, lmbda: float = 0.01):
+        """The CUDA training step of stage two (the codec frozen): `CQETrainer.step_grads` fills `.grad` of every
+        parameter from lmbda * 255^2 * (mse1 + mse2) of the enhanced pair against the originals, `train_step` also
+        all-reduces the gradients and steps the optimiser.  H and W must be multiples of 64."""
+        from .cqe_trainer import CQETrainer
+        return CQETrainer(self, batch, height, width, device, lmbda=lmbda)
+
     def forward(self, x1_hat: torch.Tensor, x2_hat: torch.Tensor, h_matrix: torch.Tensor, clone: bool = True):
         if not x1_hat.is_cuda:
             raise MasicError("Independent_EN.forward needs CUDA tensors: masic_b200 has no CPU fallback")
         if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()) and self.training:
-            raise MasicError("Independent_EN runs inference only on the CUDA engine (call .eval() / torch.no_grad())")
+            raise MasicError("Independent_EN.forward runs inference only on the CUDA engine (call .eval() / "
+                             "torch.no_grad()); the training step (forward, loss, backward) runs as fused CUDA kernels "
+                             "through model.trainer(batch, H, W, device, lmbda).train_step(...)")
         b, _, h, w = x1_hat.shape
         o = self.engine_for(b, h, w, x1_hat.device).run(x1_hat, x2_hat, h_matrix)
         c = (lambda t: t.clone()) if clone else (lambda t: t)

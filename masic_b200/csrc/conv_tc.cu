@@ -107,6 +107,8 @@ struct KParams {
   uint32_t idesc_norm;   // the GDN norm MMA always runs on bf16 operands (x^2 rounded on the ALU pipe, gamma' bf16)
   int f16;         // 16-bit operand / activation format: 0 = bf16, 1 = fp16 (cvt16.cuh)
   int gdn2;        // 1: EPI_GDN2 (two epilogue teams, resident weights, one tile per item)
+  __nv_bfloat16* act_out;          // EPI_RESA: act(conv + bias) before the residual adds (masic_conv_plan_set_act_out)
+  int ao_pitch, ao_coff;
 };
 
 // misc smem region layout (byte offsets from smem_misc_off)
@@ -258,6 +260,9 @@ __device__ __forceinline__ Item next_item(const KParams& p, Cursor& c, int u_end
 // EPI selects the epilogue at compile time so that each variant gets its own register allocation (the GDN epilogue
 // is issue- and latency-bound: a spill there costs ~40 % on the 608x1088 layers)
 constexpr int EPI_PLAIN = 0, EPI_GDN = 1, EPI_RES = 2, EPI_GDN2 = 3;
+// EPI_RESA: EPI_RES that also stores the activated value before the residual adds (the training step's LeakyReLU
+// backward needs its sign; act + residual rounded to bf16 does not keep it where |act| << |residual|).  bf16, no CTA pairs.
+constexpr int EPI_RESA = 4;
 // EPI_GDN2 (layers whose whole weight set stays in shared memory, i.e. g_a_conv1): one tile per work item, TWO epilogue
 // teams of 8 warps that alternate over the items, each with its own accumulator, its own norm accumulator (the norm
 // MMA no longer overwrites x, so nothing has to stay in registers across it) and its own A2 / staging blocks.  The
@@ -781,7 +786,7 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
           float rs = 1.0f;
           size_t pix = 0;                           // linear output pixel of this thread's row (residual / rowscale)
           bool pix_ok = false;
-          if ((p.rowscale || EPI == EPI_RES) && valid) {
+          if ((p.rowscale || EPI == EPI_RES || EPI == EPI_RESA) && valid) {
             const int y = ty0 + (t >> 3), x = tx0 + (t & 7);
             pix_ok = y < p.rs_H && x < p.rs_W;
             pix = static_cast<size_t>(tn * p.rs_H + y) * p.rs_W + x;
@@ -794,7 +799,7 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
           const int k0 = half * cpg;                  // this group's first 16-channel chunk of the block
           const bool has0 = k0 < nchunk_blk, has1 = cpg == 2 && k0 + 1 < nchunk_blk;
           // residual rows are fetched first: their latency hides behind the TMEM load and the pair barrier
-          const bool do_res = EPI == EPI_RES && pix_ok;
+          const bool do_res = (EPI == EPI_RES || EPI == EPI_RESA) && pix_ok;
           uint4 rv[8];
           if (do_res) {
 #pragma unroll
@@ -849,6 +854,13 @@ conv_tc_kernel(const __grid_constant__ KParams p) {
                 const uint64_t rs2 = pk2(rs, rs);
 #pragma unroll
                 for (int i = 0; i < 8; ++i) o2[i] = mul2(o2[i], rs2);
+              }
+              if (EPI == EPI_RESA && do_res) {         // the 16 activated channels before the residual adds
+                uint4* ao = reinterpret_cast<uint4*>(p.act_out + pix * p.ao_pitch + p.ao_coff + it.nt * p.n_tile + ch);
+                ao[0] = make_uint4(pack16x2_p(o2[0], f16), pack16x2_p(o2[1], f16), pack16x2_p(o2[2], f16),
+                                   pack16x2_p(o2[3], f16));
+                ao[1] = make_uint4(pack16x2_p(o2[4], f16), pack16x2_p(o2[5], f16), pack16x2_p(o2[6], f16),
+                                   pack16x2_p(o2[7], f16));
               }
               if (do_res) {                            // out += residual(s): 16 bf16 = two 16-byte words each
 #pragma unroll
@@ -1344,11 +1356,11 @@ extern "C" int masic_conv_plan_create(const MasicConvDesc* dp, MasicConvPlan** p
   static bool attr_set = false;
   if (!attr_set) {
 #define MASIC_K2(C, E) (const void*)conv_tc_kernel<C, E, false>, (const void*)conv_tc_kernel<C, E, true>
-    const void* fns[14] = {MASIC_K2(false, EPI_PLAIN), MASIC_K2(false, EPI_GDN), MASIC_K2(false, EPI_RES),
+    const void* fns[15] = {MASIC_K2(false, EPI_PLAIN), MASIC_K2(false, EPI_GDN), MASIC_K2(false, EPI_RES),
                            MASIC_K2(true, EPI_PLAIN),  MASIC_K2(true, EPI_GDN),  MASIC_K2(true, EPI_RES),
-                           MASIC_K2(false, EPI_GDN2)};
+                           MASIC_K2(false, EPI_GDN2), (const void*)conv_tc_kernel<false, EPI_RESA, false>};
 #undef MASIC_K2
-    for (int i = 0; i < 14 && ce == cudaSuccess; ++i)
+    for (int i = 0; i < 15 && ce == cudaSuccess; ++i)
       ce = cudaFuncSetAttribute(fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (ce != cudaSuccess) { delete pl; return (int)ce; }
     attr_set = true;
@@ -1388,11 +1400,24 @@ extern "C" int masic_conv_plan_launch(const MasicConvPlan* pl, void* stream) {
     if (epi == EPI_RES) { MASIC_LAUNCH(true, EPI_RES); }
     MASIC_LAUNCH(true, EPI_PLAIN);
   }
+  if (pl->kp.act_out) return (int)cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, EPI_RESA, false>, pl->kp);
   if (epi == EPI_GDN2) { MASIC_LAUNCH(false, EPI_GDN2); }
   if (epi == EPI_GDN) { MASIC_LAUNCH(false, EPI_GDN); }
   if (epi == EPI_RES) { MASIC_LAUNCH(false, EPI_RES); }
   MASIC_LAUNCH(false, EPI_PLAIN);
 #undef MASIC_LAUNCH
+}
+
+extern "C" int masic_conv_plan_set_act_out(MasicConvPlan* pl, void* act_out_bf16, int cpitch, int coff) {
+  if (!pl || !act_out_bf16 || cpitch % 8 || coff % 8 || coff < 0) return MASIC_EINVAL;
+  const KParams& k = pl->kp;
+  if (!k.res0 || k.out_fp32 || k.rowscale) return MASIC_EINVAL;
+  if (k.cg2 || k.f16 || k.pdl || k.blk_img) return MASIC_ENOSUP;
+  if (coff + k.n_ntiles * k.n_tile > cpitch) return MASIC_EINVAL;
+  pl->kp.act_out = static_cast<__nv_bfloat16*>(act_out_bf16);
+  pl->kp.ao_pitch = cpitch;
+  pl->kp.ao_coff = coff;
+  return MASIC_OK;
 }
 
 extern "C" void masic_conv_plan_destroy(MasicConvPlan* pl) {

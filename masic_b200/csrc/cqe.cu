@@ -141,6 +141,93 @@ feature_fuse_kernel(const __nv_bfloat16* __restrict__ self, int self_pitch, cons
   }
 }
 
+// ---- training: backward of the two blends.  The images and the other view's features reach them from the frozen codec
+// or from EB1; the mask weights come from mask2weights_EN, so they get a gradient too.
+// Backward of feature_fuse_kernel for one view, g = dL/d(fused):
+//   d_self[p][0:C]   = g[p][0:C] * w1[p]                                                      (bf16, stored)
+//   d_other[q][0:C] += tap weight(p, q) * w0[p] * g[p][C:2C] over the four bilinear taps q   (fp32, atomics)
+//   dmw[p][0] = sum_c g[p][C+c] * warp(other)[p][c];  dmw[p][1] = sum_c g[p][c] * self[p][c]  (NHWC fp32, stored)
+// A warp owns 32 consecutive pixels: lane i evaluates the coordinates of pixel i (as in the forward), then the warp walks
+// the pixels with its lanes over the channels.
+__global__ void __launch_bounds__(256)
+feature_fuse_bwd_kernel(const __nv_bfloat16* __restrict__ g, int g_pitch, const __nv_bfloat16* __restrict__ self,
+                        int self_pitch, const __nv_bfloat16* __restrict__ other, int other_pitch, int C,
+                        const float* __restrict__ wgt, const double* __restrict__ T, int h, int w,
+                        __nv_bfloat16* __restrict__ d_self, int ds_pitch, float* __restrict__ d_other, int do_pitch,
+                        float* __restrict__ dmw) {
+  const int lane = threadIdx.x & 31;
+  const unsigned hw32 = (unsigned)h * (unsigned)w;
+  const unsigned warp_px0 = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 32u;
+  if (warp_px0 >= hw32) return;
+  const int bi = blockIdx.y;
+  const long hw = hw32;
+  const unsigned my_px = warp_px0 + lane;
+  Bilin b;
+  b.x0 = b.y0 = -10; b.w00 = b.w01 = b.w10 = b.w11 = 0.0f; b.in_x0 = b.in_x1 = b.in_y0 = b.in_y1 = false;
+  float w_self = 0.0f, w_other = 0.0f;
+  if (my_px < hw32) {
+    const int y = (int)(my_px / (unsigned)w), x = (int)(my_px - (unsigned)y * (unsigned)w);
+    b = bilin_coords(T + bi * 9, x, y, h, w, h, w);
+    w_other = __ldg(wgt + ((long)bi * 2) * hw + my_px);
+    w_self = __ldg(wgt + ((long)bi * 2 + 1) * hw + my_px);
+  }
+  const uint32_t my_flags = (uint32_t)b.in_x0 | ((uint32_t)b.in_x1 << 1) | ((uint32_t)b.in_y0 << 2) | ((uint32_t)b.in_y1 << 3);
+  const int npx = (int)min(32u, hw32 - warp_px0);
+  const long img = (long)bi * hw;
+  for (int j = 0; j < npx; ++j) {
+    const int x0 = __shfl_sync(0xffffffffu, b.x0, j), y0 = __shfl_sync(0xffffffffu, b.y0, j);
+    const float w00 = __shfl_sync(0xffffffffu, b.w00, j), w01 = __shfl_sync(0xffffffffu, b.w01, j);
+    const float w10 = __shfl_sync(0xffffffffu, b.w10, j), w11 = __shfl_sync(0xffffffffu, b.w11, j);
+    const uint32_t fl = __shfl_sync(0xffffffffu, my_flags, j);
+    const float ws = __shfl_sync(0xffffffffu, w_self, j), wo = __shfl_sync(0xffffffffu, w_other, j);
+    const long p = img + warp_px0 + j;
+    float s0 = 0.0f, s1 = 0.0f;
+    for (int c = lane; c < C; c += 32) {
+      const float gs = __bfloat162float(g[p * g_pitch + c]), go = __bfloat162float(g[p * g_pitch + C + c]);
+      s1 += gs * __bfloat162float(self[p * self_pitch + c]);
+      d_self[p * ds_pitch + c] = __float2bfloat16_rn(gs * ws);
+      const float gw = go * wo;
+      float warped = 0.0f;
+      auto tap = [&](bool ok, int yy, int xx, float wt) {
+        if (!ok) return;
+        const long q = img + (long)yy * w + xx;
+        warped += __bfloat162float(other[q * other_pitch + c]) * wt;
+        atomicAdd(d_other + q * do_pitch + c, wt * gw);
+      };
+      tap((fl & 4u) && (fl & 1u), y0, x0, w00);
+      tap((fl & 4u) && (fl & 2u), y0, x0 + 1, w01);
+      tap((fl & 8u) && (fl & 1u), y0 + 1, x0, w10);
+      tap((fl & 8u) && (fl & 2u), y0 + 1, x0 + 1, w11);
+      s0 += go * warped;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      s0 += __shfl_xor_sync(0xffffffffu, s0, o);
+      s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+    }
+    if (lane == 0) { dmw[p * 2] = s0; dmw[p * 2 + 1] = s1; }
+  }
+}
+
+// Backward of blend_images_kernel w.r.t. the mask weights only, g = dL/d(out) as fp32 NHWC (channels 0..5 read):
+//   dmw[p][0] += sum_c g[p][c] * a[c][p];  dmw[p][1] += sum_c g[p][3+c] * b[c][p]
+__global__ void __launch_bounds__(256)
+blend_images_bwd_kernel(const float* __restrict__ g, int g_pitch, const float* __restrict__ a,
+                        const float* __restrict__ b, int n, long hw, float* __restrict__ dmw) {
+  const long i = blockIdx.x * (long)blockDim.x + threadIdx.x;
+  if (i >= (long)n * hw) return;
+  const int bi = (int)(i / hw);
+  const long p = i - bi * hw;
+  float s0 = 0.0f, s1 = 0.0f;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    s0 += g[i * g_pitch + c] * a[((long)bi * 3 + c) * hw + p];
+    s1 += g[i * g_pitch + 3 + c] * b[((long)bi * 3 + c) * hw + p];
+  }
+  dmw[i * 2] += s0;
+  dmw[i * 2 + 1] += s1;
+}
+
 // out_nchw[b][c][p] = conv_out_nhwc[b][p][c] + identity_nchw[b][c][p],  c < 3
 __global__ void __launch_bounds__(256)
 residual_image_kernel(const float* __restrict__ conv_out, int pitch, const float* __restrict__ identity, int n, long hw,
@@ -274,6 +361,32 @@ extern "C" int masic_cqe_feature_fuse(const void* self_bf16, int self_pitch, con
   feature_fuse_kernel<<<dim3(((unsigned)h * (unsigned)w + px_per_block - 1) / px_per_block, n), 256, 0, S(stream)>>>(
       static_cast<const __nv_bfloat16*>(self_bf16), self_pitch, static_cast<const __nv_bfloat16*>(other_bf16), other_pitch,
       c, weights_nchw2, t_prepared, n, h, w, static_cast<__nv_bfloat16*>(out_bf16), out_pitch, f16);
+  return (int)cudaGetLastError();
+}
+
+extern "C" int masic_cqe_feature_fuse_bwd(const void* g_bf16, int g_pitch, const void* self_bf16, int self_pitch,
+                                          const void* other_bf16, int other_pitch, int c, const float* weights_nchw2,
+                                          const double* t_prepared, int n, int h, int w, void* d_self_bf16,
+                                          int d_self_pitch, float* d_other_f32, int d_other_pitch,
+                                          float* dweights_nhwc2, void* stream) {
+  if (!g_bf16 || !self_bf16 || !other_bf16 || !weights_nchw2 || !t_prepared || !d_self_bf16 || !d_other_f32 ||
+      !dweights_nhwc2 || c <= 0 || n <= 0 || h < 2 || w < 2 || g_pitch < 2 * c || self_pitch < c || other_pitch < c ||
+      d_self_pitch < c || d_other_pitch < c)
+    return MASIC_EINVAL;
+  const unsigned px_per_block = 256;                         // 8 warps x 32 pixels
+  feature_fuse_bwd_kernel<<<dim3(((unsigned)h * (unsigned)w + px_per_block - 1) / px_per_block, n), 256, 0, S(stream)>>>(
+      static_cast<const __nv_bfloat16*>(g_bf16), g_pitch, static_cast<const __nv_bfloat16*>(self_bf16), self_pitch,
+      static_cast<const __nv_bfloat16*>(other_bf16), other_pitch, c, weights_nchw2, t_prepared, h, w,
+      static_cast<__nv_bfloat16*>(d_self_bf16), d_self_pitch, d_other_f32, d_other_pitch, dweights_nhwc2);
+  return (int)cudaGetLastError();
+}
+
+extern "C" int masic_cqe_blend_images_bwd(const float* g_nhwc, int g_pitch, const float* a_nchw, const float* b_nchw,
+                                          int n, int h, int w, float* dweights_nhwc2, void* stream) {
+  if (!g_nhwc || !a_nchw || !b_nchw || !dweights_nhwc2 || g_pitch < 6 || n <= 0 || h <= 0 || w <= 0) return MASIC_EINVAL;
+  const long total = (long)n * h * w;
+  blend_images_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, S(stream)>>>(g_nhwc, g_pitch, a_nchw, b_nchw, n,
+                                                                                  (long)h * w, dweights_nhwc2);
   return (int)cudaGetLastError();
 }
 

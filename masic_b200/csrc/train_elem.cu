@@ -79,6 +79,25 @@ act_bwd_bias_kernel(__nv_bfloat16* __restrict__ g, int gpitch, int gcoff, const 
   });
 }
 
+// out-of-place: dst = g * act'(y); colsum += sum_p dst.  g is left as it is (a residual block's skip still reads it).
+__global__ void __launch_bounds__(256)
+act_bwd_bias_out_kernel(const __nv_bfloat16* __restrict__ g, int gpitch, int gcoff, const __nv_bfloat16* __restrict__ y,
+                        int ypitch, int ycoff, int act, long npix, int C, __nv_bfloat16* __restrict__ dst, int dpitch,
+                        int dcoff, float* __restrict__ colsum) {
+  colsum_driver(npix, C, colsum, [&](long p, int c) {
+    float2 v = ld_bf2(g + p * gpitch + gcoff + c);
+    if (act != MASIC_ACT_NONE) {
+      const float2 yy = ld_bf2(y + p * ypitch + ycoff + c);
+      const float slope = act == MASIC_ACT_RELU ? 0.0f : 0.01f;
+      v.x = yy.x > 0.0f ? v.x : v.x * slope;
+      v.y = yy.y > 0.0f ? v.y : v.y * slope;
+    }
+    __nv_bfloat16* dp = dst + p * dpitch + dcoff + c;
+    st_bf2(dp, v.x, v.y);
+    return ld_bf2(dp);                        // sum what the dgrad / wgrad kernels will read
+  });
+}
+
 // fp32 gradient variant (sigma/mu/logit gradients arrive as bf16 already; this one serves fp32 sources): colsum only
 __global__ void __launch_bounds__(256)
 colsum_bf16_kernel(const __nv_bfloat16* __restrict__ g, int gpitch, int gcoff, long npix, int C,
@@ -286,6 +305,19 @@ extern "C" int masic_act_bwd_bias(void* g_bf16, int g_pitch, int g_coff, const v
   else
     act_bwd_bias_kernel<<<cs_grid(n_pixels, c), dim3(32, 8), 0, S(stream)>>>(BF(g_bf16), g_pitch, g_coff, CBF(y_bf16),
                                                                               y_pitch, y_coff, act, n_pixels, c, bias_grad);
+  return (int)cudaGetLastError();
+}
+
+extern "C" int masic_act_bwd_bias_out(const void* g_bf16, int g_pitch, int g_coff, const void* y_bf16, int y_pitch,
+                                      int y_coff, int act, int64_t n_pixels, int c, void* dst_bf16, int dst_pitch,
+                                      int dst_coff, float* bias_grad, void* stream) {
+  if (!g_bf16 || !dst_bf16 || n_pixels <= 0 || c <= 0 || (c & 1) || (g_pitch & 1) || (g_coff & 1) || (dst_pitch & 1) ||
+      (dst_coff & 1) || dst_coff + c > dst_pitch || g_coff + c > g_pitch)
+    return MASIC_EINVAL;
+  if (act != MASIC_ACT_NONE && (!y_bf16 || (y_pitch & 1) || (y_coff & 1) || y_coff + c > y_pitch)) return MASIC_EINVAL;
+  act_bwd_bias_out_kernel<<<cs_grid(n_pixels, c), dim3(32, 8), 0, S(stream)>>>(
+      CBF(g_bf16), g_pitch, g_coff, CBF(y_bf16), y_pitch, y_coff, act, n_pixels, c, BF(dst_bf16), dst_pitch, dst_coff,
+      bias_grad);
   return (int)cudaGetLastError();
 }
 

@@ -182,3 +182,25 @@ def wgrad_small(lo, c_lo, hi, dw):
 def colsum_nchw(g, out):
     n, c = g.shape[0], g.shape[1]
     check(_lib.load().masic_colsum_nchw(_p(g), n, c, g.numel() // (n * c), _p(out), _s()), "masic_colsum_nchw")
+
+
+def act_bwd_bias_out(g, g_coff, c, y, y_coff, act, dst, dst_coff, bias_grad):
+    npix = g.numel() // g.shape[-1]
+    check(_lib.load().masic_act_bwd_bias_out(_p(g), g.shape[-1], g_coff, _p(y), 0 if y is None else y.shape[-1], y_coff,
+                                             act, npix, c, _p(dst), dst.shape[-1], dst_coff, _p(bias_grad), _s()),
+          "masic_act_bwd_bias_out")
+
+
+def cqe_feature_fuse_bwd(g, self_, other, weights, t_prepared, d_self, d_other, dweights):
+    """Backward of masic_cqe_feature_fuse for one view; NHWC buffers, c = the channels of self_ / other."""
+    n, h, w, c = self_.shape
+    check(_lib.load().masic_cqe_feature_fuse_bwd(_p(g), g.shape[-1], _p(self_), c, _p(other), other.shape[-1], c,
+                                                 _p(weights), _p(t_prepared), n, h, w, _p(d_self), d_self.shape[-1],
+                                                 _p(d_other), d_other.shape[-1], _p(dweights), _s()),
+          "masic_cqe_feature_fuse_bwd")
+
+
+def cqe_blend_images_bwd(g, a, b, dweights):
+    n, _, h, w = a.shape
+    check(_lib.load().masic_cqe_blend_images_bwd(_p(g), g.shape[-1], _p(a), _p(b), n, h, w, _p(dweights), _s()),
+          "masic_cqe_blend_images_bwd")

@@ -64,7 +64,13 @@ class _Layer:
                  tap_mask: int = 0, gx: Optional[torch.Tensor] = None, gx_coff: int = 0, gout: Optional[torch.Tensor] = None,
                  weight: Optional[torch.Tensor] = None, bias: Optional[torch.Tensor] = None,
                  dweight: Optional[torch.Tensor] = None, dbias: Optional[torch.Tensor] = None, accumulate: bool = False,
-                 share: Optional["_Layer"] = None, wgrad_tap_mask: Optional[int] = None):
+                 share: Optional["_Layer"] = None, wgrad_tap_mask: Optional[int] = None,
+                 res0: Optional[torch.Tensor] = None, res1: Optional[torch.Tensor] = None,
+                 act_out: Optional[torch.Tensor] = None, dg_n_tile: int = 0,
+                 dg_res0: Optional[torch.Tensor] = None, dg_res0_coff: int = 0,
+                 dg_res1: Optional[torch.Tensor] = None, dg_res1_coff: int = 0):
+        """res0 / res1 / act_out: residual adds of the forward epilogue and the pre-residual activation store
+        (ResidualBlock); dg_res0 / dg_res1: residual adds of the data gradient's epilogue (the skips' gradients)."""
         self.tr, self.name = tr, name
         self.transposed, self.k, self.stride, self.c_in, self.c_out = transposed, k, stride, c_in, c_out
         self.w = weight if weight is not None else tr.param(name + ".weight")
@@ -91,7 +97,8 @@ class _Layer:
         # data gradients, which are the same operator transposed) and the wide 1x1 / 3x3 / masked layers
         pairs = (k == 5 and stride == 2 and c_in == 128 and c_out == 128 and not transposed) or (k == 1 and c_out >= 3000)
         self.fwd_plan = ConvPlan(packed=self.pack, stride=stride, tap_mask=tap_mask, x=x, in_coff=in_coff, out=out,
-                                 out_coff=out_coff, act=act, cta_pairs=pairs)
+                                 out_coff=out_coff, act=act, cta_pairs=pairs, residual0=res0, residual1=res1,
+                                 act_out=act_out)
         # ---- weight gradient: conv: LO = dL/dout, HI = input; deconv: LO = input, HI = dL/dout
         if gout is not None:
             if transposed:
@@ -111,12 +118,13 @@ class _Layer:
                     dkind = CONV if transposed else DECONV_S2
                 else:
                     dkind = CONV
-                dn = 128 if c_in % 192 else 192
+                dn = dg_n_tile or (128 if c_in % 192 else 192)
                 self.dpack = PackedConv(kind=dkind, ksize=k, c_in=c_out, c_out=c_in, n_tile=dn, weight=self.w,
                                         transposed=not transposed)
                 tr.repack.append((self.dpack, self.w, None))
             self.dg_plan = ConvPlan(packed=self.dpack, stride=stride, tap_mask=_flip_mask(tap_mask, k) if tap_mask else 0,
-                                    x=gout, in_coff=out_coff, out=gx, out_coff=gx_coff)
+                                    x=gout, in_coff=out_coff, out=gx, out_coff=gx_coff, residual0=dg_res0,
+                                    res0_coff=dg_res0_coff, residual1=dg_res1, res1_coff=dg_res1_coff)
 
     def fwd(self):
         self.fwd_plan.launch()
@@ -233,20 +241,13 @@ class _GDN3:
         T.reparam_bwd(self.dgp, self.gamma, 0.0, self.dgamma)
 
 
-class HSICTrainer:
-    def __init__(self, model, batch: int, height: int, width: int, device, lmbda: float = 0.01,
-                 use_graph: bool = True):
+class TrainStep:
+    """What every training step of this package shares: the flat gradient buffer, the weight re-packing, the
+    forward / backward op lists with their lanes and the weight-gradient side stream, and the CUDA-graph replay.
+    A subclass builds its ops in `_build()` and defines `_issue(refresh)`."""
+
+    def _init_step(self, model, use_graph: bool):
         self.use_graph, self.graph, self._warm = use_graph, None, False
-        if height % 64 or width % 64:
-            raise ValueError("HSIC needs H and W to be multiples of 64")
-        self.lib = _lib.load()
-        self.dev = torch.device(device)
-        if self.dev.type != "cuda":
-            raise MasicError("HSICTrainer runs on a CUDA device only (no CPU fallback)")
-        self.model, self.B, self.H, self.W, self.lmbda = model, batch, height, width, float(lmbda)
-        self.N, self.M, self.K = model.N, model.M, model.K
-        if (self.N, self.M, self.K) != (128, 192, 5):
-            raise MasicError("the sm_100a kernels are specialised for HSIC(N=128, M=192, K=5)")
         self._params: Dict[str, torch.nn.Parameter] = dict(torch.nn.Module.named_parameters(model))
         for n, p in self._params.items():
             if not p.is_cuda or p.dtype != F32:
@@ -262,16 +263,15 @@ class HSICTrainer:
             off += p.numel()
         self.repack: List[Tuple[PackedConv, torch.Tensor, Optional[torch.Tensor]]] = []
         self._pack_batch = None
-        self.gdn_prep: List[_GDN] = []
-        self.gdn_finish: List[_GDN] = []
         self.zero_each_step: List[torch.Tensor] = []
         self.fwd_ops: List[Tuple[str, Callable[[], None]]] = []
         self.bwd_ops: List[Tuple[str, Callable[[], None]]] = []
-        self.flops_fwd = 0.0
-        with torch.cuda.device(self.dev):
-            self._wg_stream = torch.cuda.Stream(device=self.dev)
-            self._lane_streams: List[torch.cuda.Stream] = []
-            self._build()
+        self.pre_repack: List[Callable[[], None]] = []
+        self.post_bwd: List[Callable[[], None]] = []
+
+    def _make_streams(self):
+        self._wg_stream = torch.cuda.Stream(device=self.dev)
+        self._lane_streams: List[torch.cuda.Stream] = []
 
     # ------------------------------------------------------------------ helpers
     def param(self, name):
@@ -306,6 +306,108 @@ class HSICTrainer:
         ev = torch.cuda.Event()
         ev.record(self._wg_stream)
         torch.cuda.current_stream().wait_event(ev)
+
+    def _repack_weights(self):
+        """Re-pack every weight the kernels read from the model's current fp32 parameters."""
+        for f in self.pre_repack:
+            f()
+        if self._pack_batch is None:
+            ok = all(w.dtype == F32 and w.is_contiguous() and (b is None or (b.dtype == F32 and b.is_contiguous()))
+                     for _, w, b in self.repack)
+            self._pack_batch = PackBatch(self.repack) if ok else False
+        if self._pack_batch:
+            self._pack_batch.launch()                    # every weight pack and bias copy in one launch
+        else:
+            for pk, w, b in self.repack:
+                pk.repack(w, b)
+
+    def _run(self, refresh: bool):
+        """One step: replayed as a CUDA graph once warm (eager issue through ctypes is host-bound, ~20 us per
+        launch), issued eagerly otherwise; then `.grad` of every parameter points at its flat-buffer view."""
+        if self.use_graph and self._warm and refresh:
+            if self.graph is None:
+                torch.cuda.synchronize(self.dev)
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g):
+                    self._issue(True)
+                self.graph = g
+            self.graph.replay()
+        else:
+            self._issue(refresh)
+            self._warm = True
+        for n, p in self._params.items():
+            p.grad = self._grads[n]
+
+    def _run_lanes(self, ops, lanes):
+        main = torch.cuda.current_stream()
+        while len(self._lane_streams) < len(lanes):
+            self._lane_streams.append(torch.cuda.Stream(device=self.dev))
+        on_lane = frozenset().union(*[l[0] for l in lanes])
+
+        def fork(i):                                 # the lane sees everything issued on the main stream so far
+            ev = torch.cuda.Event()
+            ev.record(main)
+            side = self._lane_streams[i]
+            side.wait_event(ev)
+            with torch.cuda.stream(side):
+                for name, fn in ops:
+                    if name in lanes[i][0]:
+                        fn()
+
+        joined = set()
+        for i, (_, fork_after, _) in enumerate(lanes):
+            if fork_after is None:
+                fork(i)
+        for name, fn in ops:
+            if name in on_lane:
+                continue
+            for i, (_, _, join_before) in enumerate(lanes):
+                if name == join_before:
+                    ev = torch.cuda.Event()
+                    ev.record(self._lane_streams[i])
+                    main.wait_event(ev)
+                    joined.add(i)
+            fn()
+            for i, (_, fork_after, _) in enumerate(lanes):
+                if name == fork_after:
+                    fork(i)
+        assert len(joined) == len(lanes), "a lane was never joined"
+
+    def profile(self, iters: int = 3):
+        """CUDA-event time of every forward / backward op group (after one warm step)."""
+        res = []
+        with torch.cuda.device(self.dev):
+            for name, fn in [("F:" + n, f) for n, f in self.fwd_ops] + [("B:" + n, f) for n, f in self.bwd_ops]:
+                ts = []
+                for _ in range(iters):
+                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                    e0.record(); fn(); e1.record()
+                    torch.cuda.synchronize()
+                    ts.append(e0.elapsed_time(e1))
+                res.append((name, sorted(ts)[len(ts) // 2]))
+        return res
+
+
+class HSICTrainer(TrainStep):
+    def __init__(self, model, batch: int, height: int, width: int, device, lmbda: float = 0.01,
+                 use_graph: bool = True):
+        if height % 64 or width % 64:
+            raise ValueError("HSIC needs H and W to be multiples of 64")
+        self.lib = _lib.load()
+        self.dev = torch.device(device)
+        if self.dev.type != "cuda":
+            raise MasicError("HSICTrainer runs on a CUDA device only (no CPU fallback)")
+        self.model, self.B, self.H, self.W, self.lmbda = model, batch, height, width, float(lmbda)
+        self.N, self.M, self.K = model.N, model.M, model.K
+        if (self.N, self.M, self.K) != (128, 192, 5):
+            raise MasicError("the sm_100a kernels are specialised for HSIC(N=128, M=192, K=5)")
+        self._init_step(model, use_graph)
+        self.gdn_prep: List[_GDN] = []
+        self.gdn_finish: List[_GDN] = []
+        self.flops_fwd = 0.0
+        with torch.cuda.device(self.dev):
+            self._make_streams()
+            self._build()
 
     # ------------------------------------------------------------------ sub-graphs
     def _encoder_pass(self, tag: str, enc: str, img_bf: torch.Tensor, img_nchw: torch.Tensor, accumulate: bool,
@@ -526,8 +628,6 @@ class HSICTrainer:
         h16, w16 = H // 16, W // 16
         lib = self.lib
         dev = self.dev
-        self.pre_repack: List[Callable[[], None]] = []
-        self.post_bwd: List[Callable[[], None]] = []
         self.noise = {k: self._z(B, (h16 // 4) if k.startswith("z") else h16, (w16 // 4) if k.startswith("z") else w16,
                                  N if k.startswith("z") else M, dtype=F32) for k in NOISE_KEYS}     # NHWC
         self.x1 = self._z(B, 3, H, W, dtype=F32)
@@ -753,18 +853,9 @@ class HSICTrainer:
     # ------------------------------------------------------------------ running
     @torch.no_grad()
     def refresh_weights(self):
-        """Re-pack every weight the kernels read from the model's current fp32 parameters."""
-        for f in self.pre_repack:
-            f()
-        if self._pack_batch is None:
-            ok = all(w.dtype == F32 and w.is_contiguous() and (b is None or (b.dtype == F32 and b.is_contiguous()))
-                     for _, w, b in self.repack)
-            self._pack_batch = PackBatch(self.repack) if ok else False
-        if self._pack_batch:
-            self._pack_batch.launch()                    # ~110 weight packs + ~50 bias copies in one launch
-        else:
-            for pk, w, b in self.repack:
-                pk.repack(w, b)
+        """Re-pack every weight the kernels read from the model's current fp32 parameters (~110 weight packs and ~50
+        bias copies in one launch) and prepare the GDN layers' effective parameters."""
+        self._repack_weights()
         for g in self.gdn_prep:
             g.prepare()
         # MaskedConv2d side effect (layers.py:77) is applied through tap_mask; keep the parameter masked too
@@ -781,21 +872,8 @@ class HSICTrainer:
         see them).  noise: NCHW fp32 tensors keyed by NOISE_KEYS, or None to draw U(-.5,.5) on the device."""
         with torch.cuda.device(self.dev):
             self._load_inputs(x1, x2, h_matrix, noise)
-            if self.use_graph and self._warm and refresh:
-                # the ~700 launches of a step (zeroing, weight re-packing, forward, backward) replayed as ONE CUDA graph:
-                # eager issue through ctypes is host-bound (~20 us per launch)
-                if self.graph is None:
-                    torch.cuda.synchronize(self.dev)
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        self._issue(True)
-                    self.graph = g
-                self.graph.replay()
-            else:
-                self._issue(refresh)
-                self._warm = True
-            for n, p in self._params.items():
-                p.grad = self._grads[n]
+            # the ~700 launches of a step (zeroing, weight re-packing, forward, backward) replayed as ONE CUDA graph
+            self._run(refresh)
             return self.read_losses() if read_back else None
 
     def _load_inputs(self, x1, x2, h_matrix, noise):
@@ -828,41 +906,6 @@ class HSICTrainer:
                   "R.mask_fuse", "wgrad.join"),)       # inputs complete after R.mask_fuse; only weight gradients come out
     # (measured and dropped: a third lane for L.gmm_net / L.context / L.hyper from the start of the backward pass,
     # joined before L.latent_merge: 8.37 vs 8.28 ms — the lanes already keep the SMs busy)
-
-    def _run_lanes(self, ops, lanes):
-        main = torch.cuda.current_stream()
-        while len(self._lane_streams) < len(lanes):
-            self._lane_streams.append(torch.cuda.Stream(device=self.dev))
-        on_lane = frozenset().union(*[l[0] for l in lanes])
-
-        def fork(i):                                 # the lane sees everything issued on the main stream so far
-            ev = torch.cuda.Event()
-            ev.record(main)
-            side = self._lane_streams[i]
-            side.wait_event(ev)
-            with torch.cuda.stream(side):
-                for name, fn in ops:
-                    if name in lanes[i][0]:
-                        fn()
-
-        joined = set()
-        for i, (_, fork_after, _) in enumerate(lanes):
-            if fork_after is None:
-                fork(i)
-        for name, fn in ops:
-            if name in on_lane:
-                continue
-            for i, (_, _, join_before) in enumerate(lanes):
-                if name == join_before:
-                    ev = torch.cuda.Event()
-                    ev.record(self._lane_streams[i])
-                    main.wait_event(ev)
-                    joined.add(i)
-            fn()
-            for i, (_, fork_after, _) in enumerate(lanes):
-                if name == fork_after:
-                    fork(i)
-        assert len(joined) == len(lanes), "a lane was never joined"
 
     def _issue(self, refresh: bool):
         self.flat_grad.zero_()
@@ -898,20 +941,6 @@ class HSICTrainer:
         optimizer.step()
         aux_optimizer.step()
         return self.read_losses()
-
-    def profile(self, iters: int = 3):
-        """CUDA-event time of every forward / backward op group (after one warm step)."""
-        res = []
-        with torch.cuda.device(self.dev):
-            for name, fn in [("F:" + n, f) for n, f in self.fwd_ops] + [("B:" + n, f) for n, f in self.bwd_ops]:
-                ts = []
-                for _ in range(iters):
-                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    e0.record(); fn(); e1.record()
-                    torch.cuda.synchronize()
-                    ts.append(e0.elapsed_time(e1))
-                res.append((name, sorted(ts)[len(ts) // 2]))
-        return res
 
 
 class _Conv1:
