@@ -469,6 +469,19 @@ int64_t masic_rd_metrics_scratch_bytes(void);
 int masic_rd_metrics(const float* const* lik4_host, const int64_t* lik_numel4_host, const float* x1_hat,
                      const float* x1, const float* x2_hat, const float* x2, int n, int c, int h, int w,
                      float lmbda, void* scratch, float* out8, void* stream);
+/* pytorch_msssim.ms_ssim / ssim (version 1.0) of two NCHW fp32 batches x, y (device), as the reference's eval loop
+ * reports it next to bpp and PSNR (coremasic/mywork/test2_real.py:88-114; test3_real.py after the enhancement net):
+ * out_nc (device, n*c floats) = per-(n, c) value.  11-tap Gaussian window (sigma 1.5, float32 taps computed on the host
+ * as the package does), valid correlation, C1 = (k1*data_range)^2, C2 = (k2*data_range)^2; `levels` (1..5) scales with
+ * avg_pool2d(2, padding (h%2, w%2), count_include_pad) between them; value = prod_{l<levels-1} relu(mean cs_l)^w_l
+ * * s^w_{levels-1}, s = mean ssim of the last level, relu'd when nonneg_last != 0 (ms_ssim always, ssim with
+ * nonnegative_ssim).  levels = 1 with weights {1} is ssim.  weights_host: HOST array of `levels` floats.  Every level
+ * must be at least 11 x 11 (MASIC_EINVAL otherwise).  scratch is masic_ms_ssim_scratch_bytes() of device memory (the
+ * pyramid and per-tile partial sums).  Deterministic (fixed-order fp64 reduction) and batch invariant: a plane's value
+ * does not depend on the other planes of the call. */
+int64_t masic_ms_ssim_scratch_bytes(int n, int c, int h, int w, int levels);
+int masic_ms_ssim(const float* x, const float* y, int n, int c, int h, int w, int levels, float data_range, float k1,
+                  float k2, const float* weights_host, int nonneg_last, void* scratch, float* out_nc, void* stream);
 
 /* ------------------------------------------------------- training: weight gradients */
 /* dW[cl][ch][ky][kx] = sum_{n,p} LO[n,p,cl] * HI[n, stride*p + k - ksize/2, ch]  on the tensor cores

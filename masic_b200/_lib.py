@@ -207,6 +207,8 @@ def _declare(lib: C.CDLL) -> None:
         "masic_cqe_blend_images_bwd": (i, [vp, i, vp, vp, i, i, i, vp, vp]),
         "masic_rd_metrics_scratch_bytes": (i64, []),
         "masic_rd_metrics": (i, [C.POINTER(vp), C.POINTER(i64), vp, vp, vp, vp, i, i, i, i, f, vp, vp, vp]),
+        "masic_ms_ssim_scratch_bytes": (i64, [i, i, i, i, i]),
+        "masic_ms_ssim": (i, [vp, vp, i, i, i, i, i, f, f, f, C.POINTER(f), i, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)      # AttributeError here = header/library mismatch

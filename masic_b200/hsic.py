@@ -19,6 +19,7 @@ from typing import Dict, Optional, Tuple
 import torch
 import torch.nn as nn
 
+from . import ops as _ops
 from ._lib import MasicError
 from .engine import HSICEngine
 from .entropy_models import EntropyBottleneck, GaussianMixtureConditional_gf
@@ -295,10 +296,12 @@ class PairStream:
         t0 = ps.submit(x1_host, x2_host, h_host)     # pinned (1,3,H,W) fp32 x2, (1,3,3) fp32
         t1 = ps.submit(...)                          # its H2D copy overlaps pair 0's kernels
         bpp, psnr1, psnr2 = ps.result(t0)            # the criterion, read back from the device (32 bytes)
+        t2 = ps.submit(..., msssim=True)             # + MS-SSIM of both views, in result(t2)[3]
 
     `depth` slots (default 2), each with its own engine and stream: the H2D copy of pair i+1 runs on a copy stream
     while pair i replays its engine's CUDA graph, and the kernels of consecutive pairs overlap on the GPU; the
-    criterion is one fused reduction pass (masic_rd_metrics) whose 8 floats come back through pinned memory.
+    criterion is one fused reduction pass (masic_rd_metrics) whose 8 floats come back through pinned memory; with
+    msssim=True the slot's stream also runs masic_ms_ssim on both views and 6 more floats ride in the same read-back.
     `outputs()` exposes the engine's output tensors of the LAST submitted pair (valid after `result(ticket)`).
     """
 
@@ -328,24 +331,35 @@ class PairStream:
                 liks = [o["lik_y1"], o["lik_y2"], o["lik_z1"], o["lik_z2"]]
                 self.slots.append(dict(
                     eng=eng, stream=torch.cuda.Stream(device=self.dev),
-                    res_d=torch.zeros(8, device=self.dev), res_h=torch.zeros(8).pin_memory(),
+                    # criterion (8 floats) | MS-SSIM per channel of view 1 (3) and view 2 (3)
+                    res_d=torch.zeros(14, device=self.dev), res_h=torch.zeros(14).pin_memory(),
                     copied=torch.cuda.Event(), done=torch.cuda.Event(), busy=False, has_result=False,
                     scratch=torch.empty(self.lib.masic_rd_metrics_scratch_bytes() // 8, dtype=torch.float64, device=self.dev),
                     lik_p=(C.c_void_p * 4)(*[t.data_ptr() for t in liks]),
                     lik_n=(C.c_int64 * 4)(*[t.numel() for t in liks])))
+        self._ms_weights = (C.c_float * 5)(*_ops.MS_SSIM_WEIGHTS)
         self._n = 0
 
     def submit(self, x1: torch.Tensor, x2: torch.Tensor, h: torch.Tensor, criterion: bool = True,
-               want_recon: bool = False) -> int:
+               want_recon: bool = False, msssim: bool = False) -> int:
         """Queue one pair.  x1 / x2: (1,3,H,W) uint8 images as they come out of the dataset's PNG files (the recommended
         host format: converted on the device exactly like torchvision's ToTensor, a quarter of the PCIe bytes, which is
         what keeps eight ranks on one host from becoming host-bound), or float32 in [0,1] as the reference's loaders
         feed them; h: (1,3,3)
         float32.  Pinned host tensors (H2D copy) or device tensors (D2D copy).  criterion=False
         skips the RateDistortionLoss reduction (forward only; `result` then just waits for the pair).  want_recon=True
-        also copies the two reconstructions (what a codec is for) to pinned host memory: `reconstructions(ticket)`."""
+        also copies the two reconstructions (what a codec is for) to pinned host memory: `reconstructions(ticket)`.
+        msssim=True (with the criterion) also computes pytorch_msssim's ms_ssim(x_hat, x, data_range=1.0) of both views
+        on the device (the third number of the reference's eval loop); `result` then reports it.  It needs
+        min(H, W) > 160, as the package does."""
         from ._lib import check
+        if msssim and not criterion:
+            raise ValueError("msssim=True is part of the criterion: it needs criterion=True")
         s = self.slots[self._n % self.depth]
+        if msssim and "ms_scratch" not in s:
+            nbytes = self.lib.masic_ms_ssim_scratch_bytes(1, 3, self.H, self.W, len(_ops.MS_SSIM_WEIGHTS))
+            check(min(int(nbytes), 0), f"masic_ms_ssim_scratch_bytes ({self.H}x{self.W}: MS-SSIM needs min(H, W) > 160)")
+            s["ms_scratch"] = torch.empty(nbytes, dtype=torch.uint8, device=self.dev)
         if s["busy"]:
             s["done"].synchronize()                 # the slot's previous pair has left its engine
         eng, st = s["eng"], s["stream"]
@@ -375,14 +389,21 @@ class PairStream:
                                                 o["x2_hat"].data_ptr(), eng.x2.data_ptr(), 1, 3, self.H, self.W,
                                                 self.lmbda, s["scratch"].data_ptr(), s["res_d"].data_ptr(),
                                                 st.cuda_stream), "masic_rd_metrics")
-                s["res_h"].copy_(s["res_d"], non_blocking=True)
+                if msssim:
+                    for v, (xh, x) in enumerate(((o["x1_hat"], eng.x1), (o["x2_hat"], eng.x2))):
+                        check(self.lib.masic_ms_ssim(xh.data_ptr(), x.data_ptr(), 1, 3, self.H, self.W, 5, 1.0, 0.01,
+                                                     0.03, self._ms_weights, 1, s["ms_scratch"].data_ptr(),
+                                                     s["res_d"][8 + 3 * v:].data_ptr(), st.cuda_stream), "masic_ms_ssim")
+                    s["res_h"].copy_(s["res_d"], non_blocking=True)
+                else:
+                    s["res_h"][:8].copy_(s["res_d"][:8], non_blocking=True)
             if want_recon:
                 if "rec_h" not in s:
                     s["rec_h"] = [torch.empty(1, 3, self.H, self.W).pin_memory() for _ in range(2)]
                 s["rec_h"][0].copy_(o["x1_hat"], non_blocking=True)
                 s["rec_h"][1].copy_(o["x2_hat"], non_blocking=True)
             s["done"].record(st)
-        s["busy"], s["has_result"], s["has_recon"] = True, criterion, want_recon
+        s["busy"], s["has_result"], s["has_recon"], s["has_msssim"] = True, criterion, want_recon, msssim
         self.eng = eng
         self._n += 1
         return self._n - 1
@@ -396,7 +417,8 @@ class PairStream:
             s["udh"] = UDHEngine(net.state_dict(), 1, self.dev, net.patch_size)
 
     def submit_patches(self, x1: torch.Tensor, x2: torch.Tensor, patch_a: torch.Tensor, patch_b: torch.Tensor,
-                       corners: torch.Tensor, criterion: bool = True, want_recon: bool = False) -> int:
+                       corners: torch.Tensor, criterion: bool = True, want_recon: bool = False,
+                       msssim: bool = False) -> int:
         """Like `submit`, but instead of h_matrix takes what the dataset hands over (datasets/utils.py:383-395): the two
         (1,1,128,128) normalised grey patches and their (1,4,2) corner coordinates.  The udh net, the 4-point DLT,
         the inverse and h_adjust (test2_real.py:201-211) run on the slot's stream ahead of the codec; the host never
@@ -421,10 +443,12 @@ class PairStream:
             ev2 = torch.cuda.Event()
             ev2.record(s["stream"])
         self.copy_stream.wait_event(ev2)            # submit() copies h on the copy stream
-        return self.submit(x1, x2, h, criterion=criterion, want_recon=want_recon)
+        return self.submit(x1, x2, h, criterion=criterion, want_recon=want_recon, msssim=msssim)
 
     def result(self, ticket: int):
-        """(bpp, psnr1_db, psnr2_db, detail) of a submitted pair; blocks until its D2H copy has landed."""
+        """(bpp, psnr1_db, psnr2_db, detail) of a submitted pair; blocks until its D2H copy has landed.  A pair
+        submitted with msssim=True also has detail["msssim1"/"msssim2"] (mean over the 3 channels, as
+        pytorch_msssim's size_average) and "msssim1_db"/"msssim2_db" = -10 log10(1 - value)."""
         if not (self._n - self.depth <= ticket < self._n):
             raise ValueError(f"ticket {ticket} is no longer (or not yet) in flight")
         s = self.slots[ticket % self.depth]
@@ -433,8 +457,14 @@ class PairStream:
             return None
         r = s["res_h"].tolist()
         psnr = [10.0 * math.log10(1.0 / m) if m > 0 else float("inf") for m in r[4:6]]
-        return r[6], psnr[0], psnr[1], {"bpp_y1": r[0], "bpp_y2": r[1], "bpp_z1": r[2], "bpp_z2": r[3],
-                                        "mse1": r[4], "mse2": r[5], "loss": r[7]}
+        detail = {"bpp_y1": r[0], "bpp_y2": r[1], "bpp_z1": r[2], "bpp_z2": r[3], "mse1": r[4], "mse2": r[5],
+                  "loss": r[7]}
+        if s["has_msssim"]:
+            for v in (1, 2):
+                m = sum(r[5 + 3 * v:8 + 3 * v]) / 3.0
+                detail[f"msssim{v}"] = m
+                detail[f"msssim{v}_db"] = -10.0 * math.log10(1.0 - m) if m < 1.0 else float("inf")
+        return r[6], psnr[0], psnr[1], detail
 
     def reconstructions(self, ticket: int):
         """(x1_hat, x2_hat) of a pair submitted with want_recon=True, as pinned HOST tensors (valid until the slot is

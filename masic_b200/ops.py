@@ -272,3 +272,44 @@ def nhwc_to_nchw_f32(x: torch.Tensor, c: Optional[int] = None, out: Optional[tor
     check(_lib.load().masic_nhwc_to_nchw_f32(x.data_ptr(), n, c, h * w, pitch, out.data_ptr(), _s()),
           "masic_nhwc_to_nchw_f32")
     return out
+
+
+# --------------------------------------------------------------------------- image quality
+MS_SSIM_WEIGHTS = (0.0448, 0.2856, 0.3001, 0.2363, 0.1333)     # pytorch_msssim's default level weights
+
+
+def ssim_per_channel(x: torch.Tensor, y: torch.Tensor, data_range: float, weights: Sequence[float],
+                     k: Tuple[float, float] = (0.01, 0.03), nonneg_last: bool = True) -> torch.Tensor:
+    """The (N, C) per-channel values of pytorch_msssim 1.0 on (N, C, H, W) fp32 CUDA tensors (csrc/msssim.cu):
+    len(weights) levels; ms_ssim is 5 levels with nonneg_last=True, ssim is weights=(1.0,)."""
+    _need_cuda(x, y)
+    if x.dtype != torch.float32 or y.dtype != torch.float32:
+        raise MasicError("masic_ms_ssim runs on float32 images only")
+    if x.dim() != 4 or x.shape != y.shape:
+        raise ValueError(f"ms_ssim needs two (N, C, H, W) tensors of one shape, got {tuple(x.shape)} and {tuple(y.shape)}")
+    x, y = x.contiguous(), y.contiguous()
+    n, c, h, w = x.shape
+    lib = _lib.load()
+    levels = len(weights)
+    nbytes = lib.masic_ms_ssim_scratch_bytes(n, c, h, w, levels)
+    check(min(int(nbytes), 0), f"masic_ms_ssim_scratch_bytes ({levels} levels of {h}x{w} need >= 11x11 each)")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+    out = torch.empty(n, c, dtype=torch.float32, device=x.device)
+    wts = (C.c_float * levels)(*map(float, weights))
+    check(lib.masic_ms_ssim(x.data_ptr(), y.data_ptr(), n, c, h, w, levels, float(data_range), float(k[0]), float(k[1]),
+                            wts, int(nonneg_last), scratch.data_ptr(), out.data_ptr(), _s()), "masic_ms_ssim")
+    return out
+
+
+def ms_ssim(x: torch.Tensor, y: torch.Tensor, data_range: float = 255, size_average: bool = True,
+            weights: Optional[Sequence[float]] = None, k: Tuple[float, float] = (0.01, 0.03)) -> torch.Tensor:
+    """pytorch_msssim.ms_ssim (1.0): the mean over (N, C), or over C only (shape (N,)) with size_average=False."""
+    v = ssim_per_channel(x, y, data_range, MS_SSIM_WEIGHTS if weights is None else weights, k, True)
+    return v.mean() if size_average else v.mean(1)
+
+
+def ssim(x: torch.Tensor, y: torch.Tensor, data_range: float = 255, size_average: bool = True,
+         k: Tuple[float, float] = (0.01, 0.03), nonnegative_ssim: bool = False) -> torch.Tensor:
+    """pytorch_msssim.ssim (1.0): single-scale SSIM, relu'd per channel with nonnegative_ssim=True."""
+    v = ssim_per_channel(x, y, data_range, (1.0,), k, nonnegative_ssim)
+    return v.mean() if size_average else v.mean(1)

@@ -16,6 +16,7 @@ PyTorch's "not differentiable" error instead of silently returning zeros.
     torch.ops.masic_b200.gc_build_indexes(scales, scale_table, scale_bound) -> Tensor(int32)
     torch.ops.masic_b200.quantize(x, means, symbols) -> Tensor
     torch.ops.masic_b200.eb_forward(z, matrices, biases, factors, quantiles) -> (z_hat, lik)
+    torch.ops.masic_b200.ms_ssim(x, y, data_range, weights, k1, k2, nonneg_last) -> Tensor(N, C)  pytorch_msssim
 """
 from __future__ import annotations
 
@@ -153,4 +154,20 @@ def _(z, matrices, biases, factors, quantiles):
     return torch.empty_like(z, dtype=torch.float32), torch.empty_like(z, dtype=torch.float32)
 
 
-OPS = ("conv2d", "gdn", "warp_perspective", "gmm_likelihood", "gc_likelihood", "gc_build_indexes", "quantize", "eb_forward")
+# ----------------------------------------------------------------------------- image quality
+@torch.library.custom_op(f"{NS}::ms_ssim", mutates_args=(), device_types="cuda")
+def ms_ssim(x: Tensor, y: Tensor, data_range: float, weights: List[float], k1: float, k2: float,
+            nonneg_last: bool) -> Tensor:
+    """pytorch_msssim 1.0 per (n, c): ms_ssim with the 5 level weights (nonneg_last=True), ssim with weights=[1.0]
+    (nonneg_last = nonnegative_ssim).  The reference's eval loop reports it per pair, test2_real.py:88-114."""
+    _cuda_only(x, y)
+    return ops.ssim_per_channel(x, y, data_range, weights, (k1, k2), nonneg_last)
+
+
+@ms_ssim.register_fake
+def _(x, y, data_range, weights, k1, k2, nonneg_last):
+    return x.new_empty((x.shape[0], x.shape[1]), dtype=torch.float32)
+
+
+OPS = ("conv2d", "gdn", "warp_perspective", "gmm_likelihood", "gc_likelihood", "gc_build_indexes", "quantize", "eb_forward",
+       "ms_ssim")
