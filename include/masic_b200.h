@@ -110,7 +110,9 @@ typedef struct MasicConvDesc {
   const int* nt_in_coff; const int* nt_out_coff; const int* nt_out_img; int out_images;
   /* 1: run the plan on CTA PAIRS (clusters of 2, tcgen05.mma.cta_group::2): each CTA stages half of every weight
    * k-block and the pair issues M = 256 MMAs, which cuts the weight traffic per SM.  Pays off on the 128 -> 128 5x5
-   * stride-2 layers and the wide 1x1 / 3x3 layers (-3..5 %), not on layers with few tiles or tiny K. */
+   * stride-2 layers and the wide 1x1 / 3x3 layers (-3..5 %), not on layers with few tiles or tiny K.
+   * Requires n_tile to be a multiple of 32 (each CTA then stages n_tile / 2 rows, a whole number of 16-wide N steps);
+   * other n_tile values with cta_pairs = 1 return MASIC_EINVAL. */
   int cta_pairs;
   /* 16-bit format of the input activations, the packed weights, gamma', the residuals and (unless out_fp32) the
    * output: MASIC_FMT_BF16 (training step: gradients need fp32's exponent range) or MASIC_FMT_F16 (inference engines:

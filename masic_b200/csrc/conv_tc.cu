@@ -1184,6 +1184,9 @@ extern "C" int masic_conv_plan_create(const MasicConvDesc* dp, MasicConvPlan** p
   if (d.n_tile % 16 || d.n_tile < 16 || d.n_tile > 256) return MASIC_EINVAL;
   if (d.c_out_pad % d.n_tile || d.c_out > d.c_out_pad) return MASIC_EINVAL;
   if (d.c_out_pad / d.n_tile > 32) return MASIC_EINVAL;
+  // CTA pairs split the N of the M = 256 MMA and every B k-block between the two CTAs (n_tile / 2 rows each); the
+  // pair kernel runs only where each half is a whole number of 16-wide N steps
+  if (d.cta_pairs && d.n_tile % 32) return MASIC_EINVAL;
   if (d.in_cpitch % 8 || d.in_coff % 8 || d.out_coff % 8) return MASIC_EINVAL;
   if ((d.kind == MASIC_CONV_XFOLD4 || d.kind == MASIC_CONV_XFOLD8) && d.c_in != 64) return MASIC_EINVAL;
   if (d.out_cpitch % (d.out_fp32 ? 4 : 8)) return MASIC_EINVAL;
