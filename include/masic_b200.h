@@ -42,7 +42,7 @@ extern "C" {
 #define MASIC_EDRIVER (-3)  /* cuTensorMapEncodeTiled unavailable / failed  */
 
 /* ---------------------------------------------------------------- version */
-int masic_abi_version(void);                 /* bumps on any signature change (2: residual inputs, 3: grouped launches of MasicConvDesc, 4: pack batches, 5: cta_pairs, 6: MASIC_CONV_XFOLD8, 7: masic_rans_*, udh front-end entry points, 8: `int f16` format selectors / MasicConvDesc.f16, 9: in_row_pixels / out_blk_images, 10: masic_warp_perspective_fwd3) */
+int masic_abi_version(void);                 /* bumps on any signature change (2: residual inputs, 3: grouped launches of MasicConvDesc, 4: pack batches, 5: cta_pairs, 6: MASIC_CONV_XFOLD8, 7: masic_rans_*, udh front-end entry points, 8: `int f16` format selectors / MasicConvDesc.f16, 9: in_row_pixels / out_blk_images, 10: masic_warp_perspective_fwd3, 11: one masic_warp_perspective_fwd (fwd2/fwd3 folded in)) */
 const char* masic_build_info(void);          /* "sm_100a nvcc 12.9 ..." */
 
 /* ------------------------------------------------------------------ convs */
@@ -357,27 +357,21 @@ int masic_homography_from_delta(const float* corners, const float* delta, int ba
 int masic_warp_prepare(const float* m_3x3, int batch, int h, int w, int h_out, int w_out, int invert_m,
                        double* t_out, void* stream);
 /* Step 2: bilinear, zero padding, align_corners=True.  src NCHW fp32 with c <= 8 channels;
- * src == NULL warps an all-ones image (mask(), MASIC.py:636-638).  Outputs: NCHW fp32 and/or
- * NHWC bf16 zero-padded to bf_pitch channels. */
+ * src == NULL warps an all-ones image (mask(), MASIC.py:636-638).  Outputs (any may be NULL, not all):
+ *   dst_nchw       NCHW fp32;
+ *   dst_nhwc_bf16  NHWC 16-bit (format f16) zero-padded to bf_pitch channels, rows as in the layout packs below;
+ *   dst2_nhwc16    a second 16-bit NHWC image (plain MASIC_FMT_BF16 / MASIC_FMT_F16 in d2_f16): the c warped channels
+ *                  are written at channel d2_coff of pixel slot (y * d2_row_pixels + x + d2_xoff) * d2_pitch, leaving
+ *                  the slot's other channels untouched — several producers fill one channels-last image (the input of
+ *                  the tensor-core after_conv).  With c = 3 and d2_coff, d2_pitch multiples of 4 the pixel is ONE
+ *                  8-byte store [c0 c1 c2 0] (channel d2_coff + 3 is zeroed);
+ *   dst_ones_nchw  (n,1,h_out,w_out): the warp of the ALL-ONES image under the same transform (mask(),
+ *                  MASIC.py:636-638: x1_mask_R) from the same launch — the coordinates are evaluated once for both. */
 int masic_warp_perspective_fwd(const float* src, int n, int c, int h, int w, int h_out, int w_out,
-                               const double* t_prepared, float* dst_nchw, void* dst_nhwc_bf16,
-                               int bf_pitch, int bf_row_pixels, int bf_xoff, int f16, void* stream);
-
-/* Same, with a second 16-bit NHWC destination (plain MASIC_FMT_BF16 / MASIC_FMT_F16): the c warped channels are written at
- * channel d2_coff of pixel slot (y * d2_row_pixels + x + d2_xoff) * d2_pitch, leaving the slot's other channels
- * untouched — several producers fill one channels-last image (the input of the tensor-core after_conv).  With c = 3
- * and d2_coff, d2_pitch multiples of 4 the pixel is ONE 8-byte store [c0 c1 c2 0] (channel d2_coff + 3 is zeroed). */
-int masic_warp_perspective_fwd2(const float* src, int n, int c, int h, int w, int h_out, int w_out,
-                                const double* t_prepared, float* dst_nchw, void* dst_nhwc_bf16, int bf_pitch,
-                                int bf_row_pixels, int bf_xoff, int f16, void* dst2_nhwc16, int d2_pitch,
-                                int d2_row_pixels, int d2_xoff, int d2_coff, int d2_f16, void* stream);
-/* Same, and the warp of the ALL-ONES image under the same transform (mask(), MASIC.py:636-638: x1_mask_R) written to
- * dst_ones_nchw (n,1,h_out,w_out) from the same launch — the coordinates are evaluated once for both (NULL = fwd2). */
-int masic_warp_perspective_fwd3(const float* src, int n, int c, int h, int w, int h_out, int w_out,
-                                const double* t_prepared, float* dst_nchw, void* dst_nhwc_bf16, int bf_pitch,
-                                int bf_row_pixels, int bf_xoff, int f16, void* dst2_nhwc16, int d2_pitch,
-                                int d2_row_pixels, int d2_xoff, int d2_coff, int d2_f16, float* dst_ones_nchw,
-                                void* stream);
+                               const double* t_prepared, float* dst_nchw, void* dst_nhwc_bf16, int bf_pitch,
+                               int bf_row_pixels, int bf_xoff, int f16, void* dst2_nhwc16, int d2_pitch,
+                               int d2_row_pixels, int d2_xoff, int d2_coff, int d2_f16, float* dst_ones_nchw,
+                               void* stream);
 
 /* Direct conv for the tiny-channel layers (c_in <= 8, c_out <= 8) on NCHW fp32:
  *   Encoder2.pre_conv+pre_gdn (MASIC.py:573-574): in0=x1_warp, in1=x2, k=5, s=1, gdn=FWD
@@ -412,8 +406,8 @@ int masic_softmax_channels(const float* in_nchw, int n, int c, int hw, float* ou
 int masic_mask2weights(const float* mask_nchw, int n, int h, int w, const float* w1, const float* b1, const float* w2,
                        const float* b2, const float* w3, const float* b3, const float* w4, const float* b4,
                        float* out_nchw, float* out_nhwc, void* stream);
-/* layout packs.  The NHWC bf16 outputs of this function, of masic_warp_perspective_fwd and of
- * masic_conv_small_nchw may have a padded row: pixel (y,x) goes to out[(y*row_pixels + x + xoff)*pitch];
+/* layout packs.  The NHWC bf16 outputs of this function, of masic_warp_perspective_fwd (both 16-bit destinations) and
+ * of masic_conv_small_nchw may have a padded row: pixel (y,x) goes to out[(y*row_pixels + x + xoff)*pitch];
  * row_pixels = 0 means a dense image (row_pixels = w, xoff = 0). */
 int masic_nchw_to_nhwc_bf16(const float* in_nchw, int n, int c, int h, int w, void* out, int pitch,
                             int row_pixels, int xoff, int f16, void* stream);

@@ -157,9 +157,7 @@ def _declare(lib: C.CDLL) -> None:
         "masic_fc_bf16": (i, [vp, i, vp, vp, i, i, i, i, vp, vp, i, i, vp]),
         "masic_homography_from_delta": (i, [vp, vp, i, i, i, i, i, i, vp, vp]),
         "masic_warp_prepare": (i, [vp, i, i, i, i, i, i, vp, vp]),
-        "masic_warp_perspective_fwd": (i, [vp, i, i, i, i, i, i, vp, vp, vp, i, i, i, i, vp]),
-        "masic_warp_perspective_fwd2": (i, [vp, i, i, i, i, i, i, vp, vp, vp, i, i, i, i, vp, i, i, i, i, i, vp]),
-        "masic_warp_perspective_fwd3": (i, [vp, i, i, i, i, i, i, vp, vp, vp, i, i, i, i, vp, i, i, i, i, i, vp, vp]),
+        "masic_warp_perspective_fwd": (i, [vp, i, i, i, i, i, i, vp, vp, vp, i, i, i, i, vp, i, i, i, i, i, vp, vp]),
         "masic_conv_small_nchw": (i, [vp, i, vp, i, i, i, i, vp, i, vp, i, i, i, i, i, vp, vp, f, vp, vp, i, i, i, i, vp]),
         "masic_mask2weights": (i, [vp, i, i, i, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
         "masic_subpix_to_nchw": (i, [vp, i, i, i, i, i, vp, vp, f, vp, vp, i, i, vp]),

@@ -13,20 +13,18 @@ The whole sequence replays as one CUDA graph.  No CPU path.
 """
 from __future__ import annotations
 
-import ctypes as C
 from typing import Dict, Tuple
 
 import torch
 import torch.nn as nn
 
-from . import _lib
-from ._lib import MasicError, check
+from . import _lib, ops
+from ._lib import MasicError
 from .convplan import ACT_LEAKY, ACT_NONE, ACT_RELU, CONV, ConvPlan, PackedConv
 from .engine import HSICEngine
 from .layers import ResidualBlock, conv, conv3x3
 
 F16 = _lib.FMT_F16              # inference runs on fp16 operands / activations (csrc/cvt16.cuh)
-ACT = _lib.act_dtype(F16)
 
 
 class Enhancement_Block(nn.Module):
@@ -54,7 +52,6 @@ class mask2weights_EN(nn.Module):
             conv(in_channels=Kw * 2, out_channels=Kw, kernel_size=3, stride=1))
 
     def forward(self, allconcat):
-        from . import ops
         x = allconcat
         for i in (0, 2, 4, 6):
             m = self.maskconv[i]
@@ -172,46 +169,40 @@ class CQEEngine(HSICEngine):
     # ------------------------------------------------------------------ the plan
     def _build(self):
         B, H, W = self.B, self.H, self.W
-        f32, lib, hw = torch.float32, self.lib, H * W
+        f32 = torch.float32
         self.x1 = self._buf(B, 3, H, W, dtype=f32)       # inputs: the codec's reconstructions
         self.x2 = self._buf(B, 3, H, W, dtype=f32)
         self.Hm = torch.eye(3, device=self.dev).repeat(B, 1, 1).contiguous()
         o = self.out = {"x1_hat": self._buf(B, 3, H, W, dtype=f32), "x2_hat": self._buf(B, 3, H, W, dtype=f32)}
         T = torch.empty(B, 3, 3, device=self.dev, dtype=torch.float64)
         Tinv = torch.empty(B, 3, 3, device=self.dev, dtype=torch.float64)
-        self._add("warp.prepare", lambda: (
-            check(lib.masic_warp_prepare(self.Hm.data_ptr(), B, H, W, H, W, 0, T.data_ptr(), self._s()), "masic_warp_prepare"),
-            check(lib.masic_warp_prepare(self.Hm.data_ptr(), B, H, W, H, W, 1, Tinv.data_ptr(), self._s()), "masic_warp_prepare")))
+        self._add("warp.prepare", lambda: (ops.warp_prepare_into(self.Hm, T, (H, W), (H, W)),
+                                           ops.warp_prepare_into(self.Hm, Tinv, (H, W), (H, W), invert=True)))
 
-        def warp(tag, src, Tm, dst, channels):
-            self._add(tag, lambda: check(lib.masic_warp_perspective_fwd(
-                None if src is None else src.data_ptr(), B, channels, H, W, H, W, Tm.data_ptr(), dst.data_ptr(), None, 0, 0,
-                0, F16, self._s()), "masic_warp_perspective_fwd"))
+        def warp(tag, src, Tm, dst):
+            self._add(tag, lambda: ops.warp_perspective_into(src, Tm, (H, W), src_shape=dst.shape, dst=dst))
 
         # masks (MASIC.py:1458 -> :627-649) and the per-pixel blend weights (:1459-1460)
         mask_r = self._buf(B, 1, H, W, dtype=f32)
         mask_l = self._buf(B, 1, H, W, dtype=f32)
-        warp("mask_R=warp(ones)", None, T, mask_r, 1)
-        warp("mask_L=warp(mask_R,Hinv)", mask_r, Tinv, mask_l, 1)
+        warp("mask_R=warp(ones)", None, T, mask_r)
+        warp("mask_L=warp(mask_R,Hinv)", mask_r, Tinv, mask_l)
         mk = "mask2weights_unit.maskconv"
         wts = {}
         mws = [self._w(f"{mk}.{i}.weight") for i in (0, 2, 4, 6)]
         mbs = [self._w(f"{mk}.{i}.bias") for i in (0, 2, 4, 6)]
-        self._keep += [mws, mbs]
-        pw = (C.c_void_p * 4)(*[t.data_ptr() for t in mws])
-        pb = (C.c_void_p * 4)(*[t.data_ptr() for t in mbs])
         for side, m in (("R", mask_r), ("L", mask_l)):
             wt = self._buf(B, 2, H, W, dtype=f32)
-            self._add(f"mask2weights_{side}(4 convs+softmax)", (lambda m=m, wt=wt: check(lib.masic_cqe_mask_weights(
-                m.data_ptr(), B, H, W, pw, pb, 2, wt.data_ptr(), self._s()), "masic_cqe_mask_weights")))
+            self._add(f"mask2weights_{side}(4 convs+softmax)",
+                      lambda m=m, wt=wt: ops.cqe_mask_weights_into(m, mws, mbs, wt))
             wts[side] = wt
         self.buf["w_R"], self.buf["w_L"] = wts["R"], wts["L"]
 
         # warped images (:1461, :1464) and bf16 NHWC copies of the inputs
         x1w = self._buf(B, 3, H, W, dtype=f32)
         x2w = self._buf(B, 3, H, W, dtype=f32)
-        warp("warp(x1_hat,H)", self.x1, T, x1w, 3)
-        warp("warp(x2_hat,Hinv)", self.x2, Tinv, x2w, 3)
+        warp("warp(x1_hat,H)", self.x1, T, x1w)
+        warp("warp(x2_hat,Hinv)", self.x2, Tinv, x2w)
         p_conv0 = self._pack3("conv0", 16, 32, 32, real_cin=3)
         p_conv1 = self._pack3("conv1", 16, 32, 32, real_cin=6)
         p_conv2 = self._pack3("conv2", 96, 3, 16)
@@ -221,14 +212,12 @@ class CQEEngine(HSICEngine):
         cat96 = {}
         for v, eb, x_self, x_other_w, wt, _, _ in views:
             xbf = self._buf(B, H, W, 16)
-            self._add(f"{v}.pack_nhwc", (lambda x_self=x_self, xbf=xbf: check(lib.masic_nchw_to_nhwc_bf16(
-                x_self.data_ptr(), B, 3, H, W, xbf.data_ptr(), 16, 0, 0, F16, self._s()), "masic_nchw_to_nhwc_bf16")))
+            self._add(f"{v}.pack_nhwc", lambda x_self=x_self, xbf=xbf: ops.nchw_to_nhwc_into(x_self, xbf))
             cat96[v] = self._buf(B, H, W, 96)                 # [EB2 output | conv0(x)]  (:1486-1487)
             self._c3(f"{v}.conv0", p_conv0, xbf, cat96[v], out_coff=64)                      # :1467-1468
             blend = self._buf(B, H, W, 16)
-            self._add(f"{v}.blend_images", (lambda a=x_other_w, b=x_self, wt=wt, blend=blend: check(
-                lib.masic_cqe_blend_images(a.data_ptr(), b.data_ptr(), wt.data_ptr(), B, H, W, blend.data_ptr(), F16, self._s()),
-                "masic_cqe_blend_images")))                                                 # :1470-1471
+            self._add(f"{v}.blend_images", lambda a=x_other_w, b=x_self, wt=wt, blend=blend:
+                      ops.cqe_blend_images_into(a, b, wt, blend))                           # :1470-1471
             f1 = self._buf(B, H, W, 32)
             self._c3(f"{v}.conv1", p_conv1, blend, f1)                                       # :1473-1474
             e1[v] = self._buf(B, H, W, 32)
@@ -236,15 +225,13 @@ class CQEEngine(HSICEngine):
         for v, eb, x_self, _, wt, Tm, okey in views:
             other = "R" if v == "L" else "L"
             fused = self._buf(B, H, W, 64)
-            self._add(f"{v}.feature_fuse", (lambda s=e1[v], ot=e1[other], wt=wt, Tm=Tm, fused=fused: check(
-                lib.masic_cqe_feature_fuse(s.data_ptr(), 32, ot.data_ptr(), 32, 32, wt.data_ptr(), Tm.data_ptr(), B, H, W,
-                                           fused.data_ptr(), 64, F16, self._s()), "masic_cqe_feature_fuse")))   # :1479-1482
+            self._add(f"{v}.feature_fuse", lambda s=e1[v], ot=e1[other], wt=wt, Tm=Tm, fused=fused:
+                      ops.cqe_feature_fuse_into(s, ot, wt, Tm, fused))                      # :1479-1482
             self._enh_block(f"{v}.EB2", f"{eb}2", 64, fused, cat96[v], out_coff=0)           # :1483-1484
             e3 = self._buf(B, H, W, 96)
             self._enh_block(f"{v}.EB3", f"{eb}3", 96, cat96[v], e3)                          # :1488-1489
             c2 = self._buf(B, H, W, 16, dtype=f32)
             self._c3(f"{v}.conv2", p_conv2, e3, c2)                                          # :1491-1492
-            self._add(f"{v}.residual_image", (lambda c2=c2, x_self=x_self, dst=o[okey]: check(
-                lib.masic_cqe_residual_image(c2.data_ptr(), 16, x_self.data_ptr(), B, H, W, dst.data_ptr(), self._s()),
-                "masic_cqe_residual_image")))                                               # :1495-1496
+            self._add(f"{v}.residual_image", lambda c2=c2, x_self=x_self, dst=o[okey]:
+                      ops.cqe_residual_image_into(c2, x_self, dst))                         # :1495-1496
         self.flops = sum(p.flops for p in self.plans.values())

@@ -30,14 +30,13 @@ No CPU fallback: everything raises on non-CUDA tensors.
 """
 from __future__ import annotations
 
-import ctypes as C
 from typing import Dict, List, Optional
 
 import torch
 
-from . import _lib
+from . import _lib, ops
 from . import train_ops as T
-from ._lib import MasicError, check
+from ._lib import MasicError
 from .convplan import ACT_LEAKY, ACT_NONE, ACT_RELU
 from .trainer import BF, F32, TrainStep, _Layer
 
@@ -112,26 +111,23 @@ class CQETrainer(TrainStep):
     # ------------------------------------------------------------------ the plan
     def _build(self):
         B, H, W = self.B, self.H, self.W
-        lib, dev, hw = self.lib, self.dev, H * W
-        s = T._s
+        dev, hw = self.dev, H * W
         self.x1_hat, self.x2_hat = self._z(B, 3, H, W, dtype=F32), self._z(B, 3, H, W, dtype=F32)
         self.x1, self.x2 = self._z(B, 3, H, W, dtype=F32), self._z(B, 3, H, W, dtype=F32)
         self.Hm = torch.eye(3, device=dev).repeat(B, 1, 1).contiguous()
         o = self.out = {"x1_hat": self._z(B, 3, H, W, dtype=F32), "x2_hat": self._z(B, 3, H, W, dtype=F32)}
         Tm = torch.empty(B, 3, 3, device=dev, dtype=torch.float64)
         Tinv = torch.empty(B, 3, 3, device=dev, dtype=torch.float64)
-        self.F("warp.prepare", lambda: (
-            check(lib.masic_warp_prepare(self.Hm.data_ptr(), B, H, W, H, W, 0, Tm.data_ptr(), s()), "masic_warp_prepare"),
-            check(lib.masic_warp_prepare(self.Hm.data_ptr(), B, H, W, H, W, 1, Tinv.data_ptr(), s()), "masic_warp_prepare")))
+        self.F("warp.prepare", lambda: (ops.warp_prepare_into(self.Hm, Tm, (H, W), (H, W)),
+                                        ops.warp_prepare_into(self.Hm, Tinv, (H, W), (H, W), invert=True)))
 
-        def warp(src, Tw, dst, ch):
-            check(lib.masic_warp_perspective_fwd(None if src is None else src.data_ptr(), B, ch, H, W, H, W, Tw.data_ptr(),
-                                                 dst.data_ptr(), None, 0, 0, 0, 0, s()), "masic_warp_perspective_fwd")
+        def warp(src, Tw, dst):
+            ops.warp_perspective_into(src, Tw, (H, W), src_shape=dst.shape, dst=dst)
 
         # masks (MASIC.py:1458 -> :627-649) and mask2weights_EN (:1459-1460, :1411-1434), layer by layer so that the
         # backward has the intermediates; weights as NCHW (blends) and NHWC (softmax backward)
         mask_r, mask_l = self._z(B, 1, H, W, dtype=F32), self._z(B, 1, H, W, dtype=F32)
-        self.F("masks", lambda: (warp(None, Tm, mask_r, 1), warp(mask_r, Tinv, mask_l, 1)))
+        self.F("masks", lambda: (warp(None, Tm, mask_r), warp(mask_r, Tinv, mask_l)))
         mk = "mask2weights_unit.maskconv"
         mk_w = [self.param(f"{mk}.{2 * i}.weight") for i in range(4)]
         mk_b = [self.param(f"{mk}.{2 * i}.bias") for i in range(4)]
@@ -145,13 +141,10 @@ class CQETrainer(TrainStep):
             side[v] = {"kb": kb, "gk": gk, "wt": wt, "wt_nhwc": wt_nhwc, "dwt": dwt}
 
             def mask_fwd(kb=kb, wt=wt, wt_nhwc=wt_nhwc):
-                for i, (ci, co) in enumerate(MASK_CH):
-                    check(lib.masic_conv_small_nchw(kb[i].data_ptr(), ci, None, 0, B, H, W, mk_w[i].data_ptr(), 0,
-                                                    mk_b[i].data_ptr(), co, 3, 1, ACT_RELU if i < 3 else ACT_NONE, 0, None,
-                                                    None, 1e-6, kb[i + 1].data_ptr(), None, 0, 0, 0, 0, s()),
-                          "masic_conv_small_nchw")
-                check(lib.masic_softmax_channels(kb[4].data_ptr(), B, 2, hw, wt.data_ptr(), wt_nhwc.data_ptr(), s()),
-                      "masic_softmax_channels")
+                for i in range(4):
+                    ops.conv_small_into(kb[i], None, mk_w[i], mk_b[i], ksize=3, stride=1,
+                                        act=ACT_RELU if i < 3 else ACT_NONE, out=kb[i + 1])
+                ops.softmax_channels_into(kb[4], wt, wt_nhwc)
             self.F(f"{v}.mask2weights", mask_fwd)
 
         # padded copies of the small-channel layers (16-channel pitches, as CQEEngine._pack3)
@@ -164,8 +157,8 @@ class CQETrainer(TrainStep):
         db2 = self.grad("conv2.bias")
 
         x_other_w = {"L": self._z(B, 3, H, W, dtype=F32), "R": self._z(B, 3, H, W, dtype=F32)}
-        self.F("warp(x2_hat,Hinv)", lambda: warp(self.x2_hat, Tinv, x_other_w["L"], 3))              # :1464
-        self.F("warp(x1_hat,H)", lambda: warp(self.x1_hat, Tm, x_other_w["R"], 3))                   # :1461
+        self.F("warp(x2_hat,Hinv)", lambda: warp(self.x2_hat, Tinv, x_other_w["L"]))                 # :1464
+        self.F("warp(x1_hat,H)", lambda: warp(self.x1_hat, Tm, x_other_w["R"]))                      # :1461
         views = {"L": ("EBl", self.x1_hat, self.x1, Tinv, "x1_hat"), "R": ("EBr", self.x2_hat, self.x2, Tm, "x2_hat")}
         d: Dict[str, dict] = {}
         first: Dict[str, _Layer] = {}
@@ -185,11 +178,9 @@ class CQETrainer(TrainStep):
             e["xbf"], e["blend"] = xbf, blend
 
             def front(xs=xs, xbf=xbf, blend=blend, e=e, v=v):
-                check(lib.masic_nchw_to_nhwc_bf16(xs.data_ptr(), B, 3, H, W, xbf.data_ptr(), 16, 0, 0, 0, s()),
-                      "masic_nchw_to_nhwc_bf16")
+                ops.nchw_to_nhwc_into(xs, xbf)
                 e["conv0"].fwd()                                                                     # :1467-1468
-                check(lib.masic_cqe_blend_images(x_other_w[v].data_ptr(), xs.data_ptr(), side[v]["wt"].data_ptr(), B, H,
-                                                 W, blend.data_ptr(), 0, s()), "masic_cqe_blend_images")  # :1470-1471
+                ops.cqe_blend_images_into(x_other_w[v], xs, side[v]["wt"], blend)                    # :1470-1471
                 e["conv1"].fwd()                                                                     # :1473-1474
                 e["eb1"][0]()                                                                        # :1476-1477
             self.F(f"{v}.front", front)
@@ -206,25 +197,18 @@ class CQETrainer(TrainStep):
             first.setdefault("conv2", e["conv2"])
 
             def back(e=e, other=other, v=v, Tv=Tv, xs=xs, okey=okey):
-                check(lib.masic_cqe_feature_fuse(e["e1"].data_ptr(), 32, other["e1"].data_ptr(), 32, 32,
-                                                 side[v]["wt"].data_ptr(), Tv.data_ptr(), B, H, W, e["fused"].data_ptr(), 64,
-                                                 0, s()), "masic_cqe_feature_fuse")                    # :1479-1482
+                ops.cqe_feature_fuse_into(e["e1"], other["e1"], side[v]["wt"], Tv, e["fused"])        # :1479-1482
                 e["eb2"][0]()                                                                        # :1483-1487
                 e["eb3"][0]()                                                                        # :1488-1489
                 e["conv2"].fwd()                                                                     # :1491-1492
-                check(lib.masic_cqe_residual_image(e["c2"].data_ptr(), 16, xs.data_ptr(), B, H, W, o[okey].data_ptr(),
-                                                   s()), "masic_cqe_residual_image")                 # :1495-1496
+                ops.cqe_residual_image_into(e["c2"], xs, o[okey])                                    # :1495-1496
             self.F(f"{v}.back", back)
 
         # ================= loss: lambda * 255^2 * (mse1 + mse2), masic_rd_metrics without likelihoods
         self.rd_out = self._z(8, dtype=F32)
-        self.rd_scratch = torch.empty(lib.masic_rd_metrics_scratch_bytes() // 8, dtype=torch.float64, device=dev)
-        lp = (C.c_void_p * 4)(None, None, None, None)
-        ln = (C.c_int64 * 4)(0, 0, 0, 0)
-        self.F("loss", lambda: check(lib.masic_rd_metrics(lp, ln, o["x1_hat"].data_ptr(), self.x1.data_ptr(),
-                                                          o["x2_hat"].data_ptr(), self.x2.data_ptr(), B, 3, H, W, self.lmbda,
-                                                          self.rd_scratch.data_ptr(), self.rd_out.data_ptr(), s()),
-                                     "masic_rd_metrics"))
+        self.rd_scratch = ops.rd_metrics_scratch(dev)
+        self.F("loss", lambda: ops.rd_metrics_into([None] * 4, o["x1_hat"], self.x1, o["x2_hat"], self.x2, self.lmbda,
+                                                   self.rd_scratch, self.rd_out))
 
         # ================= backward
         mse_scale = self.lmbda * 255.0 ** 2 * 2.0 / (B * 3 * H * W)
@@ -234,8 +218,7 @@ class CQETrainer(TrainStep):
 
             def tail_bwd(e=e, gimg=gimg, target=target, okey=okey):
                 T.mse_grad(o[okey], target, mse_scale, gimg)
-                check(lib.masic_nchw_to_nhwc_bf16(gimg.data_ptr(), B, 3, H, W, e["gc2"].data_ptr(), 16, 0, 0, 0, s()),
-                      "masic_nchw_to_nhwc_bf16")
+                ops.nchw_to_nhwc_into(gimg, e["gc2"])
                 T.colsum_nchw(gimg, db2)
                 e["conv2"].bwd(skip_act=True)
                 e["eb3"][1]()

@@ -823,29 +823,11 @@ extern "C" int masic_warp_prepare(const float* m_3x3, int batch, int h, int w, i
   return (int)cudaGetLastError();
 }
 
-extern "C" int masic_warp_perspective_fwd(const float* src, int n, int c, int h, int w, int h_out,
-                                          int w_out, const double* t_prepared, float* dst_nchw,
-                                          void* dst_nhwc_bf16, int bf_pitch, int bf_row_pixels, int bf_xoff,
-                                          int f16, void* stream) {
-  return masic_warp_perspective_fwd2(src, n, c, h, w, h_out, w_out, t_prepared, dst_nchw, dst_nhwc_bf16, bf_pitch,
-                                     bf_row_pixels, bf_xoff, f16, nullptr, 0, 0, 0, 0, 0, stream);
-}
-
-extern "C" int masic_warp_perspective_fwd2(const float* src, int n, int c, int h, int w, int h_out, int w_out,
-                                           const double* t_prepared, float* dst_nchw, void* dst_nhwc_bf16,
-                                           int bf_pitch, int bf_row_pixels, int bf_xoff, int f16, void* dst2_nhwc16,
-                                           int d2_pitch, int d2_row_pixels, int d2_xoff, int d2_coff, int d2_f16,
-                                           void* stream) {
-  return masic_warp_perspective_fwd3(src, n, c, h, w, h_out, w_out, t_prepared, dst_nchw, dst_nhwc_bf16, bf_pitch,
-                                     bf_row_pixels, bf_xoff, f16, dst2_nhwc16, d2_pitch, d2_row_pixels, d2_xoff, d2_coff,
-                                     d2_f16, nullptr, stream);
-}
-
-extern "C" int masic_warp_perspective_fwd3(const float* src, int n, int c, int h, int w, int h_out, int w_out,
-                                           const double* t_prepared, float* dst_nchw, void* dst_nhwc_bf16,
-                                           int bf_pitch, int bf_row_pixels, int bf_xoff, int f16, void* dst2_nhwc16,
-                                           int d2_pitch, int d2_row_pixels, int d2_xoff, int d2_coff, int d2_f16,
-                                           float* dst_ones_nchw, void* stream) {
+extern "C" int masic_warp_perspective_fwd(const float* src, int n, int c, int h, int w, int h_out, int w_out,
+                                          const double* t_prepared, float* dst_nchw, void* dst_nhwc_bf16,
+                                          int bf_pitch, int bf_row_pixels, int bf_xoff, int f16, void* dst2_nhwc16,
+                                          int d2_pitch, int d2_row_pixels, int d2_xoff, int d2_coff, int d2_f16,
+                                          float* dst_ones_nchw, void* stream) {
   if (!t_prepared || n <= 0 || c <= 0 || c > 8 || (!dst_nchw && !dst_nhwc_bf16 && !dst2_nhwc16 && !dst_ones_nchw))
     return MASIC_EINVAL;
   if (bf_row_pixels == 0) { bf_row_pixels = w_out; bf_xoff = 0; }

@@ -24,17 +24,16 @@ from typing import Callable, Dict, List, Optional, Tuple
 
 import torch
 
-from . import _lib
+from . import _lib, ops
 from ._lib import MasicError, check
 from .convplan import (ACT_LEAKY, ACT_NONE, ACT_RELU, CONV, CONV_XFOLD8, DECONV_S2, GDN_FWD, GDN_INV,
                        GDN_NONE, MASK_A_5x5, ConvPlan, DeconvImgPlan, PackedConv, fold8_weights_5x5_s1)
 
 F16 = _lib.FMT_F16              # the inference engines run on fp16 operands / activations (csrc/cvt16.cuh)
 ACT = _lib.act_dtype(F16)
-F16_IMG = F16 | _lib.FMT_SPLIT   # images feeding g_a_conv1: pixels stored as [hi(3) | lo(3) | 0 0] (MASIC_FMT_SPLIT)
 SCALE_BOUND = 0.11
-IMG_CP = 8           # channel pitch of the bf16 images feeding g_a_conv1 (3 real channels); rows are padded:
-XOFF, XPAD = _lib.IMG_XOFF, _lib.IMG_XPAD   # [N][H][W+XPAD][8], pixel x at column x+XOFF (MASIC_CONV_XFOLD8 input)
+IMG_CP = 8           # channel pitch of the 16-bit images feeding g_a_conv1 (3 real channels, stored split: [hi | lo]);
+XOFF, XPAD = _lib.IMG_XOFF, _lib.IMG_XPAD   # rows padded: [N][H][W+XPAD][8], pixel x at column x+XOFF (XFOLD8 input)
 
 
 class HSICEngine:
@@ -291,57 +290,11 @@ class HSICEngine:
                   "masic_latent_prep")
         self._add(f"{tag}.latent_prep", step)
 
-    def _warp(self, tag, src, T, dst, dst_bf=None, channels=3, dst2=None, dst2_coff=0, ones=None):
-        """dst: NCHW fp32; dst_bf: hi|lo image for g_a_conv1; dst2: plain 16-bit copy at channel dst2_coff of a shared
-        channels-last image (the tensor-core after_conv's input); ones: the warp of the all-ones image under the same
-        transform (x1_mask_R, MASIC.py:636-638) from the same launch.  Any of them may be None."""
-        B, H, W = self.B, self.H, self.W
-
-        def step():
-            check(self.lib.masic_warp_perspective_fwd3(None if src is None else src.data_ptr(), B, channels, H, W, H, W,
-                                                       T.data_ptr(), None if dst is None else dst.data_ptr(),
-                                                       None if dst_bf is None else dst_bf.data_ptr(),
-                                                       0 if dst_bf is None else dst_bf.shape[3],
-                                                       0 if dst_bf is None else dst_bf.shape[2],
-                                                       0 if dst_bf is None else XOFF, F16_IMG,
-                                                       None if dst2 is None else dst2.data_ptr(),
-                                                       0 if dst2 is None else dst2.shape[3],
-                                                       0 if dst2 is None else dst2.shape[2],
-                                                       0 if dst2 is None else XOFF, dst2_coff, F16,
-                                                       None if ones is None else ones.data_ptr(), self._s()),
-                  "masic_warp_perspective_fwd3")
-        self._add(tag, step)
-
-    def _conv_small(self, tag, in0, in1, wname, *, ksize, stride, act=ACT_NONE, gdn=GDN_NONE,
-                    gdn_prefix=None, out=None, out_bf=None):
-        w = self._w(wname + ".weight")
-        b = self._w(wname + ".bias")
-        beta = self._w(gdn_prefix + ".beta") if gdn else None
-        gamma = self._w(gdn_prefix + ".gamma") if gdn else None
-        self._keep += [w, b, beta, gamma]
-        n, c0, h, wd = in0.shape
-        c1 = 0 if in1 is None else in1.shape[1]
-        c_out = w.shape[0]
-
-        def step():
-            check(self.lib.masic_conv_small_nchw(in0.data_ptr(), c0, None if in1 is None else in1.data_ptr(), c1, n, h,
-                                                 wd, w.data_ptr(), 0, b.data_ptr(), c_out, ksize,
-                                                 stride, act, gdn, None if beta is None else beta.data_ptr(),
-                                                 None if gamma is None else gamma.data_ptr(), 1e-6,
-                                                 None if out is None else out.data_ptr(),
-                                                 None if out_bf is None else out_bf.data_ptr(),
-                                                 0 if out_bf is None else out_bf.shape[3],
-                                                 0 if out_bf is None else out_bf.shape[2],
-                                                 0 if out_bf is None else XOFF, F16_IMG, self._s()),
-                  "masic_conv_small_nchw")
-        self._add(tag, step)
-
     # ------------------------------------------------------------------ the plan
     def _build(self):
         B, H, W, N, M, K = self.B, self.H, self.W, self.N, self.M, self.K
         h16, w16 = H // 16, W // 16
         f32 = torch.float32
-        lib = self.lib
         # static inputs / outputs (NCHW fp32, the reference's tensor format)
         self.x1 = self._buf(B, 3, H, W, dtype=f32)
         self.x2 = self._buf(B, 3, H, W, dtype=f32)
@@ -356,8 +309,7 @@ class HSICEngine:
         # ---------------- lane 0: left encoder (MASIC.py:746, :755)
         self._on(0)
         x1_bf = self._buf(B, H, W + XPAD, IMG_CP)
-        self._add("x1.pack_nhwc", lambda: check(lib.masic_nchw_to_nhwc_bf16(
-            self.x1.data_ptr(), B, 3, H, W, x1_bf.data_ptr(), IMG_CP, W + XPAD, XOFF, F16_IMG, self._s()), "masic_nchw_to_nhwc_bf16"))
+        self._add("x1.pack_nhwc", lambda: ops.nchw_to_nhwc_into(self.x1, x1_bf, split=True))
         enc1 = self._encoder_weights("encoder1")
         y1 = self._encoder("L.g_a", enc1, x1_bf)
         y1_abs = self._buf(B, h16, w16, M)
@@ -371,28 +323,30 @@ class HSICEngine:
         self._on(2)
         T = torch.empty(B, 3, 3, device=self.dev, dtype=torch.float64)
         Tinv = torch.empty(B, 3, 3, device=self.dev, dtype=torch.float64)
-        self._add("warp.prepare", lambda: (
-            check(lib.masic_warp_prepare(self.Hm.data_ptr(), B, H, W, H, W, 0, T.data_ptr(), self._s()), "masic_warp_prepare"),
-            check(lib.masic_warp_prepare(self.Hm.data_ptr(), B, H, W, H, W, 1, Tinv.data_ptr(), self._s()), "masic_warp_prepare")))
+        self._add("warp.prepare", lambda: (ops.warp_prepare_into(self.Hm, T, (H, W), (H, W)),
+                                           ops.warp_prepare_into(self.Hm, Tinv, (H, W), (H, W), invert=True)))
         self._record("T")
         # x1 and the all-ones image are warped by ONE launch (same transform: the fp64 coordinates, ~60 % of the kernel's
         # instructions, are evaluated once)
         x1_warp = self._buf(B, 3, H, W, dtype=f32)
-        self._warp("R.warp(x1)+mask_R", self.x1, T, x1_warp, ones=o["x1_mask_R"])
-        self._warp("mask_L=warp(mask_R,Hinv)", o["x1_mask_R"], Tinv, o["x1_mask_L"], channels=1)
+        self._add("R.warp(x1)+mask_R", lambda: ops.warp_perspective_into(self.x1, T, (H, W), dst=x1_warp,
+                                                                         ones=o["x1_mask_R"]))
+        self._add("mask_L=warp(mask_R,Hinv)", lambda: ops.warp_perspective_into(o["x1_mask_R"], Tinv, (H, W),
+                                                                                dst=o["x1_mask_L"]))
         # mask2weights: 4x (conv3 s2 [+ReLU]) + softmax over 3 (MASIC.py:472-506)
         mk = "mask2weights_unit.maskconv"
         mw = self._buf(B, h16, w16, 3, dtype=f32)        # per-pixel fusion weights, NHWC
         self.mask_weights = mw
-        mp = [self._w(f"{mk}.{i}.{t}") for i in (0, 2, 4, 6) for t in ("weight", "bias")]
-        self._keep += mp
-        self._add("mask2weights(fused)", lambda: check(lib.masic_mask2weights(
-            o["x1_mask_R"].data_ptr(), B, H, W, *[t.data_ptr() for t in mp], None, mw.data_ptr(), self._s()),
-            "masic_mask2weights"))
+        mws = [self._w(f"{mk}.{i}.weight") for i in (0, 2, 4, 6)]
+        mbs = [self._w(f"{mk}.{i}.bias") for i in (0, 2, 4, 6)]
+        self._add("mask2weights(fused)", lambda: ops.mask2weights_into(o["x1_mask_R"], mws, mbs, out_nhwc=mw))
         self._record("mw")
         x2in_bf = self._buf(B, H, W + XPAD, IMG_CP)
-        self._conv_small("R.pre_conv+pre_gdn", x1_warp, self.x2, "encoder2.pre_conv", ksize=5, stride=1, gdn=GDN_FWD,
-                         gdn_prefix="encoder2.pre_gdn", out_bf=x2in_bf)
+        pre_w, pre_b = self._w("encoder2.pre_conv.weight"), self._w("encoder2.pre_conv.bias")
+        pre_beta, pre_gamma = self._w("encoder2.pre_gdn.beta"), self._w("encoder2.pre_gdn.gamma")
+        self._add("R.pre_conv+pre_gdn", lambda: ops.conv_small_into(
+            x1_warp, self.x2, pre_w, pre_b, ksize=5, stride=1, gdn=GDN_FWD, beta=pre_beta, gamma=pre_gamma, out16=x2in_bf,
+            split=True))
         y2 = self._encoder("R.g_a", self._encoder_weights("encoder2"), x2in_bf)
         y2_abs = self._buf(B, h16, w16, M)
         y2_rnd = self._buf(B, h16, w16, M)
@@ -430,7 +384,8 @@ class HSICEngine:
         # [after_gdn(g_s(y2_hat)) (3) 0 | x1_hat_warp (3) 0], each producer with one aligned 8-byte store per pixel
         ac_in = self._buf(B, H, W + XPAD, IMG_CP)
         self._wait("T")
-        self._warp("R.warp(x1_hat)", o["x1_hat"], T, None, x1hw_bf, dst2=ac_in, dst2_coff=4)
+        self._add("R.warp(x1_hat)", lambda: ops.warp_perspective_into(o["x1_hat"], T, (H, W), dst16=x1hw_bf, split=True,
+                                                                      dst2=ac_in, dst2_coff=4))
         y1w = self._encoder("R.g_a(enc1 on warped x1_hat)", enc1, x1hw_bf)                         # :822
         self._wait("mw")
         self._wait("right")

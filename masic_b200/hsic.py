@@ -337,7 +337,7 @@ class PairStream:
                     # criterion (8 floats) | MS-SSIM per channel of view 1 (3) and view 2 (3) | LPIPS of view 1, 2
                     res_d=torch.zeros(16, device=self.dev), res_h=torch.zeros(16).pin_memory(),
                     copied=torch.cuda.Event(), done=torch.cuda.Event(), busy=False, has_result=False,
-                    scratch=torch.empty(self.lib.masic_rd_metrics_scratch_bytes() // 8, dtype=torch.float64, device=self.dev),
+                    scratch=_ops.rd_metrics_scratch(self.dev),
                     lik_p=(C.c_void_p * 4)(*[t.data_ptr() for t in liks]),
                     lik_n=(C.c_int64 * 4)(*[t.numel() for t in liks])))
         self._ms_weights = (C.c_float * 5)(*_ops.MS_SSIM_WEIGHTS)

@@ -148,12 +148,8 @@ def conv_forward(x: Tensor, weight: Tensor, bias: Optional[Tensor], stride: int,
         xin[..., :c].copy_(x.permute(0, 2, 3, 1))
     plan.launch()
     if kind == DECONV_S2_SUBPIX:
-        from . import _lib
         res = torch.empty(n, cout, 2 * h, 2 * w, dtype=torch.float32, device=x.device)
-        _lib.check(_lib.load().masic_subpix_to_nchw(out.data_ptr(), n, h, w, out.shape[3], 0, None, None, 1e-6,
-                                                    res.data_ptr(), None, 0,
-                                                    F16, torch.cuda.current_stream().cuda_stream),
-                   "masic_subpix_to_nchw")
+        ops.subpix_to_nchw_into(out, res)
         return res
     return ops.nhwc_to_nchw_f32(out, cout)
 

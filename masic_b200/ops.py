@@ -26,7 +26,15 @@ def _s() -> int:
 
 
 def _p(t: Optional[torch.Tensor]) -> Optional[int]:
-    return None if t is None else t.data_ptr()
+    if t is None:
+        return None
+    if not t.is_cuda:
+        raise MasicError("masic_b200 kernels need CUDA tensors (no CPU fallback)")
+    return t.data_ptr()
+
+
+def _ptr_array(ts: Sequence[Optional[torch.Tensor]]):
+    return (C.c_void_p * len(ts))(*[_p(t) for t in ts])
 
 
 def _need_cuda(*ts: Optional[torch.Tensor]) -> None:
@@ -105,11 +113,6 @@ def quantize(x: torch.Tensor, means: Optional[torch.Tensor] = None, mode: str = 
     raise ValueError(f'Invalid quantization mode: "{mode}"')
 
 
-def _ptr_array(ts: Sequence[torch.Tensor]):
-    arr = (C.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
-    return arr
-
-
 def eb_forward(z: torch.Tensor, matrices: Sequence[torch.Tensor], biases: Sequence[torch.Tensor],
                factors: Sequence[torch.Tensor], quantiles: torch.Tensor, want_symbols: bool = False,
                want_lik: bool = True):
@@ -161,12 +164,178 @@ def pmf_table_to_cdf(pmf: torch.Tensor, tail_mass: torch.Tensor, pmf_length: tor
 
 
 # --------------------------------------------------------------------------- image domain
+# The `*_into` launchers write caller-owned tensors on the current stream, sizes, row layouts and 16-bit formats taken
+# from the tensors.  They run during CUDA-graph capture, where a temporary would go stale, so they allocate and convert
+# nothing: a CPU, non-contiguous, wrong-dtype or wrongly shaped tensor raises MasicError before anything is launched.
+_F32, _F64, _HALF = (torch.float32,), (torch.float64,), (torch.float16, torch.bfloat16)
+_FMT16 = {torch.float16: _lib.FMT_F16, torch.bfloat16: _lib.FMT_BF16}
+
+
+def _arg(t: Optional[torch.Tensor], dtypes, shape=None) -> Optional[int]:
+    """t's device pointer (None stays None) once t can be handed to the kernel as it is."""
+    if t is None:
+        return None
+    if not t.is_cuda:
+        raise MasicError(f"masic_b200 kernels need CUDA tensors (no CPU fallback); got a {t.device} tensor")
+    if t.dtype not in dtypes:
+        raise MasicError(f"got a {t.dtype} tensor where the kernel reads {' or '.join(map(str, dtypes))}")
+    if not t.is_contiguous():
+        raise MasicError("the kernel needs a contiguous tensor")
+    if shape is not None and tuple(t.shape) != tuple(shape):
+        raise MasicError(f"got a tensor of shape {tuple(t.shape)} where the kernel needs {tuple(shape)}")
+    return t.data_ptr()
+
+
+def _img16(t: Optional[torch.Tensor], n: int, h: int, w: int, split: bool = False):
+    """(pointer, pitch, row_pixels, xoff, format) of a 16-bit NHWC image (n, h, R, pitch): R == w is dense, R == w +
+    IMG_XPAD padded (pixel x at column x + IMG_XOFF).  split=True stores [hi | lo] pixels (the engine's g_a_conv1 input)."""
+    if t is None:
+        return None, 0, 0, 0, 0
+    ptr = _arg(t, _HALF)
+    if t.dim() != 4 or tuple(t.shape[:2]) != (n, h) or t.shape[2] not in (w, w + _lib.IMG_XPAD):
+        raise MasicError(f"a 16-bit image must be ({n}, {h}, {w} or {w} + IMG_XPAD, pitch), got {tuple(t.shape)}")
+    padded = t.shape[2] != w
+    return (ptr, t.shape[3], t.shape[2] if padded else 0, _lib.IMG_XOFF if padded else 0,
+            _FMT16[t.dtype] | (_lib.FMT_SPLIT if split else 0))
+
+
+def _launch(name: str, *args) -> None:
+    check(getattr(_lib.load(), name)(*args, _s()), name)
+
+
+def warp_prepare_into(M: torch.Tensor, T: torch.Tensor, src_hw: Tuple[int, int], dst_hw: Tuple[int, int],
+                      invert: bool = False) -> None:
+    """T (n,3,3) fp64 <- the transform the warp kernel reads for the (n,3,3) fp32 homographies M (or their inverses)."""
+    n = M.shape[0]
+    _launch("masic_warp_prepare", _arg(M, _F32, (n, 3, 3)), n, *src_hw, *dst_hw, int(invert), _arg(T, _F64, (n, 3, 3)))
+
+
+def warp_perspective_into(src: Optional[torch.Tensor], T: torch.Tensor, dsize: Tuple[int, int], *, src_shape=None,
+                          dst=None, dst16=None, split: bool = False, dst2=None, dst2_coff: int = 0, ones=None) -> None:
+    """src (NCHW fp32; None: all ones of src_shape) warped by T to dsize into dst (NCHW fp32), dst16, dst2 (16-bit NHWC;
+    dst2's channels at dst2_coff, the rest of the pixel untouched) and ones (the all-ones image warped, (n,1,h,w))."""
+    n, c, h, w = src.shape if src is not None else src_shape
+    ho, wo = dsize
+    p16, pitch, row, xoff, fmt = _img16(dst16, n, ho, wo, split)
+    p2, pitch2, row2, xoff2, fmt2 = _img16(dst2, n, ho, wo)
+    if dst2 is not None and not row2:
+        row2 = wo                  # the second destination's rows are always given: row_pixels = 0 is not "dense" there
+    _launch("masic_warp_perspective_fwd", _arg(src, _F32), n, c, h, w, ho, wo, _arg(T, _F64, (n, 3, 3)),
+            _arg(dst, _F32, (n, c, ho, wo)), p16, pitch, row, xoff, fmt, p2, pitch2, row2, xoff2, dst2_coff, fmt2,
+            _arg(ones, _F32, (n, 1, ho, wo)))
+
+
+def conv_small_into(in0: torch.Tensor, in1: Optional[torch.Tensor], weight: torch.Tensor, bias: Optional[torch.Tensor],
+                    *, ksize: int, stride: int, transposed_s1: bool = False, act: int = ACT_NONE, gdn: int = GDN_NONE,
+                    beta=None, gamma=None, beta_min: float = 1e-6, out=None, out16=None, split: bool = False) -> None:
+    """Tiny-channel conv of cat(in0, in1) (NCHW fp32) into out (NCHW fp32) and / or out16 (16-bit NHWC)."""
+    n, c0, h, w = in0.shape
+    c1 = 0 if in1 is None else in1.shape[1]
+    c_out = weight.shape[1] if transposed_s1 else weight.shape[0]
+    ho, wo = -(-h // stride), -(-w // stride)
+    _launch("masic_conv_small_nchw", _arg(in0, _F32), c0, _arg(in1, _F32, (n, c1, h, w)), c1, n, h, w,
+            _arg(weight, _F32), int(transposed_s1), _arg(bias, _F32, (c_out,)), c_out, ksize, stride, act, gdn,
+            _arg(beta, _F32), _arg(gamma, _F32), float(beta_min), _arg(out, _F32, (n, c_out, ho, wo)),
+            *_img16(out16, n, ho, wo, split))
+
+
+def nchw_to_nhwc_into(x: torch.Tensor, out: torch.Tensor, *, split: bool = False) -> None:
+    """NCHW fp32 (c <= 8) -> the 16-bit NHWC image out, channels beyond c zeroed."""
+    n, c, h, w = x.shape
+    _launch("masic_nchw_to_nhwc_bf16", _arg(x, _F32), n, c, h, w, *_img16(out, n, h, w, split))
+
+
+def nhwc_to_nchw_into(x: torch.Tensor, out: torch.Tensor) -> None:
+    """The first out.shape[1] channels of the NHWC fp32 x -> NCHW fp32 out."""
+    n, h, w, pitch = x.shape
+    c = out.shape[1]
+    _launch("masic_nhwc_to_nchw_f32", _arg(x, _F32), n, c, h * w, pitch, _arg(out, _F32, (n, c, h, w)))
+
+
+def subpix_to_nchw_into(x: torch.Tensor, out: torch.Tensor) -> None:
+    """A MASIC_DECONV_S2_SUBPIX plan's output (n, h, w, pitch) fp32 -> the NCHW fp32 image out (n, 3, 2h, 2w)."""
+    n, h, w, pitch = x.shape
+    _launch("masic_subpix_to_nchw", _arg(x, _F32), n, h, w, pitch, GDN_NONE, None, None, 1e-6,
+            _arg(out, _F32, (n, 3, 2 * h, 2 * w)), None, 0, 0)
+
+
+def softmax_channels_into(x: torch.Tensor, out=None, out_nhwc=None) -> None:
+    """Softmax over the channels of the NCHW fp32 x into out (NCHW) and / or out_nhwc."""
+    n, c, h, w = x.shape
+    _launch("masic_softmax_channels", _arg(x, _F32), n, c, h * w, _arg(out, _F32, (n, c, h, w)),
+            _arg(out_nhwc, _F32, (n, h, w, c)))
+
+
+def mask2weights_into(mask: torch.Tensor, weights: Sequence[torch.Tensor], biases: Sequence[Optional[torch.Tensor]],
+                      out=None, out_nhwc=None) -> None:
+    """mask2weights.forward (MASIC.py:472-506) of the (n,1,h,w) mask into out (n,3,h/16,w/16) and / or out_nhwc."""
+    n, _, h, w = mask.shape
+    ho, wo = -(-h // 16), -(-w // 16)          # four stride-2 layers, each rounding up
+    params = [_arg(t, _F32) for wb in zip(weights, biases) for t in wb]
+    _launch("masic_mask2weights", _arg(mask, _F32, (n, 1, h, w)), n, h, w, *params, _arg(out, _F32, (n, 3, ho, wo)),
+            _arg(out_nhwc, _F32, (n, ho, wo, 3)))
+
+
+def gdn_nchw_into(x: torch.Tensor, beta: torch.Tensor, gamma: torch.Tensor, out: torch.Tensor, *,
+                  inverse: bool = False, beta_min: float = 1e-6) -> None:
+    """GDN / IGDN over the channels of the NCHW fp32 x with the stored (re-parametrised) beta (c,) and gamma (c, c)."""
+    n, c, h, w = x.shape
+    _launch("masic_gdn_nchw", _arg(x, _F32), n, c, h * w, _arg(beta, _F32, (c,)), _arg(gamma, _F32, (c, c)),
+            float(beta_min), int(inverse), _arg(out, _F32, (n, c, h, w)))
+
+
+def cqe_mask_weights_into(mask: torch.Tensor, weights: Sequence[torch.Tensor], biases: Sequence[torch.Tensor], out) -> None:
+    """mask2weights_EN.forward (MASIC.py:1411-1434) of the (n,1,h,w) mask into out (n,kw,h,w)."""
+    n, _, h, w = mask.shape
+    kw = out.shape[1]
+    ws = (C.c_void_p * 4)(*[_arg(t, _F32) for t in weights])
+    bs = (C.c_void_p * 4)(*[_arg(t, _F32) for t in biases])
+    _launch("masic_cqe_mask_weights", _arg(mask, _F32, (n, 1, h, w)), n, h, w, ws, bs, kw, _arg(out, _F32, (n, kw, h, w)))
+
+
+def cqe_blend_images_into(a: torch.Tensor, b: torch.Tensor, weights: torch.Tensor, out: torch.Tensor) -> None:
+    """MASIC.py:1470-1471: out (n,h,w,16) 16-bit = [a * weights[:,0] | b * weights[:,1] | 0] of the NCHW fp32 images."""
+    n, _, h, w = b.shape
+    _launch("masic_cqe_blend_images", _arg(a, _F32, (n, 3, h, w)), _arg(b, _F32, (n, 3, h, w)),
+            _arg(weights, _F32, (n, 2, h, w)), n, h, w, _arg(out, _HALF, (n, h, w, 16)), _FMT16[out.dtype])
+
+
+def cqe_feature_fuse_into(self_: torch.Tensor, other: torch.Tensor, weights: torch.Tensor, T: torch.Tensor,
+                          out: torch.Tensor) -> None:
+    """MASIC.py:1479-1482 on 16-bit NHWC maps, c = self_.shape[3]: out[..., :2c] = [self_ * w1 | warp(other, T) * w0]."""
+    n, h, w, c = self_.shape
+    p_out = _arg(out, _HALF)
+    _launch("masic_cqe_feature_fuse", _arg(self_, (out.dtype,)), c, _arg(other, (out.dtype,)), other.shape[3], c,
+            _arg(weights, _F32, (n, 2, h, w)), _arg(T, _F64, (n, 3, 3)), n, h, w, p_out, out.shape[3], _FMT16[out.dtype])
+
+
+def cqe_residual_image_into(conv_out: torch.Tensor, identity: torch.Tensor, out: torch.Tensor) -> None:
+    """MASIC.py:1495-1496: out (NCHW fp32) = the first 3 channels of the NHWC fp32 conv_out + identity (NCHW fp32)."""
+    n, h, w, pitch = conv_out.shape
+    _launch("masic_cqe_residual_image", _arg(conv_out, _F32), pitch, _arg(identity, _F32, (n, 3, h, w)), n, h, w,
+            _arg(out, _F32, (n, 3, h, w)))
+
+
+def rd_metrics_scratch(device) -> torch.Tensor:
+    """The device scratch rd_metrics_into needs (allocate it once, outside graph capture)."""
+    return torch.empty(_lib.load().masic_rd_metrics_scratch_bytes() // 8, dtype=torch.float64, device=device)
+
+
+def rd_metrics_into(liks: Sequence[Optional[torch.Tensor]], x1_hat: torch.Tensor, x1: torch.Tensor,
+                    x2_hat: torch.Tensor, x2: torch.Tensor, lmbda: float, scratch: torch.Tensor,
+                    out: torch.Tensor) -> None:
+    """RateDistortionLoss.forward into out (8 fp32, see masic_rd_metrics); a None likelihood tensor is skipped."""
+    n, c, h, w = x1_hat.shape
+    lp = (C.c_void_p * 4)(*[_arg(t, _F32) for t in liks])
+    ln = (C.c_int64 * 4)(*[0 if t is None else t.numel() for t in liks])
+    imgs = [_arg(t, _F32, (n, c, h, w)) for t in (x1_hat, x1, x2_hat, x2)]
+    _launch("masic_rd_metrics", lp, ln, *imgs, n, c, h, w, float(lmbda), _arg(scratch, _F64), _arg(out, _F32, (8,)))
+
+
 def warp_prepare(M: torch.Tensor, src_hw: Tuple[int, int], dst_hw: Tuple[int, int], invert: bool = False):
-    _need_cuda(M)
     M = _f32c(M)
     T = torch.empty(M.shape, dtype=torch.float64, device=M.device)
-    check(_lib.load().masic_warp_prepare(M.data_ptr(), M.shape[0], src_hw[0], src_hw[1], dst_hw[0], dst_hw[1],
-                                         int(invert), T.data_ptr(), _s()), "masic_warp_prepare")
+    warp_prepare_into(M, T, src_hw, dst_hw, invert)
     return T
 
 
@@ -175,18 +344,14 @@ def warp_perspective(src: Optional[torch.Tensor], M: torch.Tensor, dsize: Tuple[
                      bf16_pitch: int = 0):
     """kornia.warp_perspective(src, M, dsize) (0.5.0: bilinear, zeros, align_corners=True).
     src=None with ones_shape=(N,C,H,W) warps an all-ones image (mask())."""
-    _need_cuda(src, M)
     if src is not None:
         src = _f32c(src)
-        n, c, h, w = src.shape
-    else:
-        n, c, h, w = ones_shape
+    n, c, h, w = src.shape if src is not None else ones_shape
     ho, wo = dsize
     T = warp_prepare(M, (h, w), (ho, wo), invert)
     dst = torch.empty(n, c, ho, wo, dtype=torch.float32, device=M.device)
     dst_bf = torch.empty(n, ho, wo, bf16_pitch, dtype=ACT16, device=M.device) if bf16_pitch else None
-    check(_lib.load().masic_warp_perspective_fwd(_p(src), n, c, h, w, ho, wo, T.data_ptr(), dst.data_ptr(),
-                                                 _p(dst_bf), bf16_pitch, 0, 0, F16, _s()), "masic_warp_perspective_fwd")
+    warp_perspective_into(src, T, dsize, src_shape=(n, c, h, w), dst=dst, dst16=dst_bf)
     return (dst, dst_bf) if bf16_pitch else dst
 
 
@@ -194,11 +359,9 @@ def conv_small(in0: torch.Tensor, in1: Optional[torch.Tensor], weight: torch.Ten
                *, ksize: int, stride: int, transposed_s1: bool = False, act: int = ACT_NONE, gdn: int = GDN_NONE,
                beta: Optional[torch.Tensor] = None, gamma: Optional[torch.Tensor] = None, beta_min: float = 1e-6,
                out: Optional[torch.Tensor] = None, out_bf16: Optional[torch.Tensor] = None):
-    _need_cuda(in0, in1, weight)
     in0 = _f32c(in0)
     in1 = None if in1 is None else _f32c(in1)
-    n, c0, h, w = in0.shape
-    c1 = 0 if in1 is None else in1.shape[1]
+    n, _, h, w = in0.shape
     weight = _f32c(weight.detach())
     c_out = weight.shape[1] if transposed_s1 else weight.shape[0]
     bias = None if bias is None else _f32c(bias.detach())
@@ -207,18 +370,14 @@ def conv_small(in0: torch.Tensor, in1: Optional[torch.Tensor], weight: torch.Ten
     ho, wo = -(-h // stride), -(-w // stride)
     if out is None and out_bf16 is None:
         out = torch.empty(n, c_out, ho, wo, dtype=torch.float32, device=in0.device)
-    check(_lib.load().masic_conv_small_nchw(in0.data_ptr(), c0, _p(in1), c1, n, h, w, weight.data_ptr(),
-                                            int(transposed_s1), _p(bias), c_out, ksize, stride, act, gdn, _p(beta),
-                                            _p(gamma), float(beta_min), _p(out), _p(out_bf16),
-                                            0 if out_bf16 is None else out_bf16.shape[3], 0, 0, F16, _s()),
-          "masic_conv_small_nchw")
+    conv_small_into(in0, in1, weight, bias, ksize=ksize, stride=stride, transposed_s1=transposed_s1, act=act, gdn=gdn,
+                    beta=beta, gamma=gamma, beta_min=beta_min, out=out, out16=out_bf16)
     return out if out is not None else out_bf16
 
 
 def mask2weights(mask: torch.Tensor, weights, biases, nhwc_out: bool = False):
     """mask2weights.forward (MASIC.py:472-506) in one launch.  weights / biases: the four conv3x3 stride-2 layers'
     parameters (maskconv.0, .2, .4, .6).  Returns the (n,3,h/16,w/16) softmax weights (and the NHWC copy)."""
-    _need_cuda(mask, *weights)
     mask = _f32c(mask)
     n, c, h, w = mask.shape
     if c != 1 or len(weights) != 4 or len(biases) != 4:
@@ -229,48 +388,37 @@ def mask2weights(mask: torch.Tensor, weights, biases, nhwc_out: bool = False):
         if tuple(t.shape) != shp:
             raise MasicError(f"mask2weights: weight shape {tuple(t.shape)} != {shp}")
     bs = [None if t is None else _f32c(t.detach()) for t in biases]
-    ho, wo = h, w
-    for _ in range(4):
-        ho, wo = (ho + 1) // 2, (wo + 1) // 2
+    ho, wo = -(-h // 16), -(-w // 16)
     out = torch.empty(n, 3, ho, wo, dtype=torch.float32, device=mask.device)
     out_nhwc = torch.empty(n, ho, wo, 3, dtype=torch.float32, device=mask.device) if nhwc_out else None
-    check(_lib.load().masic_mask2weights(mask.data_ptr(), n, h, w, ws[0].data_ptr(), _p(bs[0]), ws[1].data_ptr(), _p(bs[1]),
-                                         ws[2].data_ptr(), _p(bs[2]), ws[3].data_ptr(), _p(bs[3]), out.data_ptr(),
-                                         _p(out_nhwc), _s()), "masic_mask2weights")
+    mask2weights_into(mask, ws, bs, out, out_nhwc)
     return (out, out_nhwc) if nhwc_out else out
 
 
 def softmax_channels(x: torch.Tensor, nhwc_out: bool = False):
-    _need_cuda(x)
     x = _f32c(x)
     n, c, h, w = x.shape
     o1 = torch.empty_like(x)
     o2 = torch.empty(n, h, w, c, dtype=torch.float32, device=x.device) if nhwc_out else None
-    check(_lib.load().masic_softmax_channels(x.data_ptr(), n, c, h * w, o1.data_ptr(), _p(o2), _s()),
-          "masic_softmax_channels")
+    softmax_channels_into(x, o1, o2)
     return (o1, o2) if nhwc_out else o1
 
 
 def nchw_to_nhwc_bf16(x: torch.Tensor, pitch: int, out: Optional[torch.Tensor] = None):
-    _need_cuda(x)
     x = _f32c(x)
     n, c, h, w = x.shape
     if out is None:
         out = torch.empty(n, h, w, pitch, dtype=ACT16, device=x.device)
-    check(_lib.load().masic_nchw_to_nhwc_bf16(x.data_ptr(), n, c, h, w, out.data_ptr(), pitch, 0, 0, F16, _s()),
-          "masic_nchw_to_nhwc_bf16")
+    nchw_to_nhwc_into(x, out)
     return out
 
 
 def nhwc_to_nchw_f32(x: torch.Tensor, c: Optional[int] = None, out: Optional[torch.Tensor] = None):
-    _need_cuda(x)
-    assert x.dtype == torch.float32 and x.is_contiguous()
     n, h, w, pitch = x.shape
     c = c or pitch
     if out is None:
         out = torch.empty(n, c, h, w, dtype=torch.float32, device=x.device)
-    check(_lib.load().masic_nhwc_to_nchw_f32(x.data_ptr(), n, c, h * w, pitch, out.data_ptr(), _s()),
-          "masic_nhwc_to_nchw_f32")
+    nhwc_to_nchw_into(x, out)
     return out
 
 

@@ -61,14 +61,11 @@ def _(x, weight, bias, stride, transposed, tap_mask):
 @torch.library.custom_op(f"{NS}::gdn", mutates_args=(), device_types="cuda")
 def gdn(x: Tensor, beta: Tensor, gamma: Tensor, inverse: bool, beta_min: float) -> Tensor:
     """compressai/layers/gdn.py:77-92 with the stored (re-parametrised) beta / gamma."""
-    from . import _lib
     _cuda_only(x, beta, gamma)
-    n, c, h, w = x.shape
     x = x.float().contiguous()
     out = torch.empty_like(x)
-    _lib.check(_lib.load().masic_gdn_nchw(x.data_ptr(), n, c, h * w, beta.detach().float().contiguous().data_ptr(),
-                                          gamma.detach().float().contiguous().data_ptr(), float(beta_min), int(inverse),
-                                          out.data_ptr(), torch.cuda.current_stream().cuda_stream), "masic_gdn_nchw")
+    ops.gdn_nchw_into(x, beta.detach().float().contiguous(), gamma.detach().float().contiguous(), out, inverse=inverse,
+                      beta_min=beta_min)
     return out
 
 

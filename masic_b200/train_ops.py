@@ -4,28 +4,12 @@ from __future__ import annotations
 
 import ctypes as C
 import math
-from typing import Optional, Sequence
 
 import torch
 
 from . import _lib
-from ._lib import MasicError, check
-
-
-def _p(t: Optional[torch.Tensor]):
-    if t is None:
-        return None
-    if not t.is_cuda:
-        raise MasicError("masic_b200 training kernels need CUDA tensors (no CPU fallback)")
-    return t.data_ptr()
-
-
-def _s() -> int:
-    return torch.cuda.current_stream().cuda_stream
-
-
-def _ptr_array(ts: Sequence[torch.Tensor]):
-    return (C.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
+from ._lib import check
+from .ops import _p, _ptr_array, _s
 
 
 def lik_grad_scale(num_pixels: int) -> float:

@@ -29,19 +29,18 @@ No CPU fallback: everything raises on non-CUDA tensors.
 """
 from __future__ import annotations
 
-import ctypes as C
 from typing import Callable, Dict, List, Optional, Tuple
 
 import torch
 
-from . import _lib
+from . import _lib, ops
 from . import train_ops as T
 from ._lib import MasicError, check
 from .convplan import (ACT_LEAKY, ACT_NONE, ACT_RELU, CONV, CONV_XFOLD8, DECONV_S2, DECONV_S2_SUBPIX, GDN_NONE,
                        MASK_A_5x5, ConvPlan, PackBatch, PackedConv, WgradPlan, gdn_prepare)
 
 NOISE_KEYS = ("z1", "y1_ctx", "y1", "z2", "y2_ctx", "y1w", "y2")
-XOFF, XPAD = _lib.IMG_XOFF, _lib.IMG_XPAD
+XPAD = _lib.IMG_XPAD
 IMG_CP = 8           # MASIC_CONV_XFOLD8 input pitch
 BF = torch.bfloat16
 F32 = torch.float32
@@ -231,9 +230,7 @@ class _GDN3:
         tr.zero_each_step += [self.dbp, self.dgp]
 
     def fwd(self, x, y):
-        n, c, h, w = x.shape
-        check(self.tr.lib.masic_gdn_nchw(x.data_ptr(), n, c, h * w, self.beta.data_ptr(), self.gamma.data_ptr(), 1e-6,
-                                         int(self.inverse), y.data_ptr(), T._s()), "masic_gdn_nchw")
+        ops.gdn_nchw_into(x, self.beta, self.gamma, y, inverse=self.inverse)
 
     def bwd(self, x, g, dx):
         T.gdn_small_bwd(x, g, self.beta, self.gamma, self.inverse, dx, self.dbp, self.dgp)
@@ -483,7 +480,6 @@ class HSICTrainer(TrainStep):
         self.repack.append((d4, w4, None))
         dplan4 = ConvPlan(packed=d4, stride=2, x=gimg_bf, out=gprev)
         e3 = prev
-        lib = self.lib
         gimg16 = self._z(B, H, W, 16)                     # dense 16-pitch copy of dL/d(image) for the weight gradient
         dw16 = self._z(N, 16, 5, 5, dtype=F32)
         wg4 = WgradPlan(ksize=5, stride=2, lo=e3, c_lo=N, hi=gimg16, c_hi=16, dw=dw16)
@@ -496,11 +492,9 @@ class HSICTrainer(TrainStep):
 
         def bwd(gimg: torch.Tensor):
             """gimg: dL/d(deconv4 output image), NCHW fp32 (B,3,H,W)."""
-            check(lib.masic_nchw_to_nhwc_bf16(gimg.data_ptr(), B, 3, H, W, gimg_bf.data_ptr(), IMG_CP, W + XPAD, XOFF,
-                                              0, T._s()), "masic_nchw_to_nhwc_bf16")
+            ops.nchw_to_nhwc_into(gimg, gimg_bf)
             T.colsum_nchw(gimg, db4)
-            check(lib.masic_nchw_to_nhwc_bf16(gimg.data_ptr(), B, 3, H, W, gimg16.data_ptr(), 16, 0, 0, 0, T._s()),
-                  "masic_nchw_to_nhwc_bf16")
+            ops.nchw_to_nhwc_into(gimg, gimg16)
             self.wg_async(lambda: (wg4.launch(), dw4.add_(dw16[:, :3])))
             dplan4.launch()
             for i in (2, 1, 0):
@@ -626,7 +620,6 @@ class HSICTrainer(TrainStep):
     def _build(self):
         B, H, W, N, M, K = self.B, self.H, self.W, self.N, self.M, self.K
         h16, w16 = H // 16, W // 16
-        lib = self.lib
         dev = self.dev
         self.noise = {k: self._z(B, (h16 // 4) if k.startswith("z") else h16, (w16 // 4) if k.startswith("z") else w16,
                                  N if k.startswith("z") else M, dtype=F32) for k in NOISE_KEYS}     # NHWC
@@ -656,8 +649,7 @@ class HSICTrainer(TrainStep):
         net1 = self._gmm_net("L", "_h_s1_same_resolution", 4 * M, True, gmm1_in, g_gmm1_in)
         dec1 = self._decoder_pass("L", "decoder1", y1_hat_bf, g_y1hat)
 
-        self.F("x1.pack", lambda: check(lib.masic_nchw_to_nhwc_bf16(self.x1.data_ptr(), B, 3, H, W, x1_bf.data_ptr(), IMG_CP,
-                                                                    W + XPAD, XOFF, 0, T._s()), "pack"))
+        self.F("x1.pack", lambda: ops.nchw_to_nhwc_into(self.x1, x1_bf))
         self.F("L.encoder", encA["fwd"])
         self.F("L.latent_prep", lambda: T.latent_prep_train(y1, self.noise["y1_ctx"], y1_abs, y1_ctx))
         self.F("L.hyper", hyp1["fwd"])
@@ -667,23 +659,13 @@ class HSICTrainer(TrainStep):
             y1, self.noise["y1"], net1["sig"], net1["mu"], net1["wl"], M, K, scale, lik=o["lik_y1"], y_hat_bf=y1_hat_bf,
             y_hat=o["y1_hat"], dy=dy1_lik, dsigma=net1["gsig"], dmu=net1["gmu"], dwl=net1["gwl"]))
         self.F("L.decoder", dec1["fwd"])
-        self.F("L.x1_hat", lambda: check(lib.masic_subpix_to_nchw(dec1["sp"].data_ptr(), B, H // 2, W // 2, 16, 0, None, None,
-                                                                  1e-6, o["x1_hat"].data_ptr(), None, 0, 0, T._s()), "subpix"))
+        self.F("L.x1_hat", lambda: ops.subpix_to_nchw_into(dec1["sp"], o["x1_hat"]))
 
         # ================= right view =================
         Tm = torch.empty(B, 3, 3, device=dev, dtype=torch.float64)
-        self.F("warp.prepare", lambda: check(lib.masic_warp_prepare(self.Hm.data_ptr(), B, H, W, H, W, 0, Tm.data_ptr(), T._s()),
-                                             "masic_warp_prepare"))
+        self.F("warp.prepare", lambda: ops.warp_prepare_into(self.Hm, Tm, (H, W), (H, W)))
         mask_R = self._z(B, 1, H, W, dtype=F32)
-
-        def warp(src, dst, dst_bf=None, ch=3):
-            check(lib.masic_warp_perspective_fwd(None if src is None else src.data_ptr(), B, ch, H, W, H, W, Tm.data_ptr(),
-                                                 None if dst is None else dst.data_ptr(),
-                                                 None if dst_bf is None else dst_bf.data_ptr(),
-                                                 0 if dst_bf is None else dst_bf.shape[3],
-                                                 0 if dst_bf is None else dst_bf.shape[2], 0 if dst_bf is None else XOFF,
-                                                 0, T._s()), "masic_warp_perspective_fwd")
-        self.F("mask_R", lambda: warp(None, mask_R, ch=1))
+        self.F("mask_R", lambda: ops.warp_perspective_into(None, Tm, (H, W), src_shape=mask_R.shape, dst=mask_R))
         # mask2weights (MASIC.py:472-506)
         mk = "mask2weights_unit.maskconv"
         kshape = [(1, H, W), (3, H // 2, W // 2), (6, H // 4, W // 4), (6, H // 8, W // 8), (3, h16, w16)]
@@ -696,17 +678,11 @@ class HSICTrainer(TrainStep):
         mk_dw = [self.grad(f"{mk}.{2 * i}.weight") for i in range(4)]
         mk_db = [self.grad(f"{mk}.{2 * i}.bias") for i in range(4)]
 
-        def small(in0, in1, w, b, c_out, k, s, act, out, tr=False):
-            n, c0, h, wd = in0.shape
-            check(lib.masic_conv_small_nchw(in0.data_ptr(), c0, None if in1 is None else in1.data_ptr(),
-                                            0 if in1 is None else in1.shape[1], n, h, wd, w.data_ptr(), int(tr), b.data_ptr(),
-                                            c_out, k, s, act, 0, None, None, 1e-6, out.data_ptr(), None, 0, 0, 0, 0, T._s()),
-                  "masic_conv_small_nchw")
-
         def mask_fwd():
             for i in range(4):
-                small(kb[i], None, mk_w[i], mk_b[i], kshape[i + 1][0], 3, 2, ACT_RELU if i < 3 else ACT_NONE, kb[i + 1])
-            check(lib.masic_softmax_channels(kb[4].data_ptr(), B, 3, h16 * w16, None, mw.data_ptr(), T._s()), "softmax")
+                ops.conv_small_into(kb[i], None, mk_w[i], mk_b[i], ksize=3, stride=2, act=ACT_RELU if i < 3 else ACT_NONE,
+                                    out=kb[i + 1])
+            ops.softmax_channels_into(kb[4], out_nhwc=mw)
         self.F("mask2weights", mask_fwd)
 
         x1_warp = self._z(B, 3, H, W, dtype=F32)
@@ -716,11 +692,10 @@ class HSICTrainer(TrainStep):
         x2in_bf = self._z(B, H, W + XPAD, IMG_CP)
         pre_w, pre_b = self.param("encoder2.pre_conv.weight"), self.param("encoder2.pre_conv.bias")
         pre_gdn = _GDN3(self, "encoder2.pre_gdn", False)
-        self.F("R.warp(x1)", lambda: warp(self.x1, x1_warp))
-        self.F("R.pre_conv", lambda: small(x1_warp, self.x2, pre_w, pre_b, 3, 5, 1, ACT_NONE, pc))
+        self.F("R.warp(x1)", lambda: ops.warp_perspective_into(self.x1, Tm, (H, W), dst=x1_warp))
+        self.F("R.pre_conv", lambda: ops.conv_small_into(x1_warp, self.x2, pre_w, pre_b, ksize=5, stride=1, out=pc))
         self.F("R.pre_gdn", lambda: pre_gdn.fwd(pc, pg))
-        self.F("R.pack", lambda: check(lib.masic_nchw_to_nhwc_bf16(pg.data_ptr(), B, 3, H, W, x2in_bf.data_ptr(), IMG_CP,
-                                                                   W + XPAD, XOFF, 0, T._s()), "pack"))
+        self.F("R.pack", lambda: ops.nchw_to_nhwc_into(pg, x2in_bf))
         encB = self._encoder_pass("B", "encoder2", x2in_bf, pg, accumulate=False, share=None, need_dimg=True)
         y2, gy2 = encB["y"], encB["gy"]
         y2_abs, g_y2abs = self._z(B, h16, w16, M), self._z(B, h16, w16, M)
@@ -740,7 +715,7 @@ class HSICTrainer(TrainStep):
         # x1_hat warped once (MASIC.py:821 == :833), encoder1 again on it (:822)
         x1hw = self._z(B, 3, H, W, dtype=F32)
         x1hw_bf = self._z(B, H, W + XPAD, IMG_CP)
-        self.F("R.warp(x1_hat)", lambda: warp(o["x1_hat"], x1hw, x1hw_bf))
+        self.F("R.warp(x1_hat)", lambda: ops.warp_perspective_into(o["x1_hat"], Tm, (H, W), dst=x1hw, dst16=x1hw_bf))
         encC = self._encoder_pass("C", "encoder1", x1hw_bf, x1hw, accumulate=True, share=encA, need_dimg=True)
         y1w, gy1w = encC["y"], encC["gy"]
         self.F("R.encoder1(x1_hat_warp)", encC["fwd"])
@@ -757,22 +732,18 @@ class HSICTrainer(TrainStep):
         after_gdn = _GDN3(self, "decoder2.after_gdn", True)
         aw, ab = self.param("decoder2.after_conv.weight"), self.param("decoder2.after_conv.bias")
         self.F("R.decoder", dec2["fwd"])
-        self.F("R.core", lambda: check(lib.masic_subpix_to_nchw(dec2["sp"].data_ptr(), B, H // 2, W // 2, 16, 0, None, None, 1e-6,
-                                                                core.data_ptr(), None, 0, 0, T._s()), "subpix"))
+        self.F("R.core", lambda: ops.subpix_to_nchw_into(dec2["sp"], core))
         self.F("R.after_gdn", lambda: after_gdn.fwd(core, ag))
-        self.F("R.after_conv", lambda: small(ag, x1hw, aw, ab, 3, 5, 1, ACT_NONE, o["x2_hat"], tr=True))
+        self.F("R.after_conv", lambda: ops.conv_small_into(ag, x1hw, aw, ab, ksize=5, stride=1, transposed_s1=True,
+                                                           out=o["x2_hat"]))
         o["z1_hat"], o["lik_z1"], o["z2_hat"], o["lik_z2"] = hyp1["z_hat"], hyp1["z_lik"], hyp2["z_hat"], hyp2["z_lik"]
 
         # ================= loss =================
         self.rd_out = self._z(8, dtype=F32)
-        self.rd_scratch = torch.empty(lib.masic_rd_metrics_scratch_bytes() // 8, dtype=torch.float64, device=dev)
+        self.rd_scratch = ops.rd_metrics_scratch(dev)
         liks = [o["lik_y1"], o["lik_y2"], o["lik_z1"], o["lik_z2"]]
-        lp = (C.c_void_p * 4)(*[t.data_ptr() for t in liks])
-        ln = (C.c_int64 * 4)(*[t.numel() for t in liks])
-        self.F("loss", lambda: check(lib.masic_rd_metrics(lp, ln, o["x1_hat"].data_ptr(), self.x1.data_ptr(),
-                                                          o["x2_hat"].data_ptr(), self.x2.data_ptr(), B, 3, H, W, self.lmbda,
-                                                          self.rd_scratch.data_ptr(), self.rd_out.data_ptr(), T._s()),
-                                     "masic_rd_metrics"))
+        self.F("loss", lambda: ops.rd_metrics_into(liks, o["x1_hat"], self.x1, o["x2_hat"], self.x2, self.lmbda,
+                                                   self.rd_scratch, self.rd_out))
         # aux loss (entropy_models.py:345-348) of both bottlenecks
         self.aux_out = self._z(1, dtype=F32)
         self.zero_each_step += [self.aux_out]
@@ -816,8 +787,7 @@ class HSICTrainer(TrainStep):
         self.Bk("mask2weights", mask_bwd)
         self.Bk("R.encoder1(x1_hat_warp)", encC["bwd"])
         d_x1hw_b = self._z(B, 3, H, W, dtype=F32)
-        self.Bk("C.dimg", lambda: check(lib.masic_subpix_to_nchw(encC["dimg"].data_ptr(), B, H // 2, W // 2, 16, 0, None, None,
-                                                                 1e-6, d_x1hw_b.data_ptr(), None, 0, 0, T._s()), "subpix"))
+        self.Bk("C.dimg", lambda: ops.subpix_to_nchw_into(encC["dimg"], d_x1hw_b))
         d_x1hat_w = self._z(B, 3, H, W, dtype=F32)
         self.zero_each_step += [d_x1hat_w]
         self.Bk("warp_bwd", lambda: T.warp_bwd(d_x1hw_a, d_x1hw_b, Tm, d_x1hat_w))
@@ -828,8 +798,7 @@ class HSICTrainer(TrainStep):
         d_pgt = self._z(B, 3, H, W, dtype=F32)
         d_pc = self._z(B, 3, H, W, dtype=F32)
         pdw, pdb = self.grad("encoder2.pre_conv.weight"), self.grad("encoder2.pre_conv.bias")
-        self.Bk("B.dimg", lambda: check(lib.masic_subpix_to_nchw(encB["dimg"].data_ptr(), B, H // 2, W // 2, 16, 0, None, None,
-                                                                 1e-6, d_pgt.data_ptr(), None, 0, 0, T._s()), "subpix"))
+        self.Bk("B.dimg", lambda: ops.subpix_to_nchw_into(encB["dimg"], d_pgt))
         self.Bk("pre_gdn", lambda: pre_gdn.bwd(pc, d_pgt, d_pc))
         self.Bk("pre_conv", lambda: T.conv_small_bwd(x1_warp, self.x2, pre_w, False, 3, 5, 1, d_pc, dweight=pdw, dbias=pdb))
         # left view
@@ -980,9 +949,7 @@ class _Conv1:
         self.fwd_plan.launch()
 
     def bwd(self, skip_act: bool = True):
-        Bn, _, Hh, Ww = self.img_nchw.shape
-        check(self.tr.lib.masic_nchw_to_nhwc_bf16(self.img_nchw.data_ptr(), Bn, 3, Hh, Ww, self.img16.data_ptr(), 16, 0, 0,
-                                                  0, T._s()), "masic_nchw_to_nhwc_bf16")
+        ops.nchw_to_nhwc_into(self.img_nchw, self.img16)
         self.tr.wg_async(lambda: (self.wg_plan.launch(), self.dw.add_(self.dw16[:, :3])))
         if self.dg_plan is not None:
             self.dg_plan.launch()

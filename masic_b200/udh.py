@@ -18,7 +18,7 @@ from typing import Dict, Optional, Tuple
 import torch
 import torch.nn as nn
 
-from . import _lib
+from . import _lib, ops
 from ._lib import MasicError, check
 from .convplan import ACT_RELU, ConvPlan, PackedConv
 
@@ -151,8 +151,7 @@ class UDHEngine:
         lib, B, P = self.lib, self.B, self.P
         # cat((a, b), dim=1) (model.py:96): the two patches are the two channels of the static NCHW input pair, packed
         # into the 16-channel-pitch NHWC bf16 buffer the first conv reads (channels 2..15 stay zero)
-        check(lib.masic_nchw_to_nhwc_bf16(self.ab.data_ptr(), B, 2, P, P, self.x_in.data_ptr(), 16, P, 0, F16, self._s()),
-              "masic_nchw_to_nhwc_bf16")
+        ops.nchw_to_nhwc_into(self.ab, self.x_in)
         for _, fn in self.steps:
             fn()
         k1 = self.w1.shape[1]

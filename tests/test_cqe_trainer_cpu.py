@@ -7,14 +7,14 @@ NEW_SYMBOLS = ("masic_conv_plan_set_act_out", "masic_act_bwd_bias_out", "masic_c
                "masic_cqe_blend_images_bwd")
 
 
-def test_new_entry_points_exported_and_bound():
+def test_training_entry_points_exported_and_bound():
     from masic_b200 import _lib
     lib = _lib.load()
     declared = _lib.declared_symbols()
     for name in NEW_SYMBOLS:
         assert name in declared
         assert getattr(lib, name).argtypes
-    assert lib.masic_abi_version() == 10
+    assert lib.masic_abi_version() == 11
 
 
 def test_new_entry_points_reject_bad_arguments():

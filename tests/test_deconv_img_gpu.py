@@ -38,16 +38,15 @@ def test_deconv_img_matches_torch(n, h, w, dt, igdn):
 
 
 @pytest.mark.parametrize("n,h,w", [(1, 16, 20), (2, 32, 48), (1, 152, 272)])
-def test_after_conv_chain_on_tensor_cores(n, h, w):
+def test_after_conv_chain_on_tensor_cores_through_the_launchers(n, h, w):
     """The right view's decoder tail as the engine runs it: g_s_conv4 (col2im) + after_gdn writing 16-bit channels 0..2 of a
-    channels-last image, the warp of x1_hat writing channels 4..6 (masic_warp_perspective_fwd2), then after_conv
+    channels-last image, the warp of x1_hat writing channels 4..6 (masic_warp_perspective_fwd), then after_conv
     (ConvTranspose2d(6, 3, 5, stride 1), MASIC.py:600,616) as a conv_tc plan over the pixel-folded view of that image with
     a planar (NCHW fp32) output — against torch on the same fp16-rounded inputs."""
     from masic_b200 import _lib, ops
     from masic_b200.convplan import ConvPlan, DeconvImgPlan, PackedConv, fold8_weights_5x5_s1
     from oracle import hsic as OH
     dev = torch.device("cuda:0")
-    lib = _lib.load()
     torch.manual_seed(7 * h + w)
     H, W = 2 * h, 2 * w
     XOFF, XPAD = _lib.IMG_XOFF, _lib.IMG_XPAD
@@ -72,9 +71,7 @@ def test_after_conv_chain_on_tensor_cores(n, h, w):
     Hm = OH.synthetic_homography(n, seed=3).to(dev)
     T = ops.warp_prepare(Hm, (H, W), (H, W), False)
     w32 = torch.empty(n, 3, H, W, device=dev)
-    _lib.check(lib.masic_warp_perspective_fwd2(img.data_ptr(), n, 3, H, W, H, W, T.data_ptr(), w32.data_ptr(), None, 0, 0, 0,
-                                               1, ac_in.data_ptr(), 8, W + XPAD, XOFF, 4, 1,
-                                               torch.cuda.current_stream().cuda_stream), "masic_warp_perspective_fwd2")
+    ops.warp_perspective_into(img, T, (H, W), dst=w32, dst2=ac_in, dst2_coff=4)
     assert torch.equal(w32, ops.warp_perspective(img, Hm, (H, W)))
     assert torch.equal(ac_in[:, :, XOFF:XOFF + W, 4:7].permute(0, 3, 1, 2), w32.half())
     assert torch.equal(ac_in[:, :, XOFF:XOFF + W, :3].permute(0, 3, 1, 2), out32.half())     # channels 0..2 untouched

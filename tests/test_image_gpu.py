@@ -83,14 +83,13 @@ def test_warp_against_oracle(dev, h, w):
     assert (ident.cpu() - img).abs().max() <= 1e-5
 
 
-def test_fast_warp_is_bit_identical_to_the_generic_kernel_and_fused_mask(dev):
+def test_fast_warp_and_fused_mask_are_bit_identical_to_the_generic_kernel(dev):
     """warp_fast_kernel (the engine's configurations: 3 / 1 channels) must reproduce warp_kernel bit for bit — a 4-channel
-    image takes the generic kernel, its first three planes are the 3-channel image — and masic_warp_perspective_fwd3
+    image takes the generic kernel, its first three planes are the 3-channel image — and masic_warp_perspective_fwd
     writes the warp of the all-ones image (x1_mask_R, MASIC.py:636-638) from the same launch, equal to the separate
     ones-warp; ragged widths (not a multiple of the 256 pixels a block covers), border pixels included."""
-    from masic_b200 import _lib, ops
+    from masic_b200 import ops
     from oracle import hsic as OH
-    lib = _lib.load()
     g = torch.Generator().manual_seed(11)
     for h, w in ((128, 192), (200, 328), (64, 1000)):
         img = torch.rand(2, 3, h, w, generator=g).to(dev)
@@ -103,15 +102,12 @@ def test_fast_warp_is_bit_identical_to_the_generic_kernel_and_fused_mask(dev):
         T = ops.warp_prepare(Hm, (h, w), (h, w), False)
         out = torch.empty_like(img)
         ones = torch.empty(2, 1, h, w, device=dev)
-        s = torch.cuda.current_stream().cuda_stream
-        _lib.check(lib.masic_warp_perspective_fwd3(img.data_ptr(), 2, 3, h, w, h, w, T.data_ptr(), out.data_ptr(), None, 0, 0, 0,
-                                                   0, None, 0, 0, 0, 0, 0, ones.data_ptr(), s), "masic_warp_perspective_fwd3")
+        ops.warp_perspective_into(img, T, (h, w), dst=out, ones=ones)
         assert torch.equal(out, fast) and torch.equal(ones, ones_sep), (h, w)
         # the generic kernel's form of the same call (4 channels): the mask comes from a second launch
         out4 = torch.empty_like(img4)
         ones4 = torch.empty(2, 1, h, w, device=dev)
-        _lib.check(lib.masic_warp_perspective_fwd3(img4.data_ptr(), 2, 4, h, w, h, w, T.data_ptr(), out4.data_ptr(), None, 0, 0,
-                                                   0, 0, None, 0, 0, 0, 0, 0, ones4.data_ptr(), s), "masic_warp_perspective_fwd3")
+        ops.warp_perspective_into(img4, T, (h, w), dst=out4, ones=ones4)
         assert torch.equal(out4, generic) and torch.equal(ones4, ones_sep), (h, w)
 
 
@@ -217,3 +213,43 @@ def test_layout_packs_round_trip(dev):
     assert float(body[..., 6:].abs().max()) == 0 and float((sp[:, :, :_lib.IMG_XOFF] - 7).abs().max()) == 0
     y = torch.rand(2, 9, 11, 200, device=dev)
     assert torch.equal(ops.nhwc_to_nchw_f32(y, 192), y[..., :192].permute(0, 3, 1, 2))
+
+
+def test_launchers_refuse_what_the_kernels_cannot_use_in_place(dev):
+    """The in-place launchers raise MasicError before launching anything when handed a 16-bit image whose rows are
+    neither w_out nor w_out + IMG_XPAD pixels, a non-contiguous or wrong-dtype destination, or a CPU tensor: the
+    refused destination and the valid fp32 destination of the same call keep their contents."""
+    from masic_b200 import _lib, ops
+    from masic_b200._lib import MasicError
+    n, h, w = 2, 16, 24
+    x = torch.rand(n, 3, h, w, device=dev)
+    T = ops.warp_prepare(torch.eye(3, device=dev).repeat(n, 1, 1), (h, w), (h, w))
+    dst = torch.full((n, 3, h, w), 7.0, device=dev)
+    f16 = dict(dtype=torch.float16, device=dev)
+    bad16 = [torch.zeros(n, h, w + 1, 8, **f16),                                  # rows neither w nor w + IMG_XPAD
+             torch.zeros(n, h, w + 2 * _lib.IMG_XPAD, 8, **f16),
+             torch.zeros(n, h, 8, w, **f16).transpose(2, 3),                      # non-contiguous
+             torch.zeros(n, h, w, 8, dtype=torch.float32, device=dev),            # not a 16-bit dtype
+             torch.zeros(n, h, w, 8, dtype=torch.float16)]                        # CPU
+    for bad in bad16:
+        for call in (lambda: ops.warp_perspective_into(x, T, (h, w), dst=dst, dst16=bad),
+                     lambda: ops.warp_perspective_into(x, T, (h, w), dst=dst, dst2=bad, dst2_coff=4),
+                     lambda: ops.nchw_to_nhwc_into(x, bad)):
+            with pytest.raises(MasicError):
+                call()
+    bad32 = [torch.zeros(n, 3, w, h, device=dev).transpose(2, 3),                 # non-contiguous
+             torch.zeros(n, 3, h, w, dtype=torch.float64, device=dev),            # wrong dtype
+             torch.zeros(n, 3, h, w)]                                             # CPU
+    for bad in bad32:
+        with pytest.raises(MasicError):
+            ops.warp_perspective_into(x, T, (h, w), dst=bad)
+        with pytest.raises(MasicError):
+            ops.softmax_channels_into(x, bad)
+    for call in (lambda: ops.warp_perspective_into(x.cpu(), T, (h, w), dst=dst),          # a CPU input
+                 lambda: ops.warp_perspective_into(x, T.cpu(), (h, w), dst=dst),
+                 lambda: ops.softmax_channels_into(x.cpu(), dst)):
+        with pytest.raises(MasicError):
+            call()
+    torch.cuda.synchronize()
+    assert bool((dst == 7.0).all())
+    assert all(float(b.abs().max()) == 0 for b in bad16 + bad32)
