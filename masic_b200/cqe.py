@@ -13,7 +13,7 @@ The whole sequence replays as one CUDA graph.  No CPU path.
 """
 from __future__ import annotations
 
-from typing import Dict, Tuple
+from typing import Dict, Optional, Sequence, Tuple
 
 import torch
 import torch.nn as nn
@@ -115,10 +115,16 @@ class Independent_EN(nn.Module):
 
 
 class CQEEngine(HSICEngine):
-    """Execution plan of Independent_EN.forward for a fixed (batch, H, W): static buffers, conv plans, one graph."""
+    """Execution plan of Independent_EN.forward for a fixed (batch, H, W): static buffers, conv plans, one graph.
+
+    `inputs` (optional): caller-owned device tensors (x1_hat, x2_hat, h_matrix), two (B,3,H,W) fp32 and one (B,3,3)
+    fp32, that the engine reads in place (PairStream binds a slot's codec outputs and homography).  The graph is
+    captured against their pointers and `run()` copies nothing; by default the engine owns those buffers and `run`
+    copies its arguments into them."""
 
     def __init__(self, sd: Dict[str, torch.Tensor], batch: int, height: int, width: int,
-                 device: torch.device | str = "cuda:0", use_graph: bool = True):
+                 device: torch.device | str = "cuda:0", use_graph: bool = True,
+                 inputs: Optional[Sequence[torch.Tensor]] = None):
         if height < 2 or width < 2:
             raise ValueError("Independent_EN needs H, W >= 2 (kornia's normalised grid divides by size-1)")
         self.lib = _lib.load()
@@ -126,6 +132,17 @@ class CQEEngine(HSICEngine):
         if self.dev.type != "cuda":
             raise MasicError("CQEEngine runs on a CUDA device only (no CPU fallback)")
         self.B, self.H, self.W = batch, height, width
+        self.bound = inputs is not None
+        if self.bound:
+            if len(inputs) != 3:
+                raise MasicError("CQEEngine inputs: (x1_hat, x2_hat, h_matrix)")
+            shapes = ((batch, 3, height, width), (batch, 3, height, width), (batch, 3, 3))
+            for t, shape in zip(inputs, shapes):
+                if not (t.device == self.dev and t.dtype == torch.float32 and t.is_contiguous()
+                        and tuple(t.shape) == shape):
+                    raise MasicError(f"CQEEngine inputs must be contiguous float32 tensors of shapes {shapes} on "
+                                     f"{self.dev}; got {tuple(t.shape)} {t.dtype} on {t.device}")
+            self.x1, self.x2, self.Hm = inputs
         self.sd = {k: v.detach().to(self.dev) for k, v in sd.items()}
         self.steps, self.sched, self._lane = [], [], 0
         self.plans, self.buf, self.packs, self._keep = {}, {}, {}, []
@@ -170,9 +187,10 @@ class CQEEngine(HSICEngine):
     def _build(self):
         B, H, W = self.B, self.H, self.W
         f32 = torch.float32
-        self.x1 = self._buf(B, 3, H, W, dtype=f32)       # inputs: the codec's reconstructions
-        self.x2 = self._buf(B, 3, H, W, dtype=f32)
-        self.Hm = torch.eye(3, device=self.dev).repeat(B, 1, 1).contiguous()
+        if not self.bound:
+            self.x1 = self._buf(B, 3, H, W, dtype=f32)       # inputs: the codec's reconstructions
+            self.x2 = self._buf(B, 3, H, W, dtype=f32)
+            self.Hm = torch.eye(3, device=self.dev).repeat(B, 1, 1).contiguous()
         o = self.out = {"x1_hat": self._buf(B, 3, H, W, dtype=f32), "x2_hat": self._buf(B, 3, H, W, dtype=f32)}
         T = torch.empty(B, 3, 3, device=self.dev, dtype=torch.float64)
         Tinv = torch.empty(B, 3, 3, device=self.dev, dtype=torch.float64)
@@ -235,3 +253,9 @@ class CQEEngine(HSICEngine):
             self._add(f"{v}.residual_image", lambda c2=c2, x_self=x_self, dst=o[okey]:
                       ops.cqe_residual_image_into(c2, x_self, dst))                         # :1495-1496
         self.flops = sum(p.flops for p in self.plans.values())
+
+    def run(self, x1: Optional[torch.Tensor] = None, x2: Optional[torch.Tensor] = None,
+            h_matrix: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        if self.bound and not (x1 is None and x2 is None and h_matrix is None):
+            raise MasicError("this CQEEngine reads the tensors it was built with in place: call run() without inputs")
+        return super().run(x1, x2, h_matrix)

@@ -299,13 +299,18 @@ class PairStream:
         t2 = ps.submit(..., msssim=True)             # + MS-SSIM of both views, in result(t2)[3]
         ps.attach_lpips(lpips_net)                   # a masic_b200.lpips.LPIPS
         t3 = ps.submit(..., lpips=True)              # + LPIPS of both views, in result(t3)[3]
+        ps.attach_enhancement(en)                    # a masic_b200.cqe.Independent_EN: full MASIC (test3_real.py)
+        t4 = ps.submit(..., enhance=True, msssim=True, lpips=True)   # every number of the enhanced pair
 
     `depth` slots (default 2), each with its own engine and stream: the H2D copy of pair i+1 runs on a copy stream
     while pair i replays its engine's CUDA graph, and the kernels of consecutive pairs overlap on the GPU; the
     criterion is one fused reduction pass (masic_rd_metrics) whose 8 floats come back through pinned memory; with
     msssim=True the slot's stream also runs masic_ms_ssim on both views and 6 more floats ride in the same read-back;
-    with lpips=True its LPIPS engine compares both views and 2 more floats ride along.
-    `outputs()` exposes the engine's output tensors of the LAST submitted pair (valid after `result(ticket)`).
+    with lpips=True its LPIPS engine compares both views and 2 more floats ride along.  With enhance=True the slot's
+    CQE engine replays right after the codec, reading the codec's buffers in place, and everything above measures the
+    enhanced pair; a second masic_rd_metrics pass adds the codec's own MSE to the same read-back.
+    `outputs()` exposes the engine's output tensors of the LAST submitted pair (valid after `result(ticket)`),
+    `enhanced_outputs()` the enhanced pair of the last one submitted with enhance=True.
     """
 
     def __init__(self, model: "HSIC", height: int, width: int, device, depth: int = 2, lmbda: float = 0.0):
@@ -334,17 +339,20 @@ class PairStream:
                 liks = [o["lik_y1"], o["lik_y2"], o["lik_z1"], o["lik_z2"]]
                 self.slots.append(dict(
                     eng=eng, stream=torch.cuda.Stream(device=self.dev),
-                    # criterion (8 floats) | MS-SSIM per channel of view 1 (3) and view 2 (3) | LPIPS of view 1, 2
-                    res_d=torch.zeros(16, device=self.dev), res_h=torch.zeros(16).pin_memory(),
+                    # criterion (8 floats) | MS-SSIM per channel of view 1 (3) and view 2 (3) | LPIPS of view 1, 2 |
+                    # with enhance=True, masic_rd_metrics of the codec's (unenhanced) pair (8)
+                    res_d=torch.zeros(24, device=self.dev), res_h=torch.zeros(24).pin_memory(),
                     copied=torch.cuda.Event(), done=torch.cuda.Event(), busy=False, has_result=False,
                     scratch=_ops.rd_metrics_scratch(self.dev),
                     lik_p=(C.c_void_p * 4)(*[t.data_ptr() for t in liks]),
                     lik_n=(C.c_int64 * 4)(*[t.numel() for t in liks])))
         self._ms_weights = (C.c_float * 5)(*_ops.MS_SSIM_WEIGHTS)
+        self._no_lik_p, self._no_lik_n = (C.c_void_p * 4)(), (C.c_int64 * 4)()
         self._n = 0
+        self.enh_out: Optional[Dict[str, torch.Tensor]] = None
 
     def submit(self, x1: torch.Tensor, x2: torch.Tensor, h: torch.Tensor, criterion: bool = True,
-               want_recon: bool = False, msssim: bool = False, lpips: bool = False) -> int:
+               want_recon: bool = False, msssim: bool = False, lpips: bool = False, enhance: bool = False) -> int:
         """Queue one pair.  x1 / x2: (1,3,H,W) uint8 images as they come out of the dataset's PNG files (the recommended
         host format: converted on the device exactly like torchvision's ToTensor, a quarter of the PCIe bytes, which is
         what keeps eight ranks on one host from becoming host-bound), or float32 in [0,1] as the reference's loaders
@@ -355,13 +363,18 @@ class PairStream:
         msssim=True (with the criterion) also computes pytorch_msssim's ms_ssim(x_hat, x, data_range=1.0) of both views
         on the device (the third number of the reference's eval loop); `result` then reports it.  It needs
         min(H, W) > 160, as the package does.  lpips=True (with the criterion, after attach_lpips) also computes
-        lpips.LPIPS(x_hat, x) of both views on the device (the fourth number of the eval loop)."""
+        lpips.LPIPS(x_hat, x) of both views on the device (the fourth number of the eval loop).
+        enhance=True (after attach_enhancement) runs full MASIC, as test3_real.py does: Independent_EN post-filters the
+        decoded pair on the device, and the PSNRs, MSEs, loss, MS-SSIM, LPIPS and want_recon all refer to the enhanced
+        pair; bpp still comes from the codec's likelihoods, and `result` adds the codec's own PSNR and MSE."""
         from ._lib import check
         if msssim and not criterion:
             raise ValueError("msssim=True is part of the criterion: it needs criterion=True")
         if lpips and not criterion:
             raise ValueError("lpips=True is part of the criterion: it needs criterion=True")
         s = self.slots[self._n % self.depth]
+        if enhance and "cqe" not in s:
+            raise MasicError("submit(enhance=True): call attach_enhancement(en) first")
         if lpips and "lpips" not in s:
             raise MasicError("submit(lpips=True): call attach_lpips(net) first")
         if msssim and "ms_scratch" not in s:
@@ -392,33 +405,37 @@ class PairStream:
                     check(self.lib.masic_u8_to_unit_f32(src.data_ptr(), src.numel(), dst.data_ptr(), st.cuda_stream),
                           "masic_u8_to_unit_f32")
             o = eng.run()
+            rec = s["cqe"].run() if enhance else o      # the CQE graph reads o["x1_hat"], o["x2_hat"], eng.Hm in place
             if criterion:
-                check(self.lib.masic_rd_metrics(s["lik_p"], s["lik_n"], o["x1_hat"].data_ptr(), eng.x1.data_ptr(),
-                                                o["x2_hat"].data_ptr(), eng.x2.data_ptr(), 1, 3, self.H, self.W,
+                check(self.lib.masic_rd_metrics(s["lik_p"], s["lik_n"], rec["x1_hat"].data_ptr(), eng.x1.data_ptr(),
+                                                rec["x2_hat"].data_ptr(), eng.x2.data_ptr(), 1, 3, self.H, self.W,
                                                 self.lmbda, s["scratch"].data_ptr(), s["res_d"].data_ptr(),
                                                 st.cuda_stream), "masic_rd_metrics")
+                if enhance:                             # the codec's own MSE (no likelihoods: its bpp is the above)
+                    check(self.lib.masic_rd_metrics(self._no_lik_p, self._no_lik_n, o["x1_hat"].data_ptr(),
+                                                    eng.x1.data_ptr(), o["x2_hat"].data_ptr(), eng.x2.data_ptr(), 1, 3,
+                                                    self.H, self.W, self.lmbda, s["scratch"].data_ptr(),
+                                                    s["res_d"][16:].data_ptr(), st.cuda_stream), "masic_rd_metrics")
                 if msssim:
-                    for v, (xh, x) in enumerate(((o["x1_hat"], eng.x1), (o["x2_hat"], eng.x2))):
+                    for v, (xh, x) in enumerate(((rec["x1_hat"], eng.x1), (rec["x2_hat"], eng.x2))):
                         check(self.lib.masic_ms_ssim(xh.data_ptr(), x.data_ptr(), 1, 3, self.H, self.W, 5, 1.0, 0.01,
                                                      0.03, self._ms_weights, 1, s["ms_scratch"].data_ptr(),
                                                      s["res_d"][8 + 3 * v:].data_ptr(), st.cuda_stream), "masic_ms_ssim")
                 if lpips:
-                    total, _ = s["lpips"].run(normalize=s["lpips_normalize"])
+                    total, _ = s["lpips_enh" if enhance else "lpips"].run(normalize=self._lpips_normalize)
                     s["res_d"][14:16].copy_(total, non_blocking=True)
-                    s["res_h"].copy_(s["res_d"], non_blocking=True)
-                elif msssim:
-                    s["res_h"][:14].copy_(s["res_d"][:14], non_blocking=True)
-                else:
-                    s["res_h"][:8].copy_(s["res_d"][:8], non_blocking=True)
+                n = 24 if enhance else 16 if lpips else 14 if msssim else 8
+                s["res_h"][:n].copy_(s["res_d"][:n], non_blocking=True)
             if want_recon:
                 if "rec_h" not in s:
                     s["rec_h"] = [torch.empty(1, 3, self.H, self.W).pin_memory() for _ in range(2)]
-                s["rec_h"][0].copy_(o["x1_hat"], non_blocking=True)
-                s["rec_h"][1].copy_(o["x2_hat"], non_blocking=True)
+                s["rec_h"][0].copy_(rec["x1_hat"], non_blocking=True)
+                s["rec_h"][1].copy_(rec["x2_hat"], non_blocking=True)
             s["done"].record(st)
         s["busy"], s["has_result"], s["has_recon"], s["has_msssim"] = True, criterion, want_recon, msssim
-        s["has_lpips"] = lpips
+        s["has_lpips"], s["has_enhance"] = lpips, enhance
         self.eng = eng
+        self.enh_out = rec if enhance else None
         self._n += 1
         return self._n - 1
 
@@ -434,19 +451,45 @@ class PairStream:
     def attach_lpips(self, net, normalize: bool = True) -> None:
         """`net`: a masic_b200.lpips.LPIPS.  Each slot gets an LPIPSEngine of batch 4, [x1_hat, x2_hat, x1, x2], that
         reads the slot's codec buffers in place.  The stream's images are in [0, 1] (ToTensor), which lpips wants as
-        forward(..., normalize=True); normalize=False reproduces a script that passes them without the flag."""
-        from .lpips import LPIPSEngine
-        sd = net.state_dict()
+        forward(..., normalize=True); normalize=False reproduces a script that passes them without the flag.  Once an
+        enhancement net is attached too (either order), a second engine per slot reads the enhanced pair instead."""
+        self._lpips_sd = {k: v.detach().clone() for k, v in net.state_dict().items()}
+        self._lpips_normalize = bool(normalize)
         for s in self.slots:
+            if s["busy"]:
+                s["done"].synchronize()             # the engines replaced below may still be in use
+            s["lpips"] = self._lpips_engine(s, s["eng"].out)
+            if "cqe" in s:
+                s["lpips_enh"] = self._lpips_engine(s, s["cqe"].out)
+
+    def _lpips_engine(self, s, rec: Dict[str, torch.Tensor]):
+        """An LPIPSEngine that compares the reconstructions `rec` with the slot's originals, reading both in place."""
+        from .lpips import LPIPSEngine
+        eng = s["eng"]
+        e = LPIPSEngine(self._lpips_sd, 2, self.H, self.W, self.dev,
+                        inputs=[rec["x1_hat"], rec["x2_hat"], eng.x1, eng.x2])
+        e.prepare(self._lpips_normalize)
+        return e
+
+    # ---- full MASIC: the cross quality enhancement network after the codec (test3_real.py)
+    def attach_enhancement(self, en) -> None:
+        """`en`: a masic_b200.cqe.Independent_EN on this device.  Each slot gets a CQEEngine of batch 1 that reads the
+        slot's codec outputs and homography in place, for submit(..., enhance=True).  The engines hold a snapshot of
+        the weights taken now: call again after changing them."""
+        from .cqe import CQEEngine
+        sd = {k: v.detach().clone() for k, v in en.state_dict().items()}
+        for s in self.slots:
+            if s["busy"]:
+                s["done"].synchronize()             # the engines replaced below may still be in use
             eng = s["eng"]
-            s["lpips"] = LPIPSEngine(sd, 2, self.H, self.W, self.dev,
-                                     inputs=[eng.out["x1_hat"], eng.out["x2_hat"], eng.x1, eng.x2])
-            s["lpips"].prepare(normalize)
-            s["lpips_normalize"] = bool(normalize)
+            s["cqe"] = CQEEngine(sd, 1, self.H, self.W, self.dev, use_graph=en._use_graph,
+                                 inputs=(eng.out["x1_hat"], eng.out["x2_hat"], eng.Hm))
+            if "lpips" in s:
+                s["lpips_enh"] = self._lpips_engine(s, s["cqe"].out)
 
     def submit_patches(self, x1: torch.Tensor, x2: torch.Tensor, patch_a: torch.Tensor, patch_b: torch.Tensor,
                        corners: torch.Tensor, criterion: bool = True, want_recon: bool = False,
-                       msssim: bool = False, lpips: bool = False) -> int:
+                       msssim: bool = False, lpips: bool = False, enhance: bool = False) -> int:
         """Like `submit`, but instead of h_matrix takes what the dataset hands over (datasets/utils.py:383-395): the two
         (1,1,128,128) normalised grey patches and their (1,4,2) corner coordinates.  The udh net, the 4-point DLT,
         the inverse and h_adjust (test2_real.py:201-211) run on the slot's stream ahead of the codec; the host never
@@ -471,13 +514,16 @@ class PairStream:
             ev2 = torch.cuda.Event()
             ev2.record(s["stream"])
         self.copy_stream.wait_event(ev2)            # submit() copies h on the copy stream
-        return self.submit(x1, x2, h, criterion=criterion, want_recon=want_recon, msssim=msssim, lpips=lpips)
+        return self.submit(x1, x2, h, criterion=criterion, want_recon=want_recon, msssim=msssim, lpips=lpips,
+                           enhance=enhance)
 
     def result(self, ticket: int):
         """(bpp, psnr1_db, psnr2_db, detail) of a submitted pair; blocks until its D2H copy has landed.  A pair
         submitted with msssim=True also has detail["msssim1"/"msssim2"] (mean over the 3 channels, as
         pytorch_msssim's size_average) and "msssim1_db"/"msssim2_db" = -10 log10(1 - value); one submitted with
-        lpips=True has detail["lpips1"/"lpips2"]."""
+        lpips=True has detail["lpips1"/"lpips2"].  For a pair submitted with enhance=True the PSNRs and every value
+        above but the bpp are those of the enhanced pair, and detail["codec_psnr1"/"codec_psnr2"/"codec_mse1"/
+        "codec_mse2"] are those of the codec's reconstructions."""
         if not (self._n - self.depth <= ticket < self._n):
             raise ValueError(f"ticket {ticket} is no longer (or not yet) in flight")
         s = self.slots[ticket % self.depth]
@@ -485,7 +531,7 @@ class PairStream:
         if not s["has_result"]:
             return None
         r = s["res_h"].tolist()
-        psnr = [10.0 * math.log10(1.0 / m) if m > 0 else float("inf") for m in r[4:6]]
+        psnr = [10.0 * math.log10(1.0 / m) if m > 0 else float("inf") for m in r[4:6] + r[20:22]]
         detail = {"bpp_y1": r[0], "bpp_y2": r[1], "bpp_z1": r[2], "bpp_z2": r[3], "mse1": r[4], "mse2": r[5],
                   "loss": r[7]}
         if s["has_msssim"]:
@@ -495,6 +541,8 @@ class PairStream:
                 detail[f"msssim{v}_db"] = -10.0 * math.log10(1.0 - m) if m < 1.0 else float("inf")
         if s["has_lpips"]:
             detail["lpips1"], detail["lpips2"] = r[14], r[15]
+        if s["has_enhance"]:
+            detail.update(codec_psnr1=psnr[2], codec_psnr2=psnr[3], codec_mse1=r[20], codec_mse2=r[21])
         return r[6], psnr[0], psnr[1], detail
 
     def reconstructions(self, ticket: int):
@@ -510,6 +558,14 @@ class PairStream:
 
     def outputs(self) -> Dict[str, torch.Tensor]:
         return self.eng.out
+
+    def enhanced_outputs(self) -> Dict[str, torch.Tensor]:
+        """{"x1_hat", "x2_hat"} of the last submitted pair after the enhancement network, the keys of
+        Independent_EN.forward: the slot's CQE output buffers (valid after `result(ticket)`, until the slot is reused).
+        The last pair must have been submitted with enhance=True."""
+        if self.enh_out is None:
+            raise MasicError("enhanced_outputs: the last pair was submitted without enhance=True")
+        return self.enh_out
 
     def join(self, stream: Optional[torch.cuda.Stream] = None) -> None:
         """Make `stream` (default: the current stream) wait for every pair submitted so far (device-side, no host sync)."""
