@@ -291,6 +291,47 @@ int masic_wave_gather(const void* ypad16, int w16, int m, const void* gmm_in16, 
 /* px16[i][c0 : c0+nc] = ctx_out16[i][2][2][c0 : c0+nc] (the centre pixel of every crop's context output) */
 int masic_wave_center(const void* ctx_out16, int cin, int c0, int nc, int n, void* px16, void* stream);
 
+/* --- format 2 for several pairs at once (HSIC.compress_batch / decompress_batch in masic_b200/bitstream.py) ---
+ * All pairs share H, W and so the wave schedule.  A STREAM is one (pair, view, non-zero channel); the stream tables
+ * stream_pair / stream_ch / stream_minmax (device int32, n_streams entries) give its pair index, channel and the pair's
+ * minmax (1 <= stream_minmax[s] <= max_minmax).  Pair b's tensors follow pair b-1's in every batched buffer.  A count
+ * of zero streams or positions is an empty call; negative counts, NULL pointers and misaligned channel counts return
+ * MASIC_EINVAL before any launch.  All pointers are device pointers.
+ *
+ * masic_gmm_symbol_cdfs for listed streams: element (p, s) reads the parameters and y_hat of position
+ * stream_pair[s] * pair_stride + p; rows (optional) are (n_pos, n_streams, row_pitch) int32 with
+ * row_pitch >= 2 * max_minmax + 2, of which stream s fills 2 * stream_minmax[s] + 2; intervals (optional) are
+ * (n_pos, n_streams, 3). */
+int masic_gmm_symbol_cdfs_pairs(const float* sigma_nhwc, const float* mu_nhwc, const float* weights_nhwc,
+                                int weights_are_logits, int m, int k, int64_t n_pos, int64_t pair_stride,
+                                const int32_t* stream_pair, const int32_t* stream_ch, const int32_t* stream_minmax,
+                                int n_streams, int max_minmax, float scale_bound, const float* y_hat_nhwc, int32_t* rows,
+                                int row_pitch, int32_t* intervals, void* stream);
+/* masic_wave_gather for n_pairs pairs: ypad16 (n_pairs, h16+4, w16+4, m), gmm_in16 (n_pairs, h16, w16, cin), mask_weights
+ * (n_pairs, h16, w16, 3); position i of pair b goes to row b * n_max + i of crop16 / rs / px16 (n_max >= n). */
+int masic_wave_gather_pairs(const void* ypad16, int h16, int w16, int m, const void* gmm_in16, int cin, int c_lo,
+                            int c_hi0, const float* mask_weights, const int32_t* pos_hw, int n, int n_pairs, int n_max,
+                            void* crop16, float* rs, void* px16, void* stream);
+/* masic_range_decode_wave for listed streams: rows (n, n_streams, row_pitch) from masic_gmm_symbol_cdfs_pairs; stream s
+ * writes into pair stream_pair[s]'s slice of y_nhwc (n_pairs, h16, w16, m) and ypad16 (n_pairs, h16+4, w16+4, m). */
+int masic_range_decode_wave_pairs(const int32_t* rows, int n, int n_streams, int row_pitch, void* state,
+                                  const uint8_t* data, const int64_t* offsets, const int32_t* stream_pair,
+                                  const int32_t* stream_ch, const int32_t* stream_minmax, int max_minmax,
+                                  const int32_t* pos_hw, int h16, int w16, int m, float* y_nhwc, void* ypad16, int f16,
+                                  int* error_flag, void* stream);
+/* masic_range_encode_channels on the device, one thread per stream: stream s codes the n_pos intervals
+ * intervals[(base[s] + i * stride[s]) * 3 + 0..2] (int32 cum, freq, total; base / stride int64) into
+ * slots[s * slot_cap ...] (slot_cap >= 3 * n_pos + 16) and writes its byte count to lens[s] (int64).  The bytes equal
+ * masic_range_encode_channels' for the same intervals.  *error_flag = 1 after an interval that coder rejects
+ * (cum < 0, freq <= 0, cum + freq > total, total > 2^22), 2 after a slot overflow. */
+int masic_range_encode_streams(const int32_t* intervals, const int64_t* base, const int64_t* stride, int64_t n_pos,
+                               int n_streams, uint8_t* slots, int64_t slot_cap, int64_t* lens, int* error_flag,
+                               void* stream);
+/* offsets (n_streams + 1) int64 = exclusive prefix sum of lens (offsets[n_streams] = total bytes), then slot s copied
+ * to packed[offsets[s] ...]; packed needs room for the total (n_streams * slot_cap always suffices). */
+int masic_pack_streams(const uint8_t* slots, int64_t slot_cap, const int64_t* lens, int n_streams, int64_t* offsets,
+                       uint8_t* packed, void* stream);
+
 /* rANS serialisation of the z side information with the byte format of the reference's `compressai.ans`
  * extension (compressai/cpp_exts/rans/rans_interface.cpp: BufferedRansEncoder.encode_with_indexes :108-173,
  * flush :175-200, RansDecoder.set_stream :270-276, decode_stream :278-343; reached from

@@ -139,6 +139,11 @@ def _declare(lib: C.CDLL) -> None:
         "masic_range_decode_wave": (i, [vp, i, i, i, vp, vp, vp, vp, i, vp, i, i, vp, vp, i, vp, vp]),
         "masic_wave_gather": (i, [vp, i, i, vp, i, i, i, vp, vp, i, vp, vp, vp, vp]),
         "masic_wave_center": (i, [vp, i, i, i, i, vp, vp]),
+        "masic_gmm_symbol_cdfs_pairs": (i, [vp, vp, vp, i, i, i, i64, i64, vp, vp, vp, i, i, f, vp, vp, i, vp, vp]),
+        "masic_wave_gather_pairs": (i, [vp, i, i, i, vp, i, i, i, vp, vp, i, i, i, vp, vp, vp, vp]),
+        "masic_range_decode_wave_pairs": (i, [vp, i, i, i, vp, vp, vp, vp, vp, vp, i, vp, i, i, i, vp, vp, i, vp, vp]),
+        "masic_range_encode_streams": (i, [vp, vp, vp, i64, i, vp, i64, vp, vp, vp]),
+        "masic_pack_streams": (i, [vp, i64, vp, i, vp, vp, vp]),
         "masic_rans_encoder_create": (i, [C.POINTER(vp)]),
         "masic_rans_encoder_push": (i, [vp, vp, vp, i64, vp, i, i, vp, vp]),
         "masic_rans_encoder_flush": (i, [vp, C.POINTER(vp), C.POINTER(i64)]),

@@ -465,17 +465,22 @@ template <int K>
 __global__ void __launch_bounds__(256)
 gmm_cdf_kernel(const float* __restrict__ sigma, const float* __restrict__ mu, const float* __restrict__ wgt,
                int w_is_logits, int M, long n_pos, const int32_t* __restrict__ ch_list, int n_ch, int minmax,
-               float scale_bound, const float* __restrict__ y_hat_nhwc, int32_t* __restrict__ rows,
-               int32_t* __restrict__ intervals) {
-  extern __shared__ float cdf_smem[];             // [warps per block][L]: the clipped pmf of each warp's element
+               const int32_t* __restrict__ s_pair, const int32_t* __restrict__ s_minmax, long pair_stride,
+               int row_pitch, int L_max, float scale_bound, const float* __restrict__ y_hat_nhwc,
+               int32_t* __restrict__ rows, int32_t* __restrict__ intervals) {
+  // element (pos, j) of stream j: channel ch_list[j] of pair s_pair[j] (0 without a table) under its own minmax
+  extern __shared__ float cdf_smem[];             // [warps per block][L_max]: the clipped pmf of each warp's element
   const int warp_in_block = threadIdx.x >> 5;
   const long wid = (long)blockIdx.x * (blockDim.x >> 5) + warp_in_block;
   const int lane = threadIdx.x & 31;
   if (wid >= n_pos * n_ch) return;
-  const long pos = wid / n_ch;
-  const int ch = ch_list[wid - pos * n_ch];
+  const long pos_w = wid / n_ch;
+  const int j = (int)(wid - pos_w * n_ch);
+  const int ch = ch_list[j];
+  if (s_minmax) minmax = s_minmax[j];
+  const long pos = (s_pair ? s_pair[j] * pair_stride : 0) + pos_w;
   const int L = 2 * minmax + 1;
-  float* pmf = cdf_smem + (size_t)warp_in_block * L;
+  float* pmf = cdf_smem + (size_t)warp_in_block * L_max;
   float s_k[K], m_k[K], w_k[K];
   const long base = pos * (long)(M * K) + ch;
 #pragma unroll
@@ -512,7 +517,7 @@ gmm_cdf_kernel(const float* __restrict__ sigma, const float* __restrict__ mu, co
   // pass 2: rounded counts and their running sum, 32 samples at a time
   const int sym = y_hat_nhwc ? (int)y_hat_nhwc[pos * (long)M + ch] + minmax : -1;
   int run = 0, lo = 0, fr = 0;
-  int32_t* row = rows ? rows + wid * (long)(L + 1) : nullptr;
+  int32_t* row = rows ? rows + wid * (long)row_pitch : nullptr;
   if (row && lane == 0) row[0] = 0;
   for (int s0 = 0; s0 < L; s0 += 32) {
     const int s = s0 + lane;
@@ -633,17 +638,14 @@ extern "C" int masic_latent_prep(const float* y_nhwc, int64_t n_pixels, int c, v
   return (int)cudaGetLastError();
 }
 
-extern "C" int masic_gmm_symbol_cdfs(const float* sigma_nhwc, const float* mu_nhwc, const float* weights_nhwc,
-                                     int weights_are_logits, int m, int k, int64_t n_pos,
-                                     const int32_t* ch_list, int n_ch, int minmax, float scale_bound,
-                                     const float* y_hat_nhwc, int32_t* rows, int32_t* intervals, void* stream) {
-  if (!sigma_nhwc || !mu_nhwc || !weights_nhwc || !ch_list || m <= 0 || n_pos < 0 || n_ch < 0 || minmax < 1 ||
-      minmax > 32767 || (!rows && !intervals) || (intervals && !y_hat_nhwc))
-    return MASIC_EINVAL;
-  if (k != 5) return MASIC_ENOSUP;
+// one launch of gmm_cdf_kernel: pmf rows of up to L_max = 2 * max_minmax + 1 floats per warp in shared memory
+static int launch_gmm_cdfs(const float* sigma, const float* mu, const float* wgt, int w_is_logits, int m, int64_t n_pos,
+                           const int32_t* ch_list, int n_ch, int minmax, const int32_t* s_pair, const int32_t* s_minmax,
+                           int64_t pair_stride, int row_pitch, int max_minmax, float scale_bound, const float* y_hat,
+                           int32_t* rows, int32_t* intervals, cudaStream_t stream) {
   const long warps = n_pos * n_ch;
   if (warps == 0) return MASIC_OK;
-  const int L = 2 * minmax + 1;
+  const int L = 2 * max_minmax + 1;
   int wpb = 8;                                      // warps per block, limited by L floats of shared memory per warp
   while (wpb > 1 && (size_t)wpb * L * sizeof(float) > 96 * 1024) wpb >>= 1;
   const size_t smem = (size_t)wpb * L * sizeof(float);
@@ -653,8 +655,37 @@ extern "C" int masic_gmm_symbol_cdfs(const float* sigma_nhwc, const float* mu_nh
     if (e != cudaSuccess) return (int)e;
   }
   const long blocks = (warps + wpb - 1) / wpb;
-  gmm_cdf_kernel<5><<<(unsigned)blocks, wpb * 32, smem, static_cast<cudaStream_t>(stream)>>>(
-      sigma_nhwc, mu_nhwc, weights_nhwc, weights_are_logits, m, n_pos, ch_list, n_ch, minmax, scale_bound,
-      y_hat_nhwc, rows, intervals);
+  gmm_cdf_kernel<5><<<(unsigned)blocks, wpb * 32, smem, stream>>>(
+      sigma, mu, wgt, w_is_logits, m, n_pos, ch_list, n_ch, minmax, s_pair, s_minmax, pair_stride, row_pitch, L,
+      scale_bound, y_hat, rows, intervals);
   return (int)cudaGetLastError();
+}
+
+extern "C" int masic_gmm_symbol_cdfs(const float* sigma_nhwc, const float* mu_nhwc, const float* weights_nhwc,
+                                     int weights_are_logits, int m, int k, int64_t n_pos,
+                                     const int32_t* ch_list, int n_ch, int minmax, float scale_bound,
+                                     const float* y_hat_nhwc, int32_t* rows, int32_t* intervals, void* stream) {
+  if (!sigma_nhwc || !mu_nhwc || !weights_nhwc || !ch_list || m <= 0 || n_pos < 0 || n_ch < 0 || minmax < 1 ||
+      minmax > 32767 || (!rows && !intervals) || (intervals && !y_hat_nhwc))
+    return MASIC_EINVAL;
+  if (k != 5) return MASIC_ENOSUP;
+  return launch_gmm_cdfs(sigma_nhwc, mu_nhwc, weights_nhwc, weights_are_logits, m, n_pos, ch_list, n_ch, minmax, nullptr,
+                         nullptr, 0, 2 * minmax + 2, minmax, scale_bound, y_hat_nhwc, rows, intervals,
+                         static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int masic_gmm_symbol_cdfs_pairs(const float* sigma_nhwc, const float* mu_nhwc, const float* weights_nhwc,
+                                           int weights_are_logits, int m, int k, int64_t n_pos, int64_t pair_stride,
+                                           const int32_t* stream_pair, const int32_t* stream_ch,
+                                           const int32_t* stream_minmax, int n_streams, int max_minmax,
+                                           float scale_bound, const float* y_hat_nhwc, int32_t* rows, int row_pitch,
+                                           int32_t* intervals, void* stream) {
+  if (!sigma_nhwc || !mu_nhwc || !weights_nhwc || !stream_pair || !stream_ch || !stream_minmax || m <= 0 ||
+      n_pos < 0 || pair_stride < 0 || n_streams < 0 || max_minmax < 1 || max_minmax > 32767 || (!rows && !intervals) ||
+      (intervals && !y_hat_nhwc) || (rows && row_pitch < 2 * max_minmax + 2))
+    return MASIC_EINVAL;
+  if (k != 5) return MASIC_ENOSUP;
+  return launch_gmm_cdfs(sigma_nhwc, mu_nhwc, weights_nhwc, weights_are_logits, m, n_pos, stream_ch, n_streams, 0,
+                         stream_pair, stream_minmax, pair_stride, row_pitch, max_minmax, scale_bound, y_hat_nhwc, rows,
+                         intervals, static_cast<cudaStream_t>(stream));
 }

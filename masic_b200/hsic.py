@@ -287,6 +287,19 @@ class HSIC(nn.Module):
         return decompress(self, x1, x2, h_matrix, output_name, output_path,
                           None if device == "cpu" else device)
 
+    def compress_batch(self, x1, x2, h_matrix):
+        """Code B pairs of one size at once (B, 3, H, W device tensors; h_matrix (B, 3, 3)).  Returns one dict per pair:
+        `header` and `payload`, the bytes `compress` writes to `<name>.npz` / `<name>.bin` for that pair alone, and
+        `bpp_real`, `n_symbols`, `y_bits_ideal`.  See masic_b200/bitstream.py."""
+        from .bitstream import compress_batch
+        return compress_batch(self, x1, x2, h_matrix)
+
+    def decompress_batch(self, items, h_matrix, device=None):
+        """Decode a list of (header, payload) byte strings of pairs of one size (format 2) with their (B, 3, 3)
+        homographies.  Returns x1_hat, x2_hat, y1_hat, y2_hat, z1_hat, z2_hat, batched in the order of items."""
+        from .bitstream import decompress_batch
+        return decompress_batch(self, items, h_matrix, device)
+
 
 class PairStream:
     """Pipelined evaluation of stereo pairs that live in HOST memory (the reference's eval loop,
