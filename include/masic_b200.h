@@ -390,6 +390,10 @@ int masic_fc_bf16(const void* x_bf16, int x_batch_stride, const void* w_bf16, co
  * identity).  8x8 solve and 3x3 inverse in fp64. */
 int masic_homography_from_delta(const float* corners, const float* delta, int batch, int shift_corners, int img_h,
                                 int img_w, int pic_h, int pic_w, float* h_out, void* stream);
+/* The (n,3,3) fp32 homographies h_in in the zero-padded frame: h_out = T h_in T^-1, T the translation by (left, top)
+ * (pixel coordinates, as the warp reads them).  fp64, one thread per matrix, each product and sum rounded in a fixed
+ * order, rounded once to fp32.  h_out may be h_in. */
+int masic_homography_pad(const float* h_in, int n, int top, int left, float* h_out, void* stream);
 
 /* ------------------------------------------------------------ image domain */
 /* kornia.warp_perspective(src, M, (h_out, w_out)) — kornia 0.5.0, call sites MASIC.py:781,821,833.
@@ -457,6 +461,13 @@ int masic_nhwc_to_nchw_f32(const float* in_nhwc, int n, int c, int hw, int in_pi
 /* 8-bit image -> float32 in [0,1]: torchvision.transforms.ToTensor as the reference's datasets apply it
  * (img.float().div(255), IEEE division); lets a caller ship 8-bit images over PCIe (PairStream.submit). */
 int masic_u8_to_unit_f32(const uint8_t* in_u8, int64_t numel, float* out_f32, void* stream);
+/* Zero padding of NCHW images (n,c,h,w) into the float32 frame (n,c,hp,wp), source pixel (y,x) at (y+top, x+left): the
+ * codec's frame for pairs whose size is not a multiple of 64 (masic_b200/padding.py).  src is uint8 (src_u8 = 1,
+ * converted like masic_u8_to_unit_f32, bit for bit) or float32 (copied).  Every element of dst is written, the zero
+ * border included, so dst needs no memset.  dst_unpadded (may be NULL): the float32 (n,c,h,w) image from the same pass.
+ * Memory-bound: n*c*(h*w*s_in + hp*wp*4 [+ h*w*4]) bytes; 16-byte stores when wp % 4 == 0 and dst is 16-byte aligned. */
+int masic_pad_image(const void* src, int src_u8, int n, int c, int h, int w, int hp, int wp, int top, int left,
+                    float* dst, float* dst_unpadded, void* stream);
 
 /* ------------------------------------------------- cross quality enhancement (CQE) glue */
 /* Independent_EN (coremasic/mywork/MASIC.py:1436-1501).  Its 3x3 convs run as MASIC_CONV plans with LeakyReLU and

@@ -161,6 +161,7 @@ def _declare(lib: C.CDLL) -> None:
         "masic_fc_pack_weights": (i, [vp, i, i, i, vp, i, vp]),
         "masic_fc_bf16": (i, [vp, i, vp, vp, i, i, i, i, vp, vp, i, i, vp]),
         "masic_homography_from_delta": (i, [vp, vp, i, i, i, i, i, i, vp, vp]),
+        "masic_homography_pad": (i, [vp, i, i, i, vp, vp]),
         "masic_warp_prepare": (i, [vp, i, i, i, i, i, i, vp, vp]),
         "masic_warp_perspective_fwd": (i, [vp, i, i, i, i, i, i, vp, vp, vp, i, i, i, i, vp, i, i, i, i, i, vp, vp]),
         "masic_conv_small_nchw": (i, [vp, i, vp, i, i, i, i, vp, i, vp, i, i, i, i, i, vp, vp, f, vp, vp, i, i, i, i, vp]),
@@ -170,6 +171,7 @@ def _declare(lib: C.CDLL) -> None:
         "masic_softmax_channels": (i, [vp, i, i, i, vp, vp, vp]),
         "masic_nchw_to_nhwc_bf16": (i, [vp, i, i, i, i, vp, i, i, i, i, vp]),
         "masic_u8_to_unit_f32": (i, [vp, i64, vp, vp]),
+        "masic_pad_image": (i, [vp, i, i, i, i, i, i, i, i, i, vp, vp, vp]),
         "masic_nhwc_to_nchw_f32": (i, [vp, i, i, i, i, vp, vp]),
         "masic_wgrad_plan_create": (i, [C.POINTER(WgradDesc), C.POINTER(vp)]),
         "masic_wgrad_plan_workspace_bytes": (i64, [vp]),

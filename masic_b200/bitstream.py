@@ -42,6 +42,8 @@ from . import _lib
 from ._lib import MasicError, check
 from .convplan import ACT_LEAKY, ACT_NONE, ACT_RELU, MASK_A_5x5, ConvPlan
 from .engine import ACT, SCALE_BOUND, HSICEngine
+from .ops import _f32c
+from .padding import Padding, padding_for, run_engine
 
 
 def _stream() -> int:
@@ -236,11 +238,12 @@ def _stream_intervals(eng: HSICEngine, tag: str, y_hat_nchw: torch.Tensor, table
         SCALE_BOUND, y_nhwc.data_ptr(), None, 0, out.data_ptr(), _stream()), "masic_gmm_symbol_cdfs_pairs")
 
 
-def _encode_pairs(model, eng: HSICEngine, y_clock: Optional[list] = None):
+def _encode_pairs(model, eng: HSICEngine, pad: Padding, y_clock: Optional[list] = None):
     """Format-2 header and payload of every pair of the engine's last forward pass.  The intervals of all streams of
     both views are computed, put in wave order and range-coded on the device; only the packed payload bytes, the
     stream offsets and the flags are read back.  y_clock, if given, receives time.time() where the y coding starts.
-    y_bits_ideal is summed per stream on the device, then over the pair's streams (float64)."""
+    y_bits_ideal is summed per stream on the device, then over the pair's streams (float64).  The header holds the
+    pair's own size `pad.h`, `pad.w`; the latents are those of the padded frame the engine ran on."""
     lib, dev = eng.lib, eng.dev
     B, H, W, M = eng.B, eng.H, eng.W, eng.M
     n_pos = (H // 16) * (W // 16)
@@ -251,7 +254,8 @@ def _encode_pairs(model, eng: HSICEngine, y_clock: Optional[list] = None):
                        torch.stack([t.amax(dim=(1, 2, 3)).clamp_min(1.0) for t in a]).flatten()]).cpu().numpy()
     flags = small[:2 * B * M].reshape(2, B, M).astype(np.int64)
     minmax = small[2 * B * M:].reshape(2, B).astype(np.int64)
-    headers = [_header_bytes(H, W, [z_strings[0][b], z_strings[1][b]], minmax[:, b], flags[:, b]) for b in range(B)]
+    headers = [_header_bytes(pad.h, pad.w, [z_strings[0][b], z_strings[1][b]], minmax[:, b], flags[:, b])
+               for b in range(B)]
     tables = [_stream_table(flags[v], minmax[v]) for v in range(2)]
     S = [t.shape[1] for t in tables]
     n_streams = S[0] + S[1]
@@ -311,7 +315,7 @@ def _encode_pairs(model, eng: HSICEngine, y_clock: Optional[list] = None):
             ideal += float(bits_h[s0:s1].sum())
         payload = b"".join(parts)
         items.append({"header": headers[b], "payload": payload,
-                      "bpp_real": (len(headers[b]) + len(payload)) * 8 / (2 * H * W),
+                      "bpp_real": (len(headers[b]) + len(payload)) * 8 / (2 * pad.h * pad.w),
                       "n_symbols": n_sym, "y_bits_ideal": ideal})
     return items
 
@@ -333,10 +337,12 @@ def compress_batch(model, x1: torch.Tensor, x2: torch.Tensor, h_matrix: torch.Te
     what `compress` writes for that pair alone; `bpp_real`, `n_symbols`, `y_bits_ideal` as in `compress`."""
     _check_inputs(model, "HSIC.compress_batch", x1, x2, h_matrix)
     B, _, H, W = x1.shape
-    eng: HSICEngine = model.engine_for(B, H, W, x1.device)
+    pad = padding_for(H, W)
+    pad.check_header()
+    eng: HSICEngine = model.engine_for(B, pad.hp, pad.wp, x1.device)
     with torch.cuda.device(eng.dev):
-        eng.run(x1, x2, h_matrix)
-        return _encode_pairs(model, eng)
+        run_engine(eng, pad, x1, x2, h_matrix)
+        return _encode_pairs(model, eng, pad)
 
 
 def compress(model, x1: torch.Tensor, x2: torch.Tensor, h_matrix: torch.Tensor, output_name, output_path: str = "",
@@ -352,15 +358,17 @@ def compress(model, x1: torch.Tensor, x2: torch.Tensor, h_matrix: torch.Tensor, 
         raise ValueError(f'y_order must be one of {sorted(_ORDERS)}, got {y_order!r}')
     order = _ORDERS[y_order]
     lib = _lib.load()
-    _, _, H, W = x1.shape
+    pad = padding_for(*x1.shape[2:])
+    pad.check_header()
+    H, W = pad.hp, pad.wp                   # the coded latents are those of the padded frame
     eng: HSICEngine = model.engine_for(1, H, W, x1.device)
-    out = eng.run(x1, x2, h_matrix)
+    out = run_engine(eng, pad, x1, x2, h_matrix)
     output1 = os.path.join(output_path, str(output_name) + ".npz")
     output2 = os.path.join(output_path, str(output_name) + ".bin")
     if order == ORDER_WAVE_STREAMS:
         # one range-coded stream per (view, non-zero channel): | 2 | per view: u32 n_ch, u32 len[n_ch], streams |
         clock = []
-        item = _encode_pairs(model, eng, clock)[0]
+        item = _encode_pairs(model, eng, pad, clock)[0]
         with open(output1, "wb") as f:
             f.write(item["header"])
         with open(output2, "wb") as f:
@@ -374,7 +382,7 @@ def compress(model, x1: torch.Tensor, x2: torch.Tensor, h_matrix: torch.Tensor, 
         for tag in ("L", "R"):
             flags[tag], minmaxs[tag] = _nonzero_channels(y_hats[tag])
         with open(output1, "wb") as f:
-            f.write(_header_bytes(H, W, [zs[0] for zs in z_strings], [minmaxs["L"], minmaxs["R"]],
+            f.write(_header_bytes(pad.h, pad.w, [zs[0] for zs in z_strings], [minmaxs["L"], minmaxs["R"]],
                                   [flags["L"], flags["R"]]))
         # ---- y1, y2: all coding intervals in one kernel each, one range-coded stream
         start = time.time()
@@ -398,7 +406,7 @@ def compress(model, x1: torch.Tensor, x2: torch.Tensor, h_matrix: torch.Tensor, 
         end = time.time()
         n_symbols = int(iv.shape[0])
         ideal_bits = float(-(np.log2(iv[:, 1].astype(np.float64) / iv[:, 2])).sum()) if iv.shape[0] else 0.0
-    num_pixels = H * W * 2
+    num_pixels = pad.h * pad.w * 2
     size1, size2 = os.path.getsize(output1), os.path.getsize(output2)
     return {
         "bpp_real": (size1 + size2) * 8 / num_pixels, "bpp_side": size1 * 8 / num_pixels, "enctime": end - start,
@@ -596,6 +604,16 @@ def _parse_header(header: bytes, M: int):
     return H, W, views
 
 
+def _header_padding(H: int, W: int) -> Padding:
+    """The padded frame of a header's pair size; a size no encoder writes is a corrupt header."""
+    try:
+        pad = padding_for(H, W)
+        pad.check_header()
+    except ValueError as e:
+        raise MasicError(f"header: {e}") from None
+    return pad
+
+
 def _parse_payload(payload: bytes, hdr):
     """Format-2 `<name>.bin` -> per view (lens int64 (n_ch,), stream bytes), checked against the header's bitmaps."""
     if not payload or payload[0] != ORDER_WAVE_STREAMS:
@@ -619,12 +637,15 @@ def _parse_payload(payload: bytes, hdr):
     return views
 
 
-def _side_information(model, eng: HSICEngine, hdrs, h_matrix: torch.Tensor) -> None:
+def _side_information(model, eng: HSICEngine, pad: Padding, hdrs, h_matrix: torch.Tensor) -> None:
     """Homography products, mask weights and the hyper-synthesis parameters of every pair (MASIC.py:1190-1196,
-    :1310-1312) from the z strings of the headers."""
+    :1310-1312) from the z strings of the headers.  The homography is taken to the padded frame of `pad`."""
     o = eng.out
     z_shape = (eng.H // 64, eng.W // 64)
-    eng.Hm.copy_(h_matrix.reshape(eng.B, 3, 3).to(eng.dev))
+    if pad.aligned:
+        eng.Hm.copy_(h_matrix.reshape(eng.B, 3, 3).to(eng.dev))
+    else:
+        pad.homography_into(_f32c(h_matrix.reshape(eng.B, 3, 3).to(eng.dev)), eng.Hm)
     eng.run_steps(lambda n: n.startswith("warp.prepare") or n.startswith("mask_") or n.startswith("mask2weights"))
     for v, (tag, eb) in enumerate((("L", model.entropy_bottleneck1), ("R", model.entropy_bottleneck2))):
         # one string per call: the reference's EntropyBottleneck.decompress takes batch-1 medians
@@ -657,8 +678,10 @@ def _decode_pairs(eng: HSICEngine, hdrs, payloads) -> None:
         (_tail_left if tag == "L" else _tail_right)(eng)
 
 
-def _outputs(o) -> Dict:
-    return {k: o[k].clone() for k in ("x1_hat", "x2_hat", "y1_hat", "y2_hat", "z1_hat", "z2_hat")}
+def _outputs(o, pad: Padding) -> Dict:
+    """The decoded pair cropped to its own size, the latents on the padded grid (as HSIC.forward returns them)."""
+    return {k: (pad.crop(o[k]) if k in ("x1_hat", "x2_hat") else o[k]).clone()
+            for k in ("x1_hat", "x2_hat", "y1_hat", "y2_hat", "z1_hat", "z2_hat")}
 
 
 def decompress_batch(model, items, h_matrix: torch.Tensor, device=None) -> Dict:
@@ -686,11 +709,12 @@ def decompress_batch(model, items, h_matrix: torch.Tensor, device=None) -> Dict:
     dev = torch.device(device) if device is not None else h_matrix.device
     if dev.type != "cuda":
         raise MasicError("HSIC.decompress_batch needs a CUDA device: masic_b200 has no CPU fallback")
-    eng: HSICEngine = model.engine_for(B, H, W, dev)
+    pad = _header_padding(H, W)
+    eng: HSICEngine = model.engine_for(B, pad.hp, pad.wp, dev)
     with torch.cuda.device(eng.dev):
-        _side_information(model, eng, hdrs, h_matrix)
+        _side_information(model, eng, pad, hdrs, h_matrix)
         _decode_pairs(eng, hdrs, payloads)
-    return _outputs(eng.out)
+        return _outputs(eng.out, pad)
 
 
 def decompress(model, x1: Optional[torch.Tensor], x2: Optional[torch.Tensor], h_matrix: torch.Tensor, output_name,
@@ -707,10 +731,11 @@ def decompress(model, x1: Optional[torch.Tensor], x2: Optional[torch.Tensor], h_
     dev = h_matrix.device if device is None else torch.device(device)
     if dev.type != "cuda":
         dev = x1.device if x1 is not None else torch.device("cuda:0")
-    eng: HSICEngine = model.engine_for(1, H, W, dev)
+    pad = _header_padding(H, W)
+    eng: HSICEngine = model.engine_for(1, pad.hp, pad.wp, dev)
     o = eng.out
     with torch.cuda.device(eng.dev):
-        _side_information(model, eng, [hdr], h_matrix)
+        _side_information(model, eng, pad, [hdr], h_matrix)
         with open(output2, "rb") as f:
             raw = f.read()
         if not raw or raw[0] not in (ORDER_RASTER, ORDER_WAVE, ORDER_WAVE_STREAMS):
@@ -736,4 +761,5 @@ def decompress(model, x1: Optional[torch.Tensor], x2: Optional[torch.Tensor], h_
                 end = time.time()
             finally:
                 lib.masic_range_decoder_destroy(dec)
-    return {**_outputs(o), "dectime": end - start}
+        outputs = _outputs(o, pad)
+    return {**outputs, "dectime": end - start}

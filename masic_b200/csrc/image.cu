@@ -962,3 +962,66 @@ extern "C" int masic_u8_to_unit_f32(const uint8_t* in_u8, int64_t numel, float* 
   u8_to_unit_f32_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(in_u8, numel, out_f32);
   return (int)cudaGetLastError();
 }
+
+// ------------------------------------------------------------------ zero padding to the codec's 64-multiple frame
+namespace {
+
+constexpr int PAD_BLK = 256;
+
+// One thread per 4 consecutive output columns of one padded row (n, c, Hp, Wp): every output element is written exactly
+// once, the zero border included, so a padded buffer needs no memset and stays valid across pairs of one padded size.
+// Rows and columns inside the source window read (uint8: torchvision's ToTensor, x / 255 with the IEEE division, as
+// masic_u8_to_unit_f32) and optionally also write the unpadded float32 image from the same pass.
+template <bool U8, bool VEC>
+__global__ void __launch_bounds__(PAD_BLK)
+pad_image_kernel(const void* __restrict__ src, int h, int w, int hp, int wp, int top, int left, long n_rows,
+                 float* __restrict__ dst, float* __restrict__ dst_unpadded) {
+  __shared__ float lut[256];
+  if (U8) {
+    lut[threadIdx.x] = __fdiv_rn((float)threadIdx.x, 255.0f);
+    __syncthreads();
+  }
+  const int q_per_row = (wp + 3) / 4;
+  const long t = blockIdx.x * (long)PAD_BLK + threadIdx.x;
+  if (t >= n_rows * q_per_row) return;
+  const long row = t / q_per_row;                         // (image, channel, padded y)
+  const int x0 = (int)(t - row * q_per_row) * 4;
+  const long plane = row / hp;
+  const int sy = (int)(row - plane * hp) - top;
+  float v[4] = {0.f, 0.f, 0.f, 0.f};
+  if (sy >= 0 && sy < h) {
+    const long s_row = (plane * h + sy) * (long)w;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const int sx = x0 + i - left;
+      if (sx >= 0 && sx < w) {
+        v[i] = U8 ? lut[static_cast<const uint8_t*>(src)[s_row + sx]] : static_cast<const float*>(src)[s_row + sx];
+        if (dst_unpadded) dst_unpadded[s_row + sx] = v[i];
+      }
+    }
+  }
+  float* o = dst + row * wp + x0;
+  if (VEC) {
+    *reinterpret_cast<float4*>(o) = make_float4(v[0], v[1], v[2], v[3]);
+  } else {
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+      if (x0 + i < wp) o[i] = v[i];
+  }
+}
+
+}  // namespace
+
+extern "C" int masic_pad_image(const void* src, int src_u8, int n, int c, int h, int w, int hp, int wp, int top,
+                               int left, float* dst, float* dst_unpadded, void* stream) {
+  if (!src || !dst || n <= 0 || c <= 0 || h <= 0 || w <= 0 || top < 0 || left < 0 || hp < h + top || wp < w + left)
+    return MASIC_EINVAL;
+  const long n_rows = (long)n * c * hp;
+  const long threads = n_rows * ((wp + 3) / 4);
+  const bool vec = (wp & 3) == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0;
+  auto k = src_u8 ? (vec ? pad_image_kernel<true, true> : pad_image_kernel<true, false>)
+                  : (vec ? pad_image_kernel<false, true> : pad_image_kernel<false, false>);
+  k<<<(unsigned)((threads + PAD_BLK - 1) / PAD_BLK), PAD_BLK, 0, static_cast<cudaStream_t>(stream)>>>(
+      src, h, w, hp, wp, top, left, n_rows, dst, dst_unpadded);
+  return (int)cudaGetLastError();
+}

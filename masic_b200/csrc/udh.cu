@@ -196,3 +196,37 @@ extern "C" int masic_homography_from_delta(const float* corners, const float* de
       corners, delta, batch, shift_corners, (float)a, (float)(1.0 / a), (float)b, (float)(1.0 / b), h_out);
   return (int)cudaGetLastError();
 }
+
+// ------------------------------------------------------------------ homographies in the zero-padded frame
+namespace {
+
+// T . H . T^-1 with T the translation by (left, top), in fp64 with the products and sums rounded one at a time in a
+// fixed order (no contraction), rounded once to fp32: the same bits as the float64 expression written out on the host.
+__global__ void homography_pad_kernel(const float* __restrict__ h_in, int n, double top, double left,
+                                      float* __restrict__ h_out) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= n) return;
+  double m[9];
+#pragma unroll
+  for (int i = 0; i < 9; ++i) m[i] = (double)h_in[9 * b + i];
+  double c[3];                                            // column 2 of H . T^-1
+#pragma unroll
+  for (int r = 0; r < 3; ++r) c[r] = __dsub_rn(__dsub_rn(m[3 * r + 2], __dmul_rn(left, m[3 * r])), __dmul_rn(top, m[3 * r + 1]));
+  const float o[9] = {
+      (float)__dadd_rn(m[0], __dmul_rn(left, m[6])), (float)__dadd_rn(m[1], __dmul_rn(left, m[7])),
+      (float)__dadd_rn(c[0], __dmul_rn(left, c[2])),
+      (float)__dadd_rn(m[3], __dmul_rn(top, m[6])), (float)__dadd_rn(m[4], __dmul_rn(top, m[7])),
+      (float)__dadd_rn(c[1], __dmul_rn(top, c[2])),
+      (float)m[6], (float)m[7], (float)c[2]};
+#pragma unroll
+  for (int i = 0; i < 9; ++i) h_out[9 * b + i] = o[i];
+}
+
+}  // namespace
+
+extern "C" int masic_homography_pad(const float* h_in, int n, int top, int left, float* h_out, void* stream) {
+  if (!h_in || !h_out || n <= 0) return MASIC_EINVAL;
+  homography_pad_kernel<<<(n + 63) / 64, 64, 0, static_cast<cudaStream_t>(stream)>>>(h_in, n, (double)top,
+                                                                                       (double)left, h_out);
+  return (int)cudaGetLastError();
+}

@@ -24,6 +24,7 @@ from ._lib import MasicError
 from .engine import HSICEngine
 from .entropy_models import EntropyBottleneck, GaussianMixtureConditional_gf
 from .layers import GDN, MaskedConv2d, conv, deconv
+from .padding import padding_for, run_engine
 
 
 class _Block(nn.Module):
@@ -123,6 +124,7 @@ class HSIC(nn.Module):
         self._use_graph = use_cuda_graph
         self._engines: Dict[Tuple, HSICEngine] = {}
         self._engine_version = 0
+        self._staging_key, self._staging = None, {}
 
     # ---- CompressionModel surface (MASIC.py:59-109)
     def aux_loss(self):
@@ -186,6 +188,9 @@ class HSIC(nn.Module):
 
     # ---- forward (MASIC.py:744-851)
     def forward(self, x1: torch.Tensor, x2: torch.Tensor, h_matrix: torch.Tensor, clone: bool = True):
+        """MASIC.py:744-851 at any H, W: a pair whose size is not a multiple of 64 runs zero-padded on the device, as
+        CompressAI evaluates it (masic_b200/padding.py); x1_hat, x2_hat and the masks are cropped back to (H, W), the
+        latents and likelihoods stay on the padded grid."""
         if self.training:
             raise MasicError("HSIC.forward in train() mode does not build an autograd graph: the training step "
                              "(noise quantisation, loss, backward, aux loss) runs as fused CUDA kernels through "
@@ -193,15 +198,31 @@ class HSIC(nn.Module):
         if not x1.is_cuda:
             raise MasicError("HSIC.forward needs CUDA tensors: masic_b200 has no CPU fallback")
         b, _, h, w = x1.shape
-        eng = self.engine_for(b, h, w, x1.device)
-        o = eng.run(x1, x2, h_matrix)
+        pad = padding_for(h, w)
+        eng = self.engine_for(b, pad.hp, pad.wp, x1.device)
+        o = run_engine(eng, pad, x1, x2, h_matrix)
         c = (lambda t: t.clone()) if clone else (lambda t: t)
+        if not pad.aligned:         # the images cropped back to (h, w); latents and likelihoods stay on the padded grid
+            o = {**o, **self._crop(eng, pad, o)}
         return {
             "x1_hat": c(o["x1_hat"]), "x2_hat": c(o["x2_hat"]),
             "y1_hat": c(o["y1_hat"]), "z1_hat": c(o["z1_hat"]),
             "x1_mask_R": c(o["x1_mask_R"]), "x1_mask_L": c(o["x1_mask_L"]),
             "likelihoods": {"y1": c(o["lik_y1"]), "y2": c(o["lik_y2"]), "z1": c(o["lik_z1"]), "z2": c(o["lik_z2"])},
         }
+
+    _CROPPED = ("x1_hat", "x2_hat", "x1_mask_R", "x1_mask_L")
+
+    def _crop(self, eng: HSICEngine, pad, o) -> Dict[str, torch.Tensor]:
+        """The padded engine's images cropped to the pair's size, into staging buffers cached per (batch, h, w)."""
+        key = (eng.B, pad.h, pad.w, str(eng.dev))
+        if self._staging_key != key:
+            self._staging_key = key
+            self._staging = {k: torch.empty(eng.B, o[k].shape[1], pad.h, pad.w, device=eng.dev) for k in self._CROPPED}
+        with torch.cuda.device(eng.dev):
+            for k in self._CROPPED:
+                pad.crop_into(o[k], self._staging[k])
+        return self._staging
 
     # ---- the same forward, layer by layer (what the unmodified MASIC.py does on masic_b200/compat)
     @torch.no_grad()
@@ -324,6 +345,8 @@ class PairStream:
     enhanced pair; a second masic_rd_metrics pass adds the codec's own MSE to the same read-back.
     `outputs()` exposes the engine's output tensors of the LAST submitted pair (valid after `result(ticket)`),
     `enhanced_outputs()` the enhanced pair of the last one submitted with enhance=True.
+    H and W need not be multiples of 64: each pair is then zero-padded on the device into an engine of the padded size
+    and its reconstructions cropped back (masic_b200/padding.py); every number and image refers to the H x W pair.
     """
 
     def __init__(self, model: "HSIC", height: int, width: int, device, depth: int = 2, lmbda: float = 0.0):
@@ -335,13 +358,17 @@ class PairStream:
             raise MasicError("PairStream needs a CUDA device: masic_b200 has no CPU fallback")
         self.model, self.H, self.W, self.lmbda = model, height, width, float(lmbda)
         self.depth = depth
+        self.pad = pad = padding_for(height, width)
         # One engine (static buffers + CUDA graph) per slot, each replayed on its own stream: the H2D copy lands
         # directly in the engine's input buffers (no staging copy), and the kernels of consecutive pairs overlap —
         # the tail of a pair is a chain of launches that leave SMs idle (conv4: 85 tiles, hyper-prior layers: 10-40),
         # which the next pair's kernels fill (+3.6 % pairs/s on a B200 with two engines).
         # (private engines: model.forward() keeps its own cached one, so the two can be used side by side)
-        first = model.engine_for(1, height, width, self.dev)          # also applies MaskedConv2d's weight masking
-        self.engines = [HSICEngine(model.state_dict(), 1, height, width, self.dev, model.N, model.M, model.K,
+        # A pair whose size is not a multiple of 64 runs an engine of the padded size (masic_b200/padding.py): the slot
+        # then holds the pair at its own size around it (x1, x2, h as submitted, the cropped x1_hat, x2_hat), and
+        # everything after the codec reads those; at a multiple of 64 they are the engine's own buffers.
+        first = model.engine_for(1, pad.hp, pad.wp, self.dev)          # also applies MaskedConv2d's weight masking
+        self.engines = [HSICEngine(model.state_dict(), 1, pad.hp, pad.wp, self.dev, model.N, model.M, model.K,
                                    use_graph=first.use_graph) for _ in range(depth)]
         self.eng = self.engines[0]
         with torch.cuda.device(self.dev):
@@ -350,8 +377,14 @@ class PairStream:
             for eng in self.engines:
                 o = eng.out
                 liks = [o["lik_y1"], o["lik_y2"], o["lik_z1"], o["lik_z2"]]
+                if pad.aligned:
+                    own = dict(x1=eng.x1, x2=eng.x2, h=eng.Hm, rec={"x1_hat": o["x1_hat"], "x2_hat": o["x2_hat"]})
+                else:
+                    img = lambda: torch.empty(1, 3, height, width, device=self.dev)   # noqa: E731
+                    own = dict(x1=img(), x2=img(), h=torch.eye(3, device=self.dev).reshape(1, 3, 3),
+                               rec={"x1_hat": img(), "x2_hat": img()})
                 self.slots.append(dict(
-                    eng=eng, stream=torch.cuda.Stream(device=self.dev),
+                    eng=eng, stream=torch.cuda.Stream(device=self.dev), **own,
                     # criterion (8 floats) | MS-SSIM per channel of view 1 (3) and view 2 (3) | LPIPS of view 1, 2 |
                     # with enhance=True, masic_rd_metrics of the codec's (unenhanced) pair (8)
                     res_d=torch.zeros(24, device=self.dev), res_h=torch.zeros(24).pin_memory(),
@@ -400,6 +433,7 @@ class PairStream:
         caller = torch.cuda.current_stream(self.dev)
         self.copy_stream.wait_stream(caller)        # inputs produced on the caller's stream are complete
         as_u8 = x1.dtype == torch.uint8
+        pad = self.pad
         if as_u8 and "u8" not in s:                 # 8-bit images: a quarter of the PCIe bytes, converted on the device
             s["u8"] = [torch.empty(1, 3, self.H, self.W, dtype=torch.uint8, device=self.dev) for _ in range(2)]
         with torch.cuda.stream(self.copy_stream):
@@ -407,30 +441,39 @@ class PairStream:
                 s["u8"][0].copy_(x1.reshape(1, 3, self.H, self.W), non_blocking=True)
                 s["u8"][1].copy_(x2.reshape(1, 3, self.H, self.W), non_blocking=True)
             else:
-                eng.x1.copy_(x1.reshape(1, 3, self.H, self.W), non_blocking=True)
-                eng.x2.copy_(x2.reshape(1, 3, self.H, self.W), non_blocking=True)
-            eng.Hm.copy_(h.reshape(1, 3, 3), non_blocking=True)
+                s["x1"].copy_(x1.reshape(1, 3, self.H, self.W), non_blocking=True)
+                s["x2"].copy_(x2.reshape(1, 3, self.H, self.W), non_blocking=True)
+            s["h"].copy_(h.reshape(1, 3, 3), non_blocking=True)
             s["copied"].record(self.copy_stream)
         with torch.cuda.stream(st):
             st.wait_event(s["copied"])
-            if as_u8:                               # torchvision's ToTensor: img.float().div(255), bit for bit
+            if not pad.aligned:                     # into the padded frame; 8-bit pairs also leave the fp32 originals
+                for i, (x, dst) in enumerate(((s["x1"], eng.x1), (s["x2"], eng.x2))):
+                    pad.image_into(s["u8"][i] if as_u8 else x, dst, unpadded=x if as_u8 else None)
+                pad.homography_into(s["h"], eng.Hm)
+            elif as_u8:                             # torchvision's ToTensor: img.float().div(255), bit for bit
                 for src, dst in ((s["u8"][0], eng.x1), (s["u8"][1], eng.x2)):
                     check(self.lib.masic_u8_to_unit_f32(src.data_ptr(), src.numel(), dst.data_ptr(), st.cuda_stream),
                           "masic_u8_to_unit_f32")
             o = eng.run()
-            rec = s["cqe"].run() if enhance else o      # the CQE graph reads o["x1_hat"], o["x2_hat"], eng.Hm in place
+            if not pad.aligned:
+                for k in ("x1_hat", "x2_hat"):
+                    pad.crop_into(o[k], s["rec"][k])
+            codec = s["rec"]
+            rec = s["cqe"].run() if enhance else codec  # the CQE graph reads the codec's x1_hat, x2_hat and h in place
+            x1_, x2_ = s["x1"], s["x2"]
             if criterion:
-                check(self.lib.masic_rd_metrics(s["lik_p"], s["lik_n"], rec["x1_hat"].data_ptr(), eng.x1.data_ptr(),
-                                                rec["x2_hat"].data_ptr(), eng.x2.data_ptr(), 1, 3, self.H, self.W,
+                check(self.lib.masic_rd_metrics(s["lik_p"], s["lik_n"], rec["x1_hat"].data_ptr(), x1_.data_ptr(),
+                                                rec["x2_hat"].data_ptr(), x2_.data_ptr(), 1, 3, self.H, self.W,
                                                 self.lmbda, s["scratch"].data_ptr(), s["res_d"].data_ptr(),
                                                 st.cuda_stream), "masic_rd_metrics")
                 if enhance:                             # the codec's own MSE (no likelihoods: its bpp is the above)
-                    check(self.lib.masic_rd_metrics(self._no_lik_p, self._no_lik_n, o["x1_hat"].data_ptr(),
-                                                    eng.x1.data_ptr(), o["x2_hat"].data_ptr(), eng.x2.data_ptr(), 1, 3,
+                    check(self.lib.masic_rd_metrics(self._no_lik_p, self._no_lik_n, codec["x1_hat"].data_ptr(),
+                                                    x1_.data_ptr(), codec["x2_hat"].data_ptr(), x2_.data_ptr(), 1, 3,
                                                     self.H, self.W, self.lmbda, s["scratch"].data_ptr(),
                                                     s["res_d"][16:].data_ptr(), st.cuda_stream), "masic_rd_metrics")
                 if msssim:
-                    for v, (xh, x) in enumerate(((rec["x1_hat"], eng.x1), (rec["x2_hat"], eng.x2))):
+                    for v, (xh, x) in enumerate(((rec["x1_hat"], x1_), (rec["x2_hat"], x2_))):
                         check(self.lib.masic_ms_ssim(xh.data_ptr(), x.data_ptr(), 1, 3, self.H, self.W, 5, 1.0, 0.01,
                                                      0.03, self._ms_weights, 1, s["ms_scratch"].data_ptr(),
                                                      s["res_d"][8 + 3 * v:].data_ptr(), st.cuda_stream), "masic_ms_ssim")
@@ -471,16 +514,15 @@ class PairStream:
         for s in self.slots:
             if s["busy"]:
                 s["done"].synchronize()             # the engines replaced below may still be in use
-            s["lpips"] = self._lpips_engine(s, s["eng"].out)
+            s["lpips"] = self._lpips_engine(s, s["rec"])
             if "cqe" in s:
                 s["lpips_enh"] = self._lpips_engine(s, s["cqe"].out)
 
     def _lpips_engine(self, s, rec: Dict[str, torch.Tensor]):
         """An LPIPSEngine that compares the reconstructions `rec` with the slot's originals, reading both in place."""
         from .lpips import LPIPSEngine
-        eng = s["eng"]
         e = LPIPSEngine(self._lpips_sd, 2, self.H, self.W, self.dev,
-                        inputs=[rec["x1_hat"], rec["x2_hat"], eng.x1, eng.x2])
+                        inputs=[rec["x1_hat"], rec["x2_hat"], s["x1"], s["x2"]])
         e.prepare(self._lpips_normalize)
         return e
 
@@ -494,9 +536,8 @@ class PairStream:
         for s in self.slots:
             if s["busy"]:
                 s["done"].synchronize()             # the engines replaced below may still be in use
-            eng = s["eng"]
             s["cqe"] = CQEEngine(sd, 1, self.H, self.W, self.dev, use_graph=en._use_graph,
-                                 inputs=(eng.out["x1_hat"], eng.out["x2_hat"], eng.Hm))
+                                 inputs=(s["rec"]["x1_hat"], s["rec"]["x2_hat"], s["h"]))
             if "lpips" in s:
                 s["lpips_enh"] = self._lpips_engine(s, s["cqe"].out)
 
@@ -570,7 +611,14 @@ class PairStream:
         return s["rec_h"][0], s["rec_h"][1]
 
     def outputs(self) -> Dict[str, torch.Tensor]:
-        return self.eng.out
+        """The engine's output buffers of the last submitted pair.  For a size that is not a multiple of 64, x1_hat and
+        x2_hat are the slot's cropped copies and the masks are views of the pair's window; the latents and likelihoods
+        stay on the padded grid, as `HSIC.forward` returns them."""
+        if self.pad.aligned:
+            return self.eng.out
+        s = next(s for s in self.slots if s["eng"] is self.eng)
+        o = self.eng.out
+        return {**o, **s["rec"], "x1_mask_R": self.pad.crop(o["x1_mask_R"]), "x1_mask_L": self.pad.crop(o["x1_mask_L"])}
 
     def enhanced_outputs(self) -> Dict[str, torch.Tensor]:
         """{"x1_hat", "x2_hat"} of the last submitted pair after the enhancement network, the keys of

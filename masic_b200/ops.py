@@ -316,6 +316,21 @@ def cqe_residual_image_into(conv_out: torch.Tensor, identity: torch.Tensor, out:
             _arg(out, _F32, (n, 3, h, w)))
 
 
+def pad_image_into(src: torch.Tensor, dst: torch.Tensor, top: int, left: int, unpadded=None) -> None:
+    """src (n,c,h,w) uint8 (ToTensor's x / 255) or fp32 -> dst (n,c,hp,wp) fp32 zero-padded, src at (top, left), every
+    element of dst written; unpadded (n,c,h,w) fp32, if given, receives the converted src from the same pass."""
+    n, c, h, w = src.shape
+    hp, wp = dst.shape[2:]
+    _launch("masic_pad_image", _arg(src, (torch.uint8, torch.float32)), int(src.dtype == torch.uint8), n, c, h, w, hp,
+            wp, top, left, _arg(dst, _F32, (n, c, hp, wp)), _arg(unpadded, _F32, (n, c, h, w)))
+
+
+def homography_pad_into(h: torch.Tensor, out: torch.Tensor, top: int, left: int) -> None:
+    """out (n,3,3) fp32 <- T h T^-1 for the (n,3,3) fp32 homographies h, T the translation by (left, top)."""
+    n = h.shape[0]
+    _launch("masic_homography_pad", _arg(h, _F32, (n, 3, 3)), n, top, left, _arg(out, _F32, (n, 3, 3)))
+
+
 def rd_metrics_scratch(device) -> torch.Tensor:
     """The device scratch rd_metrics_into needs (allocate it once, outside graph capture)."""
     return torch.empty(_lib.load().masic_rd_metrics_scratch_bytes() // 8, dtype=torch.float64, device=device)
