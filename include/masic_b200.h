@@ -530,6 +530,20 @@ int masic_rd_metrics(const float* const* lik4_host, const int64_t* lik_numel4_ho
 int64_t masic_ms_ssim_scratch_bytes(int n, int c, int h, int w, int levels);
 int masic_ms_ssim(const float* x, const float* y, int n, int c, int h, int w, int levels, float data_range, float k1,
                   float k2, const float* weights_host, int nonneg_last, void* scratch, float* out_nc, void* stream);
+/* Gradient of masic_ms_ssim with respect to its first argument: dx (device, NCHW fp32 like x) =
+ * grad_scale * d(sum over the n*c planes of out_nc)/dx [+ addend].  addend (device, or NULL) may be dx itself.
+ * fwd_scratch must hold the scratch of a masic_ms_ssim call with the same x, y, sizes and constants, issued earlier on
+ * the same stream (or completed before this call) and not overwritten since: the backward reads that call's pyramid
+ * levels 1..levels-1 and re-adds its per-tile partial sums in the final launch's order, so the level means it
+ * differentiates are the ones behind the forward's value.  A level whose relu'd mean clamps to 0 contributes 0 and, as
+ * in torch's prod backward, zeroes the gradient of every other level.  work is masic_ms_ssim_bwd_work_bytes() of device
+ * memory (per-level coefficient maps and gradients).  2 + levels launches; deterministic (no atomics) and batch
+ * invariant.  MASIC_EINVAL for the sizes masic_ms_ssim rejects and for a NULL x, y, weights_host, fwd_scratch, dx or
+ * work. */
+int64_t masic_ms_ssim_bwd_work_bytes(int n, int c, int h, int w, int levels);
+int masic_ms_ssim_bwd(const float* x, const float* y, int n, int c, int h, int w, int levels, float data_range,
+                      float k1, float k2, const float* weights_host, int nonneg_last, const void* fwd_scratch,
+                      float grad_scale, const float* addend, float* dx, void* work, void* stream);
 /* lpips.LPIPS(net='alex') (lpips 0.1, version '0.1'), as the reference's eval loop reports it next to bpp, PSNR and
  * MS-SSIM (coremasic/mywork/test2_real.py:88-114; test3_real.py).  The five AlexNet convolutions run as conv_tc plans;
  * these four entry points are the rest.  All activations are fp16 NHWC; a batch holds 2n images and image i is

@@ -214,6 +214,8 @@ def _declare(lib: C.CDLL) -> None:
         "masic_rd_metrics": (i, [C.POINTER(vp), C.POINTER(i64), vp, vp, vp, vp, i, i, i, i, f, vp, vp, vp]),
         "masic_ms_ssim_scratch_bytes": (i64, [i, i, i, i, i]),
         "masic_ms_ssim": (i, [vp, vp, i, i, i, i, i, f, f, f, C.POINTER(f), i, vp, vp, vp]),
+        "masic_ms_ssim_bwd_work_bytes": (i64, [i, i, i, i, i]),
+        "masic_ms_ssim_bwd": (i, [vp, vp, i, i, i, i, i, f, f, f, C.POINTER(f), i, vp, f, vp, vp, vp, vp]),
         "masic_lpips_prep": (i, [vp, i, i, i, i, C.POINTER(f), C.POINTER(f), vp, vp]),
         "masic_maxpool3s2_nhwc": (i, [vp, i, i, i, i, i, i, i, i, vp, vp]),
         "masic_lpips_distance_scratch_bytes": (i64, [i, i, i]),

@@ -291,6 +291,341 @@ bool plan(int n, int c, int h, int w, int levels, Args* a, size_t* bytes) {
   return true;
 }
 
+// Window, constants and level weights of a call (the pyramid pointers are set by the caller).
+void set_constants(Args* a, int levels, float data_range, float k1, float k2, const float* weights_host,
+                   int nonneg_last) {
+  // the window of pytorch_msssim's _fspecial_gauss_1d(11, 1.5), in float32 as the package computes it
+  float g[WIN], gs = 0.f;
+  for (int i = 0; i < WIN; ++i) {
+    const float d = (float)(i - WIN / 2);
+    g[i] = expf(-(d * d) / (2.f * 1.5f * 1.5f));
+    gs += g[i];
+  }
+  for (int i = 0; i < WIN; ++i) a->taps[i] = g[i] / gs;
+  a->shift = 0.5f * data_range;
+  a->c1 = (k1 * data_range) * (k1 * data_range);
+  a->c2 = (k2 * data_range) * (k2 * data_range);
+  for (int l = 0; l < MAX_LEVELS; ++l) a->weights[l] = l < levels ? (double)weights_host[l] : 0.0;
+  a->nonneg_last = nonneg_last ? 1 : 0;
+}
+
+// ------------------------------------------------------------------------------------------------- backward
+// d(sum over planes of MS-SSIM)/dx.  With m_l the mean of level l's map (cs, the last level's ssim) and
+// V = prod_l relu(m_l)^w_l, dV/dm_l = w_l m_l^(w_l - 1) prod_{k != l} relu(m_k)^w_k, and 0 where relu clamps m_l (as
+// torch's relu / prod backward give: a zero factor zeroes every level).  Per level, the map at p depends on x through
+// mu_x = G(x), E[x^2] = G(x^2) and E[xy] = G(xy) at p, so
+//   dm_l/dx(q) = (1 / cnt) (G^T a + 2 x G^T b + y G^T c)(q),   a, b, c = d map / d(mu_x, E[x^2], E[xy]) per pixel,
+// with x, y shifted by data_range/2 like the forward (the shift is a constant: the gradient is the same).  Levels are
+// joined through the transpose of the pooling: each fine pixel takes 1/4 of the one coarse cell whose window holds it.
+//
+// Launches: one coefficient launch (per plane and level: grad_scale dV/dm_l / cnt_l, from the forward's tile partials),
+// one map launch over every level (the statistics grid, writing a, b, c), then one gather launch per level, coarsest
+// first.  Every output element is a fixed-order gather of its plane's data: deterministic and batch invariant.
+
+struct Bwd {
+  float* map[MAX_LEVELS];     // level l: a, b, c, each planes x (h - 10) x (w - 10), mstride floats apart
+  long mstride[MAX_LEVELS];
+  float* grad[MAX_LEVELS];    // level l's gradient, planes x h x w (level 0: dx)
+  const float* coef;          // [plane][MAX_LEVELS]: grad_scale * dV/dm_l / cnt_l
+};
+
+constexpr size_t GA_SMEM = sizeof(float) * (3 * PR * PC + 3 * PR * TW);
+
+// One block per plane: the level sums in msssim_final_kernel's order, then the per-level coefficients in fp64.
+__global__ void msssim_bwd_coef_kernel(const Args a, const double* __restrict__ partial, float grad_scale,
+                                       float* __restrict__ coef) {
+  __shared__ double tot[MAX_LEVELS * 2];
+  const int p = blockIdx.x, wp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (wp < 2 * a.levels) {
+    const Level& L = a.lv[wp >> 1];
+    const double* src = partial + 2 * ((long)L.block0 + (long)p * L.tiles) + (wp & 1);
+    double s = 0.0;
+    for (int t = lane; t < L.tiles; t += 32) s += src[2 * t];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) tot[wp] = s;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double m[MAX_LEVELS], f[MAX_LEVELS], cnt[MAX_LEVELS];
+    bool clamps[MAX_LEVELS];
+    for (int l = 0; l < a.levels; ++l) {
+      cnt[l] = (double)(a.lv[l].h - (WIN - 1)) * (double)(a.lv[l].w - (WIN - 1));
+      const bool last = l == a.levels - 1;
+      m[l] = tot[2 * l + (last ? 1 : 0)] / cnt[l];
+      clamps[l] = (!last || a.nonneg_last) && !(m[l] > 0.0);
+      f[l] = pow(clamps[l] ? 0.0 : m[l], a.weights[l]);
+    }
+    for (int l = 0; l < MAX_LEVELS; ++l) {
+      double d = 0.0;
+      if (l < a.levels && !clamps[l]) {
+        d = a.weights[l] * pow(m[l], a.weights[l] - 1.0);
+        for (int k = 0; k < a.levels; ++k)
+          if (k != l) d *= f[k];
+        d = (double)grad_scale * d / cnt[l];
+      }
+      coef[p * MAX_LEVELS + l] = (float)d;
+    }
+  }
+}
+
+// The statistics grid again (the same loads and filter passes as msssim_stats_kernel, so the same filtered values);
+// per output pixel it writes d map / d(mu_x, E[x^2], E[xy]) instead of summing the map.
+__global__ void __launch_bounds__(ST_THREADS, 3) msssim_bwd_maps_kernel(const Args a, const Bwd bw) {
+  extern __shared__ float4 smem4[];
+  float* px = reinterpret_cast<float*>(smem4);   // [PR][PC]  x - shift
+  float* py = px + PR * PC;                      // [PR][PC]  y - shift
+  float* hq = py + PR * PC;                      // [5][PR][TW]  horizontal pass of x, y, x^2, y^2, xy
+
+  const int b = blockIdx.x;
+  int l = 0;
+#pragma unroll
+  for (int i = 1; i < MAX_LEVELS; ++i)
+    if (i < a.levels && b >= a.lv[i].block0) l = i;
+  const Level& L = a.lv[l];
+  const int rel = b - L.block0;
+  const int plane = rel / L.tiles, tile = rel - plane * L.tiles;
+  const int oy = (tile / L.tiles_x) * TH, ox = (tile % L.tiles_x) * TW;
+  const long poff = (long)plane * L.h * L.w;
+  const float* __restrict__ xs = L.x + poff;
+  const float* __restrict__ ys = L.y + poff;
+
+  constexpr int LOADS = (PR * PC + ST_THREADS - 1) / ST_THREADS;
+  float lx[LOADS], ly[LOADS];
+#pragma unroll
+  for (int k = 0; k < LOADS; ++k) {
+    const int i = threadIdx.x + k * ST_THREADS;
+    const int r = i / PC, c = i - r * PC;
+    const int gy = oy + r, gx = ox + c;
+    lx[k] = ly[k] = a.shift;
+    if (i < PR * PC && gy < L.h && gx < L.w) {
+      lx[k] = __ldg(xs + (long)gy * L.w + gx);
+      ly[k] = __ldg(ys + (long)gy * L.w + gx);
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < LOADS; ++k) {
+    const int i = threadIdx.x + k * ST_THREADS;
+    if (i < PR * PC) {
+      px[i] = lx[k] - a.shift;
+      py[i] = ly[k] - a.shift;
+    }
+  }
+  __syncthreads();
+
+  for (int it = threadIdx.x; it < PR * (TW / HSEG); it += ST_THREADS) {
+    const int r = it / (TW / HSEG), c0 = (it % (TW / HSEG)) * HSEG;
+    const float4* rx = reinterpret_cast<const float4*>(px + r * PC + c0);
+    const float4* ry = reinterpret_cast<const float4*>(py + r * PC + c0);
+    float vx[16], vy[16];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const float4 u = rx[q], v = ry[q];
+      vx[4 * q] = u.x; vx[4 * q + 1] = u.y; vx[4 * q + 2] = u.z; vx[4 * q + 3] = u.w;
+      vy[4 * q] = v.x; vy[4 * q + 1] = v.y; vy[4 * q + 2] = v.z; vy[4 * q + 3] = v.w;
+    }
+    float s[5][HSEG];
+#pragma unroll
+    for (int j = 0; j < HSEG; ++j) s[0][j] = s[1][j] = s[2][j] = s[3][j] = s[4][j] = 0.f;
+#pragma unroll
+    for (int k = 0; k < HSEG + WIN - 1; ++k) {
+      const float xx = vx[k] * vx[k], yy = vy[k] * vy[k], xy = vx[k] * vy[k];
+#pragma unroll
+      for (int j = 0; j < HSEG; ++j) {
+        const int t = k - j;
+        if (t >= 0 && t < WIN) {
+          const float g = a.taps[t];
+          s[0][j] = fmaf(g, vx[k], s[0][j]);
+          s[1][j] = fmaf(g, vy[k], s[1][j]);
+          s[2][j] = fmaf(g, xx, s[2][j]);
+          s[3][j] = fmaf(g, yy, s[3][j]);
+          s[4][j] = fmaf(g, xy, s[4][j]);
+        }
+      }
+    }
+#pragma unroll
+    for (int q = 0; q < 5; ++q)
+      *reinterpret_cast<float4*>(hq + (q * PR + r) * TW + c0) = make_float4(s[q][0], s[q][1], s[q][2], s[q][3]);
+  }
+  __syncthreads();
+
+  const int col = threadIdx.x % TW, r0 = (threadIdx.x / TW) * VSEG;
+  float m[5][VSEG];
+#pragma unroll
+  for (int j = 0; j < VSEG; ++j) m[0][j] = m[1][j] = m[2][j] = m[3][j] = m[4][j] = 0.f;
+#pragma unroll
+  for (int k = 0; k < VSEG + WIN - 1; ++k) {
+    float v[5];
+#pragma unroll
+    for (int q = 0; q < 5; ++q) v[q] = hq[(q * PR + r0 + k) * TW + col];
+#pragma unroll
+    for (int j = 0; j < VSEG; ++j) {
+      const int t = k - j;
+      if (t >= 0 && t < WIN) {
+        const float g = a.taps[t];
+#pragma unroll
+        for (int q = 0; q < 5; ++q) m[q][j] = fmaf(g, v[q], m[q][j]);
+      }
+    }
+  }
+  const int ho = L.h - (WIN - 1), wo = L.w - (WIN - 1);
+  if (ox + col >= wo) return;
+  const bool last = l == a.levels - 1;
+  float* __restrict__ ma = bw.map[l] + (long)plane * ho * wo + ox + col;
+  const long ms = bw.mstride[l];
+#pragma unroll
+  for (int j = 0; j < VSEG; ++j) {
+    const int row = oy + r0 + j;
+    if (row < ho) {
+      const float mx = m[0][j], my = m[1][j];
+      const float vxx = m[2][j] - mx * mx, vyy = m[3][j] - my * my, vxy = m[4][j] - mx * my;
+      const float csn = 2.f * vxy + a.c2, csd = 1.f / (vxx + vyy + a.c2);
+      const float cs = csn * csd;
+      float db = -cs * csd;                               // d cs / d var_x    (= d cs / d E[x^2])
+      float dc = 2.f * csd;                               // d cs / d cov_xy   (= d cs / d E[xy])
+      float da = -2.f * mx * db - my * dc;                // d cs / d mu_x through var_x and cov_xy
+      if (last) {                                         // ssim = lum * cs
+        const float ux = mx + a.shift, uy = my + a.shift;
+        const float ln = 2.f * ux * uy + a.c1, ld = 1.f / (ux * ux + uy * uy + a.c1);
+        const float lum = ln * ld;
+        const float dlum = 2.f * (uy - lum * ux) * ld;    // d lum / d mu_x
+        da = lum * da + cs * dlum;
+        db *= lum;
+        dc *= lum;
+      }
+      float* o = ma + (long)row * wo;
+      o[0] = da;
+      o[ms] = db;
+      o[2 * ms] = dc;
+    }
+  }
+}
+
+// Level l's gradient over TW x TH output pixels of one plane: G^T of the three coefficient maps (zero outside the
+// valid maps), combined with x and y, scaled by the level's coefficient, plus 1/4 of the coarser level's gradient at the
+// pooling cell that holds the pixel; level 0 adds `addend` (which may be dx itself).
+__global__ void __launch_bounds__(ST_THREADS, 3) msssim_bwd_gather_kernel(const Args a, const Bwd bw, int l,
+                                                                          const float* addend) {
+  extern __shared__ float4 smem4[];
+  float* pm = reinterpret_cast<float*>(smem4);   // [3][PR][PC]  maps, rows oy - 10 .., columns ox - 10 ..
+  float* hq = pm + 3 * PR * PC;                  // [3][PR][TW]  horizontal pass
+
+  const Level& L = a.lv[l];
+  const int tiles_x = (L.w + TW - 1) / TW, tiles = tiles_x * ((L.h + TH - 1) / TH);
+  const int plane = blockIdx.x / tiles, tile = blockIdx.x - plane * tiles;
+  const int oy = (tile / tiles_x) * TH, ox = (tile % tiles_x) * TW;
+  const int ho = L.h - (WIN - 1), wo = L.w - (WIN - 1);
+  const long ms = bw.mstride[l];
+  const float* __restrict__ src = bw.map[l] + (long)plane * ho * wo;
+
+  constexpr int LOADS = (PR * PC + ST_THREADS - 1) / ST_THREADS;
+  float lv[3][LOADS];
+#pragma unroll
+  for (int k = 0; k < LOADS; ++k) {
+    const int i = threadIdx.x + k * ST_THREADS;
+    const int r = i / PC, c = i - r * PC;
+    const int gy = oy - (WIN - 1) + r, gx = ox - (WIN - 1) + c;
+    lv[0][k] = lv[1][k] = lv[2][k] = 0.f;
+    if (i < PR * PC && gy >= 0 && gy < ho && gx >= 0 && gx < wo) {
+      const float* p = src + (long)gy * wo + gx;
+      lv[0][k] = __ldg(p);
+      lv[1][k] = __ldg(p + ms);
+      lv[2][k] = __ldg(p + 2 * ms);
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < LOADS; ++k) {
+    const int i = threadIdx.x + k * ST_THREADS;
+    if (i < PR * PC) {
+#pragma unroll
+      for (int q = 0; q < 3; ++q) pm[q * PR * PC + i] = lv[q][k];
+    }
+  }
+  __syncthreads();
+
+  // horizontal pass of G^T: out(j) = sum_t g[10 - t] map(j - 10 + t), i.e. patch columns j .. j + 10
+  for (int it = threadIdx.x; it < 3 * PR * (TW / HSEG); it += ST_THREADS) {
+    const int q = it / (PR * (TW / HSEG)), rem = it - q * (PR * (TW / HSEG));
+    const int r = rem / (TW / HSEG), c0 = (rem % (TW / HSEG)) * HSEG;
+    const float4* rv = reinterpret_cast<const float4*>(pm + (q * PR + r) * PC + c0);
+    float v[16];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const float4 t4 = rv[u];
+      v[4 * u] = t4.x; v[4 * u + 1] = t4.y; v[4 * u + 2] = t4.z; v[4 * u + 3] = t4.w;
+    }
+    float s[HSEG];
+#pragma unroll
+    for (int j = 0; j < HSEG; ++j) s[j] = 0.f;
+#pragma unroll
+    for (int k = 0; k < HSEG + WIN - 1; ++k) {
+#pragma unroll
+      for (int j = 0; j < HSEG; ++j) {
+        const int t = k - j;
+        if (t >= 0 && t < WIN) s[j] = fmaf(a.taps[WIN - 1 - t], v[k], s[j]);
+      }
+    }
+    *reinterpret_cast<float4*>(hq + (q * PR + r) * TW + c0) = make_float4(s[0], s[1], s[2], s[3]);
+  }
+  __syncthreads();
+
+  const int col = threadIdx.x % TW, r0 = (threadIdx.x / TW) * VSEG;
+  float m[3][VSEG];
+#pragma unroll
+  for (int j = 0; j < VSEG; ++j) m[0][j] = m[1][j] = m[2][j] = 0.f;
+#pragma unroll
+  for (int k = 0; k < VSEG + WIN - 1; ++k) {
+    float v[3];
+#pragma unroll
+    for (int q = 0; q < 3; ++q) v[q] = hq[(q * PR + r0 + k) * TW + col];
+#pragma unroll
+    for (int j = 0; j < VSEG; ++j) {
+      const int t = k - j;
+      if (t >= 0 && t < WIN) {
+        const float g = a.taps[WIN - 1 - t];
+#pragma unroll
+        for (int q = 0; q < 3; ++q) m[q][j] = fmaf(g, v[q], m[q][j]);
+      }
+    }
+  }
+  const int ix = ox + col;
+  if (ix >= L.w) return;
+  const float kl = bw.coef[plane * MAX_LEVELS + l];
+  const bool coarse = l + 1 < a.levels;
+  const int hc = coarse ? a.lv[l + 1].h : 0, wc = coarse ? a.lv[l + 1].w : 0;
+  const float* gc = coarse ? bw.grad[l + 1] + (long)plane * hc * wc + (ix + (L.w & 1)) / 2 : nullptr;
+  const long poff = (long)plane * L.h * L.w;
+#pragma unroll
+  for (int j = 0; j < VSEG; ++j) {
+    const int iy = oy + r0 + j;
+    if (iy < L.h) {
+      const long e = poff + (long)iy * L.w + ix;
+      const float xv = __ldg(L.x + e) - a.shift, yv = __ldg(L.y + e) - a.shift;
+      float g = kl * (m[0][j] + 2.f * xv * m[1][j] + yv * m[2][j]);
+      if (coarse) g += 0.25f * gc[(long)((iy + (L.h & 1)) / 2) * wc];
+      if (l == 0 && addend) g += addend[e];
+      bw.grad[l][e] = g;
+    }
+  }
+}
+
+// work layout: coefficients, then per level the three coefficient maps, then the gradients of levels 1..L-1
+bool plan_bwd(const Args& a, size_t* coef_bytes, size_t map_bytes[MAX_LEVELS], size_t grad_bytes[MAX_LEVELS],
+              size_t* total) {
+  *coef_bytes = align256(sizeof(float) * (size_t)a.planes * MAX_LEVELS);
+  size_t t = *coef_bytes;
+  for (int l = 0; l < a.levels; ++l) {
+    map_bytes[l] = align256(sizeof(float) * (size_t)a.planes * (a.lv[l].h - (WIN - 1)) * (a.lv[l].w - (WIN - 1)));
+    grad_bytes[l] = l ? align256(sizeof(float) * (size_t)a.planes * a.lv[l].h * a.lv[l].w) : 0;
+    t += 3 * map_bytes[l] + grad_bytes[l];
+  }
+  // the gather grid of level 0 must fit one launch dimension
+  const long tiles0 = (long)((a.lv[0].w + TW - 1) / TW) * ((a.lv[0].h + TH - 1) / TH);
+  if (tiles0 * a.planes > 0x7fffffffL) return false;
+  *total = t;
+  return true;
+}
+
 }  // namespace
 
 extern "C" int64_t masic_ms_ssim_scratch_bytes(int n, int c, int h, int w, int levels) {
@@ -308,19 +643,7 @@ extern "C" int masic_ms_ssim(const float* x, const float* y, int n, int c, int h
   Args a;
   size_t bytes;
   if (!plan(n, c, h, w, levels, &a, &bytes)) return MASIC_EINVAL;
-  // the window of pytorch_msssim's _fspecial_gauss_1d(11, 1.5), in float32 as the package computes it
-  float g[WIN], gs = 0.f;
-  for (int i = 0; i < WIN; ++i) {
-    const float d = (float)(i - WIN / 2);
-    g[i] = expf(-(d * d) / (2.f * 1.5f * 1.5f));
-    gs += g[i];
-  }
-  for (int i = 0; i < WIN; ++i) a.taps[i] = g[i] / gs;
-  a.shift = 0.5f * data_range;
-  a.c1 = (k1 * data_range) * (k1 * data_range);
-  a.c2 = (k2 * data_range) * (k2 * data_range);
-  for (int l = 0; l < MAX_LEVELS; ++l) a.weights[l] = l < levels ? (double)weights_host[l] : 0.0;
-  a.nonneg_last = nonneg_last ? 1 : 0;
+  set_constants(&a, levels, data_range, k1, k2, weights_host, nonneg_last);
 
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   char* base = static_cast<char*>(scratch);
@@ -348,5 +671,70 @@ extern "C" int masic_ms_ssim(const float* x, const float* y, int n, int c, int h
   const int blocks = a.lv[levels - 1].block0 + a.planes * a.lv[levels - 1].tiles;
   msssim_stats_kernel<<<blocks, ST_THREADS, ST_SMEM, s>>>(a, partial);
   msssim_final_kernel<<<a.planes, 32 * 2 * levels, 0, s>>>(a, partial, out_nc);
+  return (int)cudaGetLastError();
+}
+
+extern "C" int64_t masic_ms_ssim_bwd_work_bytes(int n, int c, int h, int w, int levels) {
+  Args a;
+  size_t bytes, coef_bytes, total, map_bytes[MAX_LEVELS], grad_bytes[MAX_LEVELS];
+  if (!plan(n, c, h, w, levels, &a, &bytes)) return MASIC_EINVAL;
+  if (!plan_bwd(a, &coef_bytes, map_bytes, grad_bytes, &total)) return MASIC_EINVAL;
+  return (int64_t)total;
+}
+
+extern "C" int masic_ms_ssim_bwd(const float* x, const float* y, int n, int c, int h, int w, int levels,
+                                 float data_range, float k1, float k2, const float* weights_host, int nonneg_last,
+                                 const void* fwd_scratch, float grad_scale, const float* addend, float* dx, void* work,
+                                 void* stream) {
+  if (!x || !y || !weights_host || !fwd_scratch || !dx || !work) return MASIC_EINVAL;
+  if (!(data_range > 0.f) || !(k1 >= 0.f) || !(k2 >= 0.f)) return MASIC_EINVAL;
+  Args a;
+  size_t bytes, coef_bytes, total, map_bytes[MAX_LEVELS], grad_bytes[MAX_LEVELS];
+  if (!plan(n, c, h, w, levels, &a, &bytes)) return MASIC_EINVAL;
+  if (!plan_bwd(a, &coef_bytes, map_bytes, grad_bytes, &total)) return MASIC_EINVAL;
+  set_constants(&a, levels, data_range, k1, k2, weights_host, nonneg_last);
+
+  // the forward's pyramid and tile partials, at the offsets masic_ms_ssim wrote them
+  const char* fs = static_cast<const char*>(fwd_scratch);
+  a.lv[0].x = x;
+  a.lv[0].y = y;
+  size_t off = 0;
+  for (int l = 1; l < levels; ++l) {
+    const size_t lb = align256(sizeof(float) * a.planes * a.lv[l].h * a.lv[l].w);
+    a.lv[l].x = reinterpret_cast<const float*>(fs + off);
+    a.lv[l].y = reinterpret_cast<const float*>(fs + off + lb);
+    off += 2 * lb;
+  }
+  const double* partial = reinterpret_cast<const double*>(fs + off);
+
+  Bwd bw = {};
+  char* wb = static_cast<char*>(work);
+  float* coef = reinterpret_cast<float*>(wb);
+  bw.coef = coef;
+  size_t woff = coef_bytes;
+  for (int l = 0; l < levels; ++l) {
+    bw.map[l] = reinterpret_cast<float*>(wb + woff);
+    bw.mstride[l] = (long)(map_bytes[l] / sizeof(float));
+    woff += 3 * map_bytes[l];
+  }
+  bw.grad[0] = dx;
+  for (int l = 1; l < levels; ++l) {
+    bw.grad[l] = reinterpret_cast<float*>(wb + woff);
+    woff += grad_bytes[l];
+  }
+
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  cudaError_t e = cudaFuncSetAttribute(msssim_bwd_maps_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)ST_SMEM);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(msssim_bwd_gather_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GA_SMEM);
+  if (e != cudaSuccess) return (int)e;
+  msssim_bwd_coef_kernel<<<a.planes, 32 * 2 * levels, 0, s>>>(a, partial, grad_scale, coef);
+  const int blocks = a.lv[levels - 1].block0 + a.planes * a.lv[levels - 1].tiles;
+  msssim_bwd_maps_kernel<<<blocks, ST_THREADS, ST_SMEM, s>>>(a, bw);
+  for (int l = levels - 1; l >= 0; --l) {
+    const int tiles = ((a.lv[l].w + TW - 1) / TW) * ((a.lv[l].h + TH - 1) / TH);
+    msssim_bwd_gather_kernel<<<a.planes * tiles, ST_THREADS, GA_SMEM, s>>>(a, bw, l, l == 0 ? addend : nullptr);
+  }
   return (int)cudaGetLastError();
 }

@@ -288,12 +288,13 @@ class HSIC(nn.Module):
         """Pipelined host-to-host evaluation of batch-1 stereo pairs (see PairStream)."""
         return PairStream(self, height, width, device, depth=depth, lmbda=lmbda)
 
-    def trainer(self, batch: int, height: int, width: int, device, lmbda: float = 0.01):
+    def trainer(self, batch: int, height: int, width: int, device, lmbda: float = 0.01, metric: str = "mse"):
         """The CUDA training step for this model (forward in train() mode + loss + backward + aux loss):
         `HSICTrainer.step_grads` fills `.grad` of every parameter, `train_step` also all-reduces and steps the
-        two optimisers (coremasic/mywork/newtrain_codec_real.py:105-146)."""
+        two optimisers (coremasic/mywork/newtrain_codec_real.py:105-146).  metric: "mse" (the reference's loss) or
+        "ms-ssim" (CompressAI's MS-SSIM rate-distortion loss on both views, min(H, W) > 160; see HSICTrainer)."""
         from .trainer import HSICTrainer
-        return HSICTrainer(self, batch, height, width, device, lmbda=lmbda)
+        return HSICTrainer(self, batch, height, width, device, lmbda=lmbda, metric=metric)
 
     # ---- bitstreams (MASIC.py:855-1158, :1161-1408)
     def compress(self, x1, x2, h_matrix, output_name, output_path="", device="cpu", y_order="wavefront_streams"):

@@ -131,6 +131,36 @@ def mse_grad(x_hat, x, scale, g, addend=None):
     check(_lib.load().masic_mse_grad(_p(x_hat), _p(x), _p(addend), scale, x.numel(), _p(g), _s()), "masic_mse_grad")
 
 
+def ms_ssim_buffers(n, c, h, w, device, levels=5):
+    """(fwd_scratch, work): device bytes for ms_ssim_fwd and ms_ssim_grad of (n, c, h, w) images (allocate once,
+    outside graph capture)."""
+    lib = _lib.load()
+    fb, wb = lib.masic_ms_ssim_scratch_bytes(n, c, h, w, levels), lib.masic_ms_ssim_bwd_work_bytes(n, c, h, w, levels)
+    check(min(int(fb), int(wb), 0), f"masic_ms_ssim_bwd_work_bytes ({levels} levels of {h}x{w} need >= 11x11 each)")
+    return (torch.empty(int(fb), dtype=torch.uint8, device=device), torch.empty(int(wb), dtype=torch.uint8, device=device))
+
+
+def _msssim_args(x_hat, data_range):
+    from .ops import MS_SSIM_WEIGHTS
+    n, c, h, w = x_hat.shape
+    wts = (C.c_float * len(MS_SSIM_WEIGHTS))(*MS_SSIM_WEIGHTS)
+    return (n, c, h, w, len(MS_SSIM_WEIGHTS), float(data_range), 0.01, 0.03, wts, 1)
+
+
+def ms_ssim_fwd(x_hat, x, fwd_scratch, out, data_range=1.0):
+    """out (n, c) <- pytorch_msssim.ms_ssim(x_hat, x, data_range, size_average=False) per plane; fwd_scratch keeps
+    what ms_ssim_grad reads."""
+    check(_lib.load().masic_ms_ssim(_p(x_hat), _p(x), *_msssim_args(x_hat, data_range), _p(fwd_scratch), _p(out), _s()),
+          "masic_ms_ssim")
+
+
+def ms_ssim_grad(x_hat, x, fwd_scratch, scale, g, addend=None, *, work, data_range=1.0):
+    """g = scale * d(sum of the per-plane MS-SSIM)/d(x_hat) [+ addend], from the scratch of the ms_ssim_fwd call on
+    the same tensors issued before it on the stream."""
+    check(_lib.load().masic_ms_ssim_bwd(_p(x_hat), _p(x), *_msssim_args(x_hat, data_range), _p(fwd_scratch), scale,
+                                        _p(addend), _p(g), _p(work), _s()), "masic_ms_ssim_bwd")
+
+
 def warp_bwd(g0, g1, T, dsrc):
     n, c, h, w = dsrc.shape
     check(_lib.load().masic_warp_perspective_bwd(_p(g0), _p(g1), n, c, h, w, g0.shape[2], g0.shape[3], _p(T), _p(dsrc),

@@ -387,9 +387,18 @@ class TrainStep:
 
 class HSICTrainer(TrainStep):
     def __init__(self, model, batch: int, height: int, width: int, device, lmbda: float = 0.01,
-                 use_graph: bool = True):
+                 use_graph: bool = True, metric: str = "mse"):
+        """metric: the distortion term of the loss, per view.  "mse" is the reference's
+        lambda * 255^2 * (mse1 + mse2) + bpp; "ms-ssim" is CompressAI's RateDistortionLoss(metric="ms-ssim") on both
+        views, lambda * ((1 - ms1) + (1 - ms2)) + bpp with ms_v = pytorch_msssim.ms_ssim(x_v_hat, x_v, data_range=1.0)
+        (MS-SSIM lambdas are on a different scale from MSE ones)."""
+        if metric not in ("mse", "ms-ssim"):
+            raise ValueError(f"metric must be 'mse' or 'ms-ssim', got {metric!r}")
+        if metric == "ms-ssim" and min(height, width) <= 160:
+            raise ValueError(f"metric='ms-ssim' needs min(H, W) > 160 (5 MS-SSIM levels), got {height}x{width}")
         if height % 64 or width % 64:
             raise ValueError("HSIC needs H and W to be multiples of 64")
+        self.metric = metric
         self.lib = _lib.load()
         self.dev = torch.device(device)
         if self.dev.type != "cuda":
@@ -629,6 +638,7 @@ class HSICTrainer(TrainStep):
         npx16 = B * h16 * w16
         scale = T.lik_grad_scale(B * H * W)
         mse_scale = self.lmbda * 255.0 ** 2 * 2.0 / (B * 3 * H * W)
+        ms_scale = -self.lmbda / (B * 3)            # d(lambda (1 - mean over (B, 3) of MS-SSIM)) / d(sum of MS-SSIM)
         o = self.out = {"x1_hat": self._z(B, 3, H, W, dtype=F32), "x2_hat": self._z(B, 3, H, W, dtype=F32),
                         "lik_y1": self._z(B, h16, w16, M, dtype=F32), "lik_y2": self._z(B, h16, w16, M, dtype=F32),
                         "y1_hat": self._z(B, h16, w16, M, dtype=F32), "y2_hat": self._z(B, h16, w16, M, dtype=F32)}
@@ -742,8 +752,24 @@ class HSICTrainer(TrainStep):
         self.rd_out = self._z(8, dtype=F32)
         self.rd_scratch = ops.rd_metrics_scratch(dev)
         liks = [o["lik_y1"], o["lik_y2"], o["lik_z1"], o["lik_z2"]]
-        self.F("loss", lambda: ops.rd_metrics_into(liks, o["x1_hat"], self.x1, o["x2_hat"], self.x2, self.lmbda,
-                                                   self.rd_scratch, self.rd_out))
+        if self.metric == "mse":
+            self.F("loss", lambda: ops.rd_metrics_into(liks, o["x1_hat"], self.x1, o["x2_hat"], self.x2, self.lmbda,
+                                                       self.rd_scratch, self.rd_out))
+        else:
+            # bpp and the MSEs stay as diagnostics; each view's MS-SSIM keeps its own scratch for its backward
+            self.ms_out = self._z(2, B, 3, dtype=F32)
+            self.ms_res = self._z(3, dtype=F32)                   # ms1, ms2, loss
+            s1, self.ms_work = T.ms_ssim_buffers(B, 3, H, W, dev)  # one work: the backward calls run one by one
+            self.ms_scratch = [s1, T.ms_ssim_buffers(B, 3, H, W, dev)[0]]
+
+            def loss():
+                ops.rd_metrics_into(liks, o["x1_hat"], self.x1, o["x2_hat"], self.x2, self.lmbda, self.rd_scratch,
+                                    self.rd_out)
+                T.ms_ssim_fwd(o["x1_hat"], self.x1, self.ms_scratch[0], self.ms_out[0])
+                T.ms_ssim_fwd(o["x2_hat"], self.x2, self.ms_scratch[1], self.ms_out[1])
+                torch.mean(self.ms_out, dim=(1, 2), out=self.ms_res[0:2])
+                torch.add(self.rd_out[6:7], self.lmbda * (2.0 - self.ms_res[0:2].sum()), out=self.ms_res[2:3])
+            self.F("loss", loss)
         # aux loss (entropy_models.py:345-348) of both bottlenecks
         self.aux_out = self._z(1, dtype=F32)
         self.zero_each_step += [self.aux_out]
@@ -767,7 +793,11 @@ class HSICTrainer(TrainStep):
         d_x1hw_a = self._z(B, 3, H, W, dtype=F32)
         d_core = self._z(B, 3, H, W, dtype=F32)
         adw, adb = self.grad("decoder2.after_conv.weight"), self.grad("decoder2.after_conv.bias")
-        self.Bk("mse2", lambda: T.mse_grad(o["x2_hat"], self.x2, mse_scale, gx2))
+        if self.metric == "mse":
+            self.Bk("mse2", lambda: T.mse_grad(o["x2_hat"], self.x2, mse_scale, gx2))
+        else:
+            self.Bk("mse2", lambda: T.ms_ssim_grad(o["x2_hat"], self.x2, self.ms_scratch[1], ms_scale, gx2,
+                                                   work=self.ms_work))
         self.Bk("after_conv", lambda: T.conv_small_bwd(ag, x1hw, aw, True, 3, 5, 1, gx2, din0=d_ag, din1=d_x1hw_a, dweight=adw,
                                                        dbias=adb))
         self.Bk("after_gdn", lambda: after_gdn.bwd(core, d_ag, d_core))
@@ -803,7 +833,11 @@ class HSICTrainer(TrainStep):
         self.Bk("pre_conv", lambda: T.conv_small_bwd(x1_warp, self.x2, pre_w, False, 3, 5, 1, d_pc, dweight=pdw, dbias=pdb))
         # left view
         gx1 = self._z(B, 3, H, W, dtype=F32)
-        self.Bk("mse1", lambda: T.mse_grad(o["x1_hat"], self.x1, mse_scale, gx1, addend=d_x1hat_w))
+        if self.metric == "mse":
+            self.Bk("mse1", lambda: T.mse_grad(o["x1_hat"], self.x1, mse_scale, gx1, addend=d_x1hat_w))
+        else:
+            self.Bk("mse1", lambda: T.ms_ssim_grad(o["x1_hat"], self.x1, self.ms_scratch[0], ms_scale, gx1,
+                                                   addend=d_x1hat_w, work=self.ms_work))
         self.Bk("L.decoder", lambda: dec1["bwd"](gx1))
         self.Bk("L.gmm_net", net1["bwd"])
         self.Bk("L.context", ctx1.bwd)
@@ -857,8 +891,11 @@ class HSICTrainer(TrainStep):
 
     def read_losses(self) -> Dict[str, float]:
         """Loss terms of the last step (one device -> host read; synchronises with the step)."""
-        r = torch.cat([self.rd_out, self.aux_out]).tolist()
-        return {"loss": r[7], "bpp": r[6], "mse": r[4] + r[5], "aux": r[8]}
+        if self.metric == "mse":
+            r = torch.cat([self.rd_out, self.aux_out]).tolist()
+            return {"loss": r[7], "bpp": r[6], "mse": r[4] + r[5], "aux": r[8]}
+        r = torch.cat([self.rd_out, self.aux_out, self.ms_res]).tolist()
+        return {"loss": r[11], "bpp": r[6], "mse": r[4] + r[5], "aux": r[8], "msssim1": r[9], "msssim2": r[10]}
 
     # Lanes, like the inference engine's: the right view's own encoder chain (homography products, mask weights,
     # pre_conv, encoder2, hyperprior 2, context 2) depends on nothing the left view computes, and its backward
